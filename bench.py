@@ -2,11 +2,19 @@
 """Headline benchmark: ViT-B/16 224px bf16 inference images/sec (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl vitk|reference] [--batch B]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (vitk_forward: patch-embed GEMM, 12 pre-LN blocks, CLS
 LayerNorm + 6-class head) over one batch of 256 synthetic images per GPU.  Prints ONE JSON line.
 For N>1 launch under torchrun (one rank per GPU); the batch shards across ranks with no data-path
 collective (weak scaling); time = max over ranks of the device-timed region.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step to DIR/logits.npy
+(float32, one row per image of the timed batch; for N>1 the ranks' shards in rank order).  Weights
+and images are seeded, so two builds run with the same arguments can be compared output for output.
+bench_outputs/ in the repository is git-ignored for such dumps.  The two --impl arms run different
+batches (256 seeded images per GPU against 32 for the CPU arm), so only dumps of the same --impl
+compare.
 
 Next to the headline the same line carries, each device-timed with its own TFLOP/s and fraction
 of the measured burst peak: the other BASELINE.json configurations (`configs`: ViT-L/16 weak and
@@ -52,6 +60,15 @@ def fwd_flops_per_image(cfg=VIT_B16, n_prefix=1, n_classes=N_CLASSES) -> float:
     Kp = cfg["in_channels"] * cfg["patch_size"] ** 2
     return 2 * P * Kp * D + L * (2 * N * D * 3 * D + 4 * N * N * D + 2 * N * D * D + 4 * N * D * M) \
         + 2 * D * n_classes
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each tensor as <out_dir>/<name>.npy in float32."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(d / f"{name}.npy", t.detach().float().cpu().numpy())
 
 
 def measured_peaks() -> tuple[dict, str]:
@@ -196,15 +213,17 @@ def run_reference(args) -> None:
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     run, kind, what = _cpu_forward_fn(batch)
-    steps = min(args.steps, 8)   # bounded: a step is ~1-4 s of host time
+    steps = args.steps
     warm = min(args.warmup, 1)
     with torch.no_grad():
         for _ in range(max(warm, 1)):
             run()
         t0 = time.perf_counter()
         for _ in range(steps):
-            run()
+            logits = run()
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": logits})
     val = batch * steps / dt
     sample = f"{what}, {cores} threads; {steps} steps x batch {batch} of the ViT-B/16 workload"
     _emit(json.dumps({
@@ -721,6 +740,13 @@ def run_vitk(args) -> None:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
         value = n_gpus * B * args.steps / (ms * 1e-3)
+        if args.dump_outputs:
+            shards = [logits]
+            if world > 1:
+                shards = [torch.empty_like(logits) for _ in range(world)]
+                dist.all_gather(shards, logits)
+            if rank == 0:
+                dump_outputs(args.dump_outputs, {"logits": torch.cat(shards)})
 
         # ---- per-kernel-class device times over the same steps (events around every launch)
         vitk._lib.profile_enable(True)
@@ -933,7 +959,11 @@ def main():
                     help="skip the ViT-L/16 and 384 px legs (BASELINE.json configs[3], configs[4])")
     ap.add_argument("--no-eager-baseline", action="store_true",
                     help="skip the PyTorch-eager bf16 run of the reference's classes on this GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the logits of the last timed step to DIR/logits.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -51,15 +51,18 @@ def test_oracle_train_step_matches_reference(name):
 
 
 def test_module_mirrors_reproduce_reference_state_dict(vitk):
-    """Same constructor order => same RNG stream => identical random init; same keys/shapes."""
-    z, cfg = H.load("tiny_vit_full")
-    torch.manual_seed(int(z["seed"]))
-    m = vitk.ViTClassifier(num_classes=6, **cfg)
-    ref = H.weights(z)
-    sd = m.state_dict()
-    assert list(sd.keys()) == list(ref.keys())
-    for k in ref:
-        assert torch.equal(sd[k], ref[k]), k
+    """Same constructor order => same RNG stream => identical random init; same keys/shapes.
+    Checked for the ViT and the DeiT mirror against the weights (in the reference's key order)
+    that the reference's own constructors produced for each *_full fixture."""
+    for name in FULL:
+        z, cfg = H.load(name)
+        torch.manual_seed(int(z["seed"]))
+        m = vitk.ViTClassifier(num_classes=6, deit=str(z["kind"]) == "deit", **cfg)
+        ref = H.weights(z)
+        sd = m.state_dict()
+        assert list(sd.keys()) == list(ref.keys()), name
+        for k in ref:
+            assert torch.equal(sd[k], ref[k]), (name, k)
 
 
 @pytest.mark.skipif(not ref_loader.reference_available(), reason="reference only in the build box")
