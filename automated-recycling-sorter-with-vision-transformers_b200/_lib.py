@@ -15,7 +15,7 @@ PKG_DIR = Path(__file__).resolve().parent
 # VITK_LIB: another build of the same library (same ABI), for A/B timing of kernel variants on one box
 LIB_PATH = Path(os.environ["VITK_LIB"]) if os.environ.get("VITK_LIB") else PKG_DIR / "libvitk.so"
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 EPI_BF16 = 0
 EPI_GELU_BF16 = 1
@@ -130,7 +130,6 @@ _SIGNATURES = {
     "vitk_launch_count": (C.c_longlong, []),
     "vitk_gemm_set_cta_group": (C.c_int, [C.c_int]),
     "vitk_gemm_set_direct_epilogue": (C.c_int, [C.c_int]),
-    "vitk_gemm_set_fused_layernorm": (C.c_int, [C.c_int]),
     "vitk_debug_gemm_trace": (C.c_int, [C.c_void_p, C.c_int]),
     "vitk_set_layernorm_folding": (C.c_int, [C.c_int]),
     "vitk_fold_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -146,7 +145,6 @@ _SIGNATURES = {
                                              C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_void_p]),
     "vitk_attention_set_impl": (C.c_int, [C.c_int]),
     "vitk_reserve_sms": (C.c_int, [C.c_int]),
-    "vitk_set_pdl": (C.c_int, [C.c_int]),
     "vitk_postprocess_scores": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p]),
     "vitk_postprocess_detections": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
@@ -173,7 +171,7 @@ _SIGNATURES = {
     "vitk_gemm_resid_layernorm": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                             C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
-                                            C.c_void_p, C.c_void_p]),
+                                            C.c_void_p]),
     "vitk_gemm_wgrad": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                   C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_int, C.c_void_p]),
     "vitk_layernorm": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -321,12 +319,6 @@ def set_gemm_cta_group(ctas: int) -> None:
 
 def set_gemm_direct_epilogue(on: bool) -> None:
     check(lib().vitk_gemm_set_direct_epilogue(1 if on else 0))
-
-
-def set_gemm_fused_layernorm(on: bool) -> None:
-    """True = the LayerNorm after a residual GEMM runs inside the GEMM kernel (A/B, tests);
-    default False: a separate launch (measured faster).  Same bits either way."""
-    check(lib().vitk_gemm_set_fused_layernorm(1 if on else 0))
 
 
 def set_layernorm_folding(on: bool) -> None:

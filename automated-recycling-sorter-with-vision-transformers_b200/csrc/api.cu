@@ -66,8 +66,6 @@ struct Workspace {
   float* c_x;   // f32 [B, D]
   void* c_b;    // bf16 [B, D]  (attention context, then the LayerNorm output)
   void* c_h;    // bf16 [B, Mlp]
-  unsigned int* ln_cnt;  // per 128-row block arrival counters of the fused LayerNorm tail
-  size_t ln_cnt_bytes;
   float2* stats;         // folded LayerNorm: [gemm_stats_parts(D)][M] partial (sum, sum of squares)
   size_t bytes;
 };
@@ -89,39 +87,9 @@ Workspace carve(const Dims& d, void* base) {
   w.c_x = static_cast<float*>(take(static_cast<size_t>(d.B) * d.D * 4));
   w.c_b = take(static_cast<size_t>(d.B) * d.D * 2);
   w.c_h = take(static_cast<size_t>(d.B) * d.Mlp * 2);
-  w.ln_cnt_bytes = static_cast<size_t>((d.M + 127) / 128) * 4;
-  w.ln_cnt = static_cast<unsigned int*>(take(w.ln_cnt_bytes));
   w.stats = static_cast<float2*>(take(static_cast<size_t>(gemm_stats_parts(d.D)) * d.M * 8));
   w.bytes = off;
   return w;
-}
-
-// x += A W^T + bias, then xn = LN(x) * gamma + beta as bf16 - one launch (gemm_sm100.cu: the
-// residual GEMM's LayerNorm tail).  train.py:586-591.
-int linear_resid_ln(const void* A, int lda, const void* W, int M, int N, int K, const float* bias,
-                    float* x, const float* gamma, const float* beta, float eps, void* xn,
-                    unsigned int* counters, cudaStream_t stream) {
-  GemmProblem p;
-  p.A = A;
-  p.lda = lda;
-  p.B = W;
-  p.ldb = K;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = EPI_RESID_F32;
-  p.e.bias = bias;
-  p.e.resid = x;
-  p.e.ldr = N;
-  p.e.out = x;
-  p.e.ldo = N;
-  p.e.ln_out = xn;
-  p.e.ln_ldo = N;
-  p.e.ln_gamma = gamma;
-  p.e.ln_beta = beta;
-  p.e.ln_eps = eps;
-  p.e.ln_counters = counters;
-  return gemm_bf16_tn(p, stream);
 }
 
 int linear(const void* A, int lda, const void* W, int M, int N, int K, GemmEpi epi,
@@ -143,6 +111,15 @@ int linear(const void* A, int lda, const void* W, int M, int N, int K, GemmEpi e
   p.e.out2 = out2;
   p.e.ldo = ldo;
   return gemm_bf16_tn(p, stream);
+}
+
+// x += A W^T + bias, then xn = LN(x) * gamma + beta as bf16: the residual GEMM and a layernorm_fwd
+// launch.  train.py:586-591.
+int linear_resid_ln(const void* A, int lda, const void* W, int M, int N, int K, const float* bias,
+                    float* x, const float* gamma, const float* beta, float eps, void* xn,
+                    cudaStream_t stream) {
+  VITK_TRY(linear(A, lda, W, M, N, K, EPI_RESID_F32, bias, x, N, x, nullptr, N, stream));
+  return layernorm_fwd(x, N, gamma, beta, xn, 0, N, nullptr, nullptr, M, N, eps, stream);
 }
 
 // x += A W^T + bias in place; xb = bf16(x); partial row statistics of the updated x.
@@ -244,8 +221,6 @@ int forward_bf16(const VitkConfig* cfg, const VitkWeights* w, const float* image
                  const U8Input* u8 = nullptr, bool cls_only_tail = false) {
   const int M = static_cast<int>(d.M), D = d.D;
   SweepAlternation sweep;  // consecutive row-ordered kernels run in opposite directions (L2 reuse)
-  // the fused LayerNorm tails leave their counters zero-filled; start from a known state anyway
-  VITK_CHECK_CUDA(cudaMemsetAsync(ws.ln_cnt, 0, ws.ln_cnt_bytes, stream));
   // -- patch embedding as a GEMM; epilogue adds bias + position embedding and writes each patch
   //    row at its token slot (evaluation.py:142-149)
   if (u8 != nullptr)
@@ -310,9 +285,9 @@ int forward_bf16(const VitkConfig* cfg, const VitkWeights* w, const float* image
     return VITK_OK;
   }
   // -- encoder blocks (train.py:584-593)
-  // LayerNorm 1 of block 0 is the only stand-alone normalisation between blocks: every later one
-  // is the tail of the residual GEMM that produces its input (projection -> LN2, linear2 -> LN1
-  // of the next block)
+  // LayerNorm 1 of block 0 runs on its own; every later one follows the residual GEMM that
+  // produces its input in linear_resid_ln (projection -> LN2, linear2 -> LN1 of the next
+  // block)
   VITK_TRY(layernorm_fwd(ws.x, D, w->blocks[0].ln1_w, w->blocks[0].ln1_b, ws.xn, 0, D, nullptr,
                          nullptr, M, D, cfg->ln_eps, stream));
   for (int l = 0; l < d.L; ++l) {
@@ -322,13 +297,13 @@ int forward_bf16(const VitkConfig* cfg, const VitkWeights* w, const float* image
     if (cls_only_tail && l == d.L - 1) return cls_tail(cfg, w, d, ws, logits_out, stream);
     VITK_TRY(attention_fwd(ws.qkv, ws.ctx, nullptr, d.B, d.N, d.H, d.hd, stream));
     VITK_TRY(linear_resid_ln(ws.ctx, D, bw.proj_w, M, D, D, bw.proj_b, ws.x, bw.ln2_w, bw.ln2_b,
-                             cfg->ln_eps, ws.xn, ws.ln_cnt, stream));
+                             cfg->ln_eps, ws.xn, stream));
     VITK_TRY(linear(ws.xn, D, bw.fc1_w, M, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b, nullptr, 0, ws.h,
                     nullptr, d.Mlp, stream));
     if (l + 1 < d.L) {
       const VitkBlockWeights& nx = w->blocks[l + 1];
       VITK_TRY(linear_resid_ln(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, bw.fc2_b, ws.x, nx.ln1_w,
-                               nx.ln1_b, cfg->ln_eps, ws.xn, ws.ln_cnt, stream));
+                               nx.ln1_b, cfg->ln_eps, ws.xn, stream));
     } else {
       VITK_TRY(linear(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.x, D, ws.x,
                       nullptr, D, stream));
@@ -475,10 +450,6 @@ int vitk_gemm_set_direct_epilogue(int on) {
   return VITK_OK;
 }
 int vitk_debug_gemm_trace(long long* out_host, int n) { return gemm_debug_trace(out_host, n); }
-int vitk_gemm_set_fused_layernorm(int on) {
-  gemm_set_fused_layernorm(on != 0);
-  return VITK_OK;
-}
 int vitk_set_layernorm_folding(int on) {
   g_ln_fold = on != 0;
   return VITK_OK;
@@ -565,10 +536,6 @@ int vitk_linear_rows_backward(const float* x, long long row_stride, const float*
                               int in_features, int out_features, vitk_stream_t stream) {
   return linear_rows_bwd(x, row_stride, weight, dy, dx, dweight, dbias, rows, in_features,
                          out_features, static_cast<cudaStream_t>(stream));
-}
-int vitk_set_pdl(int on) {
-  set_pdl(on);
-  return VITK_OK;
 }
 int vitk_reserve_sms(int n) {
   VITK_REQUIRE(n >= 0 && n <= 64, "reserve_sms: 0 <= n <= 64");
@@ -725,8 +692,10 @@ int vitk_gemm(const void* A, int lda, const void* B, int ldb, int M, int N, int 
 int vitk_gemm_resid_layernorm(const void* A, int lda, const void* W, int ldb, int M, int N, int K,
                               const float* bias, float* x_inout, const float* gamma,
                               const float* beta, float eps, void* ln_out, float* mean_out,
-                              float* rstd_out, unsigned int* counters, vitk_stream_t stream) {
-  VITK_REQUIRE(ln_out != nullptr && x_inout != nullptr, "gemm_resid_layernorm: null output");
+                              float* rstd_out, vitk_stream_t stream) {
+  // checked before the GEMM updates x: layernorm_fwd takes rows of at most 1024 features
+  VITK_REQUIRE(ln_out && x_inout && gamma && beta && N <= 1024,
+               "gemm_resid_layernorm: null operand or N > 1024");
   GemmProblem p;
   p.A = A;
   p.lda = lda;
@@ -741,15 +710,9 @@ int vitk_gemm_resid_layernorm(const void* A, int lda, const void* W, int ldb, in
   p.e.ldr = N;
   p.e.out = x_inout;
   p.e.ldo = N;
-  p.e.ln_out = ln_out;
-  p.e.ln_ldo = N;
-  p.e.ln_gamma = gamma;
-  p.e.ln_beta = beta;
-  p.e.ln_eps = eps;
-  p.e.ln_mean = mean_out;
-  p.e.ln_rstd = rstd_out;
-  p.e.ln_counters = counters;
-  return gemm_bf16_tn(p, static_cast<cudaStream_t>(stream));
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  VITK_TRY(gemm_bf16_tn(p, st));
+  return layernorm_fwd(x_inout, N, gamma, beta, ln_out, 0, N, mean_out, rstd_out, M, N, eps, st);
 }
 
 int vitk_gemm_wgrad(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* out,

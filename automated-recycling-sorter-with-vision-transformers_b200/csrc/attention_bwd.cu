@@ -8,8 +8,6 @@
 // N <= 256 tokens, head_dim 64.
 #include <cuda_bf16.h>
 
-#include <cstdlib>
-
 #include <mutex>
 
 #include "common.h"
@@ -271,12 +269,7 @@ int attention_bwd(const void* qkv, const void* ctx, const void* dctx, const floa
   VITK_REQUIRE(qkv && ctx && dctx && lse && dqkv, "attention_bwd: null operand");
   const bool dropping = drop != nullptr && drop->thresh != 0u;
   if ((attention_impl() != 1 || dropping) && hd == 64 && N <= 256 && device_cc() >= 100) {
-    // VITK_ATTN_BWD_PIPELINE=0 keeps the block-serial kernel for every shape (A/B measurements)
-    static const bool pipelined = [] {
-      const char* v = std::getenv("VITK_ATTN_BWD_PIPELINE");
-      return v == nullptr || v[0] != '0';
-    }();
-    if (pipelined && attention_bwd_tc2_fits(N, H, dbias != nullptr))
+    if (attention_bwd_tc2_fits(N, H, dbias != nullptr))
       return attention_bwd_tc2(qkv, ctx, dctx, lse, dqkv, B, N, H, hd, stream, drop, dbias);
     return attention_bwd_tc(qkv, ctx, dctx, lse, dqkv, B, N, H, hd, stream, drop, dbias);
   }

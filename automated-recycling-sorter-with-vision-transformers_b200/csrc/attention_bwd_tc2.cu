@@ -185,8 +185,6 @@ attn_bwd_tc2_kernel(const __grid_constant__ CUtensorMap tm_qkv,   // box {64, mi
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-  pdl_launch_dependents();
 
   auto rows_in_tile = [&](int t) { return min(128, Nk - t * 128); };  // multiple of 16
 
@@ -712,15 +710,10 @@ int attention_bwd_tc2(const void* qkv, const void* ctx, const void* dctx, const 
   int grid = sm_count();
   if (B * H < grid) grid = B * H;
   ProfileScope prof(PROF_ATTN, 10.0 * B * H * static_cast<double>(N) * N * hd, stream);
-  const cudaError_t le =
-      prm.drop.thresh != 0u
-          ? launch_pdl(attn_bwd_tc2_kernel<true>, dim3(grid), dim3(kThreads), smem, stream, tq, tdo,
-                       tq1, tdo1, tout, prm)
-          : launch_pdl(attn_bwd_tc2_kernel<false>, dim3(grid), dim3(kThreads), smem, stream, tq, tdo,
-                       tq1, tdo1, tout, prm);
-  if (le != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "launch of attn_bwd_tc2_kernel failed: %s",
-                     cudaGetErrorString(le));
+  if (prm.drop.thresh != 0u)
+    attn_bwd_tc2_kernel<true><<<grid, kThreads, smem, stream>>>(tq, tdo, tq1, tdo1, tout, prm);
+  else
+    attn_bwd_tc2_kernel<false><<<grid, kThreads, smem, stream>>>(tq, tdo, tq1, tdo1, tout, prm);
   VITK_CHECK_LAUNCH("attn_bwd_tc2_kernel");
   return VITK_OK;
 }

@@ -201,8 +201,6 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tm_q,
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();  // the prologue above overlapped the previous kernel; qkv is read from here on
-  pdl_launch_dependents();
 
   // 768 threads x 80 registers at launch; the producer / issuer warpgroup hands most of its share to
   // the four softmax warpgroups: 128 x (40 + 4 x 88 + 72) = 58 K <= the 60 K allocated at launch.
@@ -516,15 +514,10 @@ int attention_fwd_tc2(const void* qkv, void* ctx, float* lse, int B, int N, int 
   int grid = sm_count();
   if (B * H < grid) grid = B * H;
   ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(N) * N * hd, stream);
-  const cudaError_t le =
-      prm.drop.thresh != 0u
-          ? launch_pdl(attn_fwd_tc2_kernel<true>, dim3(grid), dim3(kThreads2), smem, stream, tq, tkv,
-                       to, prm)
-          : launch_pdl(attn_fwd_tc2_kernel<false>, dim3(grid), dim3(kThreads2), smem, stream, tq, tkv,
-                       to, prm);
-  if (le != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "launch of attn_fwd_tc2_kernel failed: %s",
-                     cudaGetErrorString(le));
+  if (prm.drop.thresh != 0u)
+    attn_fwd_tc2_kernel<true><<<grid, kThreads2, smem, stream>>>(tq, tkv, to, prm);
+  else
+    attn_fwd_tc2_kernel<false><<<grid, kThreads2, smem, stream>>>(tq, tkv, to, prm);
   VITK_CHECK_LAUNCH("attn_fwd_tc2_kernel");
   return VITK_OK;
 }

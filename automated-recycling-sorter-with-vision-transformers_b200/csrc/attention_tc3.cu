@@ -156,8 +156,6 @@ attn_fwd_tc3_kernel(const __grid_constant__ CUtensorMap tm_q,    // box {64, 128
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-  pdl_launch_dependents();
 
   if (warp < 4) {
     setmaxnreg_dec<40>();
@@ -603,11 +601,7 @@ int attention_fwd_tc3(const void* qkv, void* ctx, float* lse, int B, int N, int 
   }
   if (static_cast<long long>(B) * H * prm.parts < grid) grid = B * H * prm.parts;
   ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(N) * N * hd, stream);
-  const cudaError_t le = launch_pdl(attn_fwd_tc3_kernel, dim3(grid), dim3(kThreads3), smem, stream,
-                                    tq, tkv, tkv_tail, to, prm);
-  if (le != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "launch of attn_fwd_tc3_kernel failed: %s",
-                     cudaGetErrorString(le));
+  attn_fwd_tc3_kernel<<<grid, kThreads3, smem, stream>>>(tq, tkv, tkv_tail, to, prm);
   VITK_CHECK_LAUNCH("attn_fwd_tc3_kernel");
   return VITK_OK;
 }

@@ -1,7 +1,5 @@
 #include "common.h"
 
-#include <cstdlib>
-
 #include <cstdarg>
 #include <cstring>
 #include <atomic>
@@ -102,17 +100,10 @@ SweepAlternation::SweepAlternation() {
 }
 SweepAlternation::~SweepAlternation() { --t_sweep_depth; }
 int sweep_next() {
-  if (t_sweep_depth == 0 || std::getenv("VITK_NO_SWEEP_ALTERNATION") != nullptr) return 0;
+  if (t_sweep_depth == 0) return 0;
   const int d = t_sweep_dir;
   t_sweep_dir ^= 1;
   return d;
-}
-
-static int g_pdl = -1;  // -1: from the environment
-void set_pdl(int on) { g_pdl = on ? 1 : 0; }
-bool pdl_enabled() {
-  if (g_pdl < 0) g_pdl = std::getenv("VITK_PDL") != nullptr ? 1 : 0;
-  return g_pdl != 0;
 }
 
 static int g_sm_reserve = 0;

@@ -74,29 +74,6 @@ struct SweepAlternation {
 };
 int sweep_next();  // direction for the kernel being launched: 0 ascending, 1 descending
 
-// Launch with programmatic stream serialization (see ptx.cuh: pdl_wait): the kernel's CTAs may be
-// scheduled as soon as the preceding kernel's CTAs drain instead of after the whole grid has been
-// retired and the next launch processed.  Off unless VITK_PDL=1 / vitk_set_pdl(1): measured on
-// B200 (tests/ab_pdl.py, interleaved A/B) it changes the ViT-B/16 forward by < 1 % - the host runs
-// far ahead of the device, so launch latency is already hidden.
-bool pdl_enabled();
-void set_pdl(int on);
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                       cudaStream_t stream, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 // Cached per current device, minus the SMs set aside with reserve_sms (persistent kernels size
 // their grids with it: a data-parallel backward leaves a few SMs to the NCCL kernels it overlaps).
 int sm_count();

@@ -15,12 +15,10 @@
 //                     register->global path remains for the token-row remap of the patch embed.
 #include "gemm_sm100.cuh"
 
-#include <cstdlib>
 #include <mutex>
 
 #include "common.h"
 #include "ptx.cuh"
-#include "rowops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -46,33 +44,6 @@ constexpr int kNumEpiWarps = 8;
 constexpr int kFirstEpiWarp = 4;
 constexpr int kNumThreads = (kFirstEpiWarp + kNumEpiWarps) * 32;  // 384
 constexpr int kAccStages = 2;
-// Fused LayerNorm tail (opt-in, vitk_gemm_set_fused_layernorm): two more warpgroups normalise
-// finished row blocks.  640 threads x 96 registers at launch = 61 440; setmaxnreg re-balances
-// within that (an .inc can only take what a .dec of the same CTA released): producer / MMA
-// warpgroup 40, epilogue warpgroups 128, LayerNorm warpgroups 88.  The rows arrive by bulk copies
-// into a shared-memory ring, so that what the tail keeps in flight is bounded by shared memory and
-// not by registers: under a DRAM-saturated GEMM the memory system answers in microseconds and a
-// reader gets bandwidth in proportion to its bytes in flight.
-// Measured on B200, ViT-B/16 batch 256, projection shape (M 50 432, N = K = 768), per call:
-//   GEMM + layernorm_fwd, two launches ................................ 124 us   <- default
-//   4 LayerNorm warps, rows loaded into registers (24 KB in flight) ... 410 us
-//   4 warps, bulk-copy ring (64 KB in flight) .......................... 296 us
-//   8 warps, bulk-copy ring ............................................ 235 us
-//   same, rows fetched but not normalised .............................. 125 us
-//   same, no LayerNorm work at all (4 stages, 1 slab, counters) ........ 94 us (80 us: 5 stages)
-// The tail is bound by instruction latency: ~300 dependent instructions per row on 8 warps per SM
-// against the 40 warps per SM of the stand-alone kernel, plus the spread of the "last arriver"
-// assignment (2.7 row blocks per CTA on average, 6 on the unluckiest).  Bit-exact and tested, but
-// not the default.
-constexpr int kNumLnWarps = 8;
-constexpr int kFirstLnWarp = kFirstEpiWarp + kNumEpiWarps;            // 12
-constexpr int kNumThreadsLn = kNumThreads + kNumLnWarps * 32;         // 640
-constexpr int kLnSlots = 8;   // at most this many rows in flight per LayerNorm warp
-// Ring of rows in flight: 64 KB for the CTA-pair kernels (16 rows of 1024 floats; with one output
-// slab per epilogue warp that leaves four operand stages), 32 KB for the single-CTA ones.
-__host__ __device__ constexpr int ln_ring_bytes(int ctas) { return ctas == 2 ? 65536 : 32768; }
-constexpr int kLnJobs = 8;    // depth of the per-CTA ring of row blocks waiting for LayerNorm
-constexpr int kLnMaxVec = 8;  // float4 per lane and row: D <= 1024 (as layernorm_fwd_kernel)
 
 // CTAS == 1: one CTA computes a 128 x BLOCK_N tile (tcgen05.mma.cta_group::1, M = 128).
 // CTAS == 2: a CTA pair (cluster of 2, same TPC) computes a 256 x BLOCK_N tile with
@@ -80,10 +51,8 @@ constexpr int kLnMaxVec = 8;  // float4 per lane and row: D <= 1024 (as layernor
 //            the B rows, so per-SM L2->SMEM traffic and SMEM read bandwidth per flop drop by 1/3.
 // Epilogue staging: per warp SLABS 32-row x 128-byte slabs (two alternate for TMA stores; the
 // gelu'-epilogue adds one that receives the pre-activation tile by TMA load).
-// LN_RING: bytes of the LayerNorm tail's row ring (0 = no tail).
-template <int BLOCK_N, int CTAS, int SLABS = 2, int LN_RING = 0>
+template <int BLOCK_N, int CTAS, int SLABS = 2>
 struct Cfg {
-  static constexpr int kLnRingBytes = LN_RING;
   static constexpr int kStagingPerWarp = SLABS * 4096;
   static constexpr int kStagingBytes = kNumEpiWarps * kStagingPerWarp;
   static constexpr int kABytes = kBlockM * kBlockK * 2;
@@ -91,18 +60,16 @@ struct Cfg {
   static constexpr int kBBytes = kBRows * kBlockK * 2;
   static constexpr int kStageBytes = kABytes + kBBytes;
   static constexpr int kBarBytes = 1024;
-  static constexpr int kBudget = 232448 - 1024 - kBarBytes - kStagingBytes - kLnRingBytes;
+  static constexpr int kBudget = 232448 - 1024 - kBarBytes - kStagingBytes;
   static constexpr int kStages = kBudget / kStageBytes > 8 ? 8 : kBudget / kStageBytes;
   static constexpr int kTmemCols = kAccStages * BLOCK_N;  // 512 or 256 (power of two)
   static constexpr int kSmemBytes =
-      kStages * kStageBytes + kStagingBytes + kLnRingBytes + kBarBytes + 1024;
+      kStages * kStageBytes + kStagingBytes + kBarBytes + 1024;
   static_assert(kStages >= 3, "pipeline too shallow");
   static_assert(kSmemBytes <= 232448, "exceeds 227 KB of shared memory");
-  // barriers: operand ring, accumulator stages, TMEM slot, aux slabs, LayerNorm job ring (+ its
-  // job ids and two counters)
-  static constexpr int kNumBars = 2 * kStages + 2 * kAccStages + 1 + kNumEpiWarps + 2 * kLnJobs +
-                                  kNumLnWarps * kLnSlots + kNumEpiWarps;
-  static_assert(8 * kNumBars + 4 * (kLnJobs + 2) <= kBarBytes, "barrier block too small");
+  // barriers: operand ring, accumulator stages, TMEM slot, two aux slabs per epilogue warp
+  static constexpr int kNumBars = 2 * kStages + 2 * kAccStages + 1 + 2 * kNumEpiWarps;
+  static_assert(8 * kNumBars <= kBarBytes, "barrier block too small");
 };
 
 __device__ __forceinline__ float gelu_erf(float x) {
@@ -485,12 +452,11 @@ __device__ __forceinline__ void resid_chunk_staged(const uint32_t (&v)[32], int 
 
 // One epilogue warp: stage a 32-row x 128-byte slab (row = lane) in swizzled smem and hand it to
 // the TMA engine.  `pk` holds the lane's 128 output bytes. Two buffers alternate per warp.
-template <int NBUF = 2>
 __device__ __forceinline__ void stage_and_store(const uint32_t (&pk)[32], uint32_t stg, int& buf,
                                                 int lane, const CUtensorMap* tmap, int c0, int c1,
                                                 bool reduce) {
-  // the slab stored NBUF steps ago has been read out
-  if (lane == 0) tma_store_wait_read<NBUF - 1>();
+  // the slab stored two steps ago has been read out
+  if (lane == 0) tma_store_wait_read<1>();
   __syncwarp();
   const uint32_t slab = stg + static_cast<uint32_t>(buf) * 4096u;
   const uint32_t row = slab + static_cast<uint32_t>(lane) * 128u;
@@ -507,132 +473,28 @@ __device__ __forceinline__ void stage_and_store(const uint32_t (&pk)[32], uint32
       tma_store_2d(tmap, slab, c0, c1);
     tma_store_commit();
   }
-  buf = (NBUF == 2) ? (buf ^ 1) : 0;
+  buf ^= 1;
 }
-
-__device__ __forceinline__ float ln_warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-
-// LayerNorm tail of the residual GEMM.  nn.LayerNorm(D), eps inside the sqrt, biased variance
-// (train.py:581-582,586,590); the lane -> element mapping and the order of every sum are those of
-// layernorm_fwd_kernel (rowops.cu), so the fused and the stand-alone forms agree bit for bit.
-// NV > 0: D == 128 * NV exactly (no predicates: 768 -> 6, 1024 -> 8); NV == 0: any D <= 1024.
-template <int NV>
-struct LnTail {
-  static constexpr int kVec = NV > 0 ? NV : kLnMaxVec;
-  static __device__ __forceinline__ bool has(int j, int lane, int nvec) {
-    return NV > 0 || lane + 32 * j < nvec;
-  }
-  // this lane's float4s of a row that a bulk copy has landed in shared memory
-  static __device__ __forceinline__ void load_row(float4 (&v)[kVec], uint32_t row_smem, int lane,
-                                                  int nvec) {
-#pragma unroll
-    for (int j = 0; j < kVec; ++j)
-      if (has(j, lane, nvec))
-        asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];"
-                     : "=f"(v[j].x), "=f"(v[j].y), "=f"(v[j].z), "=f"(v[j].w)
-                     : "r"(row_smem + static_cast<uint32_t>(lane + 32 * j) * 16u)
-                     : "memory");
-  }
-  // statistics, normalisation and the bf16 store of one row held in registers (v is consumed:
-  // centred in place, so that one copy of the row is live)
-  static __device__ __forceinline__ void finish_row(float4 (&v)[kVec], int r, int D,
-                                                    const GemmEpilogue& e, int lane, int nvec) {
-    if (e.ln_xcopy != nullptr) {
-      float4* xc = reinterpret_cast<float4*>(e.ln_xcopy + static_cast<size_t>(r) * D) + lane;
-#pragma unroll
-      for (int j = 0; j < kVec; ++j)
-        if (has(j, lane, nvec)) xc[32 * j] = v[j];
-    }
-    float s = 0.f;
-#pragma unroll
-    for (int j = 0; j < kVec; ++j)
-      if (has(j, lane, nvec)) s += (v[j].x + v[j].y) + (v[j].z + v[j].w);
-    const float mean = ln_warp_sum(s) / static_cast<float>(D);
-    float sq = 0.f;
-#pragma unroll
-    for (int j = 0; j < kVec; ++j)
-      if (has(j, lane, nvec)) {
-        v[j].x -= mean;
-        v[j].y -= mean;
-        v[j].z -= mean;
-        v[j].w -= mean;
-        sq += (v[j].x * v[j].x + v[j].y * v[j].y) + (v[j].z * v[j].z + v[j].w * v[j].w);
-      }
-    const float rstd = rsqrtf(ln_warp_sum(sq) / static_cast<float>(D) + e.ln_eps);
-    if (lane == 0) {
-      if (e.ln_mean) e.ln_mean[r] = mean;
-      if (e.ln_rstd) e.ln_rstd[r] = rstd;
-    }
-    uint2* yr = reinterpret_cast<uint2*>(static_cast<__nv_bfloat16*>(e.ln_out) +
-                                         static_cast<size_t>(r) * e.ln_ldo) + lane;
-    const float4* const g4 = reinterpret_cast<const float4*>(e.ln_gamma) + lane;
-    const float4* const b4 = reinterpret_cast<const float4*>(e.ln_beta) + lane;
-#pragma unroll
-    for (int j = 0; j < kVec; ++j)
-      if (has(j, lane, nvec)) {
-        const float4 g = __ldg(g4 + 32 * j);
-        const float4 b = __ldg(b4 + 32 * j);
-        uint2 pk;
-        pk.x = pack_bf16x2(v[j].x * rstd * g.x + b.x, v[j].y * rstd * g.y + b.y);
-        pk.y = pack_bf16x2(v[j].z * rstd * g.z + b.z, v[j].w * rstd * g.w + b.w);
-        yr[32 * j] = pk;
-      }
-  }
-  // One warp normalises rows r_first, r_first + r_step, ... < r_end of x.  Up to `slots` rows are
-  // in flight as bulk copies (global -> this warp's part of the ring, completion on one mbarrier
-  // per slot); a slot is refilled as soon as every lane has taken its part of the row.
-  // `phases`: parity bit per slot, carried across calls.
-  static __device__ __forceinline__ void rows(const float* __restrict__ x, int ldx, int r_first,
-                                              int r_end, int r_step, int D, const GemmEpilogue& e,
-                                              int lane, uint32_t ring, uint32_t bar0, int slots,
-                                              uint32_t& phases) {
-    const int nvec = NV > 0 ? 32 * NV : (D >> 2);
-    const uint32_t row_bytes = static_cast<uint32_t>(D) * 4u;
-    auto fetch = [&](int r, int slot) {  // lane 0
-      mbar_arrive_expect_tx(bar0 + 8u * slot, row_bytes);
-      bulk_load_1d(ring + static_cast<uint32_t>(slot) * row_bytes,
-                   x + static_cast<size_t>(r) * ldx, row_bytes, bar0 + 8u * slot);
-    };
-    if (lane == 0) {
-      int r = r_first;
-      for (int sl = 0; sl < slots && r < r_end; ++sl, r += r_step) fetch(r, sl);
-    }
-    int slot = 0;
-    for (int r = r_first; r < r_end; r += r_step) {
-      mbar_wait(bar0 + 8u * slot, (phases >> slot) & 1u);
-      phases ^= 1u << slot;
-      float4 v[kVec];
-      load_row(v, ring + static_cast<uint32_t>(slot) * row_bytes, lane, nvec);
-      __syncwarp();  // (the loads above are volatile asm: they stay before this point)
-      const int r_next = r + slots * r_step;
-      if (lane == 0 && r_next < r_end) fetch(r_next, slot);
-      finish_row(v, r, D, e, lane, nvec);
-      if (++slot == slots) slot = 0;
-    }
-  }
-};
 
 // MN == false: A[M,K], B[N,K] with K contiguous (activations x nn.Linear weights).
 // MN == true : A[K,M], B[K,N] with M / N contiguous - the weight-gradient contraction
 //              dW[out,in] = sum_tokens dY[token,out] * X[token,in] reads both activations in place
 //              as MN-major tcgen05 operands (64x64 TMA boxes, LBO = 8 KB between 64-wide chunks).
 // The K range can be split across `num_splits` work items per tile (reduce-add epilogue).
-// LNF: fused LayerNorm tail (GemmEpilogue::ln_out), EPI_RESID_F32 with the TMA reduce-add epilogue.
-template <int BLOCK_N, int EPI, int CTAS, bool TMA_EPI, bool MN, bool LNF = false>
-__global__ void __launch_bounds__(LNF ? kNumThreadsLn : kNumThreads, 1)
+// `e` is __grid_constant__: its fields are read from parameter space where they are used, not
+// loaded into registers at the kernel's start.
+template <int BLOCK_N, int EPI, int CTAS, bool TMA_EPI, bool MN>
+__global__ void __launch_bounds__(kNumThreads, 1)
 gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
                const __grid_constant__ CUtensorMap tmap_b,
                const __grid_constant__ CUtensorMap tmap_c,
                const __grid_constant__ CUtensorMap tmap_c2, int M, int N, int K,
-               int kb_per_split, int num_splits, int descending, const GemmEpilogue e) {
+               int kb_per_split, int num_splits, int descending,
+               const __grid_constant__ GemmEpilogue e) {
   constexpr bool kAuxTma = TMA_EPI && (EPI == EPI_DGELU_BF16);
   constexpr bool kStats = TMA_EPI && (EPI == EPI_RESID_STATS_F32);
   static_assert(EPI != EPI_RESID_STATS_F32 || TMA_EPI, "the statistics epilogue is TMA-only");
-  using C = Cfg<BLOCK_N, CTAS, LNF ? 1 : (kAuxTma ? 3 : 2), LNF ? ln_ring_bytes(CTAS) : 0>;
+  using C = Cfg<BLOCK_N, CTAS, kAuxTma ? 3 : 2>;
   constexpr int kStagingBytes = C::kStagingBytes;
   constexpr int kStagingPerWarp = C::kStagingPerWarp;
   constexpr int kTileM = kBlockM * CTAS;  // rows of C per cluster tile
@@ -642,31 +504,18 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
   uint8_t* smem = smem_raw + (base - raw_addr);
 
   const uint32_t staging_base = base + C::kStages * C::kStageBytes;  // 1024-aligned
-  [[maybe_unused]] const uint32_t ln_ring_base = staging_base + kStagingBytes;
-  const uint32_t bar_base = staging_base + kStagingBytes + C::kLnRingBytes;
+  const uint32_t bar_base = staging_base + kStagingBytes;
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
   auto empty_bar = [&](int s) { return bar_base + 8u * (C::kStages + s); };
   auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * C::kStages + a); };
   auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * C::kStages + kAccStages + a); };
   volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(
-      smem + C::kStages * C::kStageBytes + kStagingBytes + C::kLnRingBytes +
-      8 * (2 * C::kStages + 2 * kAccStages));
+      smem + C::kStages * C::kStageBytes + kStagingBytes + 8 * (2 * C::kStages + 2 * kAccStages));
   auto aux_bar = [&](int w) { return bar_base + 8u * (2 * C::kStages + 2 * kAccStages + 1 + w); };
-  // LayerNorm job ring: row blocks whose last column tile this CTA completed
-  constexpr int kJobBar0 = 2 * C::kStages + 2 * kAccStages + 1 + kNumEpiWarps;
-  [[maybe_unused]] auto job_full = [&](int j) { return bar_base + 8u * (kJobBar0 + j); };
-  [[maybe_unused]] auto job_empty = [&](int j) { return bar_base + 8u * (kJobBar0 + kLnJobs + j); };
-  [[maybe_unused]] auto ln_row_bar = [&](int w, int sl) {
-    return bar_base + 8u * (kJobBar0 + 2 * kLnJobs + w * kLnSlots + sl);
-  };
   // second slab barrier of the statistics epilogue (the first is aux_bar)
   [[maybe_unused]] auto aux2_bar = [&](int w) {
-    return bar_base + 8u * (kJobBar0 + 2 * kLnJobs + kNumLnWarps * kLnSlots + w);
+    return bar_base + 8u * (2 * C::kStages + 2 * kAccStages + 1 + kNumEpiWarps + w);
   };
-  [[maybe_unused]] volatile int* ln_job = reinterpret_cast<volatile int*>(
-      smem + C::kStages * C::kStageBytes + kStagingBytes + C::kLnRingBytes + 8 * C::kNumBars);
-  [[maybe_unused]] int* ln_ticket = const_cast<int*>(ln_job) + kLnJobs;  // next ring position
-  [[maybe_unused]] int* ln_done = ln_ticket + 1;                         // epilogue warps finished
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -709,16 +558,6 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
       for (int w2 = 0; w2 < kNumEpiWarps; ++w2) mbar_init(aux_bar(w2), 1);
     if constexpr (kStats)
       for (int w2 = 0; w2 < kNumEpiWarps; ++w2) mbar_init(aux2_bar(w2), 1);
-    if constexpr (LNF) {
-      for (int j = 0; j < kLnJobs; ++j) {
-        mbar_init(job_full(j), 1);             // the epilogue lane that queued the job
-        mbar_init(job_empty(j), kNumLnWarps);  // every LayerNorm warp has read it
-      }
-      for (int w2 = 0; w2 < kNumLnWarps; ++w2)
-        for (int sl = 0; sl < kLnSlots; ++sl) mbar_init(ln_row_bar(w2, sl), 1);
-      *ln_ticket = 0;
-      *ln_done = 0;
-    }
     fence_mbar_init();
   }
   if (warp == 2) {
@@ -734,12 +573,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
   if constexpr (CTAS == 2) cluster_sync_all(); else __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // everything above overlapped the tail of the previous kernel; its results are needed from here
-  pdl_wait();
-  pdl_launch_dependents();
 
-  if (warp < kFirstEpiWarp) {
-  if constexpr (LNF) setmaxnreg_dec<40>();
   if (warp == 0) {
     // ======================= TMA producer (every CTA stages its own operand slices) ==========
     if (lane == 0) {
@@ -876,10 +710,8 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
       }
 #endif
     }
-  }
-  } else if (warp < kFirstEpiWarp + kNumEpiWarps) {
+  } else if (warp >= kFirstEpiWarp) {
     // ======================= epilogue =======================
-    if constexpr (LNF) setmaxnreg_inc<128>();
     const int q = warp & 3;                        // TMEM lane quarter this warp may access
     const int half = (warp - kFirstEpiWarp) >> 2;  // which half of the tile's columns
     constexpr int kColsPerWarp = BLOCK_N / 2;
@@ -893,28 +725,6 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
     [[maybe_unused]] const uint32_t my_aux_bar = aux_bar(warp - kFirstEpiWarp);
     [[maybe_unused]] const uint32_t my_aux2_bar = aux2_bar(warp - kFirstEpiWarp);
     [[maybe_unused]] uint32_t x_phase = 0;  // statistics epilogue: parity bit per slab
-    // ---- fused LayerNorm tail: bookkeeping done by lane 0 of every epilogue warp
-    // queue a 128-row block (or the -1 sentinel) for this CTA's LayerNorm warps
-    [[maybe_unused]] auto ln_push = [&](int blk) {
-      const int ticket = atomicAdd(ln_ticket, 1);
-      const int slot = ticket % kLnJobs;
-      mbar_wait(job_empty(slot), (static_cast<uint32_t>(ticket / kLnJobs) & 1u) ^ 1u);
-      ln_job[slot] = blk;
-      mbar_arrive(job_full(slot));
-    };
-    // this warp's reduce-adds of its previous tile have landed: count them; whoever completes the
-    // count of a 128-row block (all column tiles x all epilogue warps, across CTAs) owns its LN
-    [[maybe_unused]] auto ln_signal = [&](int blk) {
-      asm volatile("fence.proxy.async.global;" ::: "memory");
-      unsigned int old;
-      asm volatile("atom.add.acq_rel.gpu.global.u32 %0, [%1], 1;"
-                   : "=r"(old) : "l"(e.ln_counters + blk) : "memory");
-      if (old + 1u == static_cast<unsigned int>(num_n_tiles * kNumEpiWarps)) {
-        e.ln_counters[blk] = 0u;  // left zero-filled for the next launch
-        ln_push(blk);
-      }
-    };
-    [[maybe_unused]] int ln_pending = -1;
     [[maybe_unused]] long long gt_epi_wait = 0, gt_epi_ld = 0, gt_epi_math = 0, gt_epi_store = 0;
     // folded LayerNorm (consumer side): partial sums of the next tile's row, in flight
     [[maybe_unused]] float2 ln_next[8];
@@ -998,7 +808,6 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
       mbar_wait(tfull_bar(acc), acc_phase);
       GT_ADD(gt_epi_wait, gt_w);
       tc_fence_after();
-      [[maybe_unused]] int ln_commits = 0;  // bulk groups this warp commits for this tile
       const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) +
                              static_cast<uint32_t>(acc * BLOCK_N + half * kColsPerWarp);
       const int n_base = n_blk * BLOCK_N + half * kColsPerWarp;
@@ -1131,8 +940,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
               uint32_t pk[32];
 #pragma unroll
               for (int j = 0; j < 32; ++j) pk[j] = __float_as_uint(x[j]);
-              stage_and_store<LNF ? 1 : 2>(pk, stg, buf, lane, &tmap_c, n0, row0, reduce);
-              if constexpr (LNF) ++ln_commits;
+              stage_and_store(pk, stg, buf, lane, &tmap_c, n0, row0, reduce);
             }
           }
         } else {
@@ -1271,17 +1079,6 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
           ln_rstd_next = ln_finish(s1, s2);
         }
       }
-      if constexpr (LNF) {
-        // The PREVIOUS tile's reductions had this whole tile's epilogue to land: waiting for all
-        // but the groups committed since does not stall (waiting for this tile's own would expose
-        // the write latency once per tile).
-        if (lane == 0 && ln_pending >= 0) {
-          if (ln_commits == kColsPerWarp / 32) tma_store_wait<kColsPerWarp / 32>();
-          else tma_store_wait<0>();
-          ln_signal(ln_pending);
-        }
-        ln_pending = m_blk * CTAS + static_cast<int>(cta_rank);
-      }
     }
 #ifdef VITK_GEMM_TRACE
     if (lane == 0 && warp == kFirstEpiWarp && is_leader && cluster_id < 160) {
@@ -1293,45 +1090,6 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
 #endif
     if constexpr (TMA_EPI) {
       if (lane == 0) tma_store_wait<0>();  // all bulk stores of this warp have completed
-    }
-    if constexpr (LNF) {
-      if (lane == 0) {
-        if (ln_pending >= 0) ln_signal(ln_pending);
-        // the last epilogue warp to finish closes the ring: no further row block can complete here
-        if (atomicAdd(ln_done, 1) == kNumEpiWarps - 1) ln_push(-1);
-      }
-    }
-  } else if (LNF && warp >= kFirstLnWarp) {
-    // ======================= LayerNorm tail =======================
-    setmaxnreg_dec<88>();
-
-    const int lw = warp - kFirstLnWarp;
-    const float* xs = reinterpret_cast<const float*>(e.out);
-    constexpr uint32_t kRingPerWarp = C::kLnRingBytes / kNumLnWarps;
-    const uint32_t ring = ln_ring_base + static_cast<uint32_t>(lw) * kRingPerWarp;
-    int slots = static_cast<int>(kRingPerWarp / (static_cast<uint32_t>(N) * 4u));
-    if (slots > kLnSlots) slots = kLnSlots;  // (>= 1: the ring holds a 1024-float row per warp)
-    uint32_t phases = 0;
-    for (int j = 0;; ++j) {
-      const int slot = j % kLnJobs;
-      mbar_wait(job_full(slot), static_cast<uint32_t>(j / kLnJobs) & 1u);
-      const int blk = ln_job[slot];
-      __syncwarp();
-      if (lane == 0) mbar_arrive(job_empty(slot));
-      if (blk < 0) break;
-      // the rows were written by other SMs' bulk reductions and published through the counter:
-      // order that acquisition before this warp's own async-proxy reads
-      asm volatile("fence.proxy.async;" ::: "memory");
-      // rows of the block interleaved over the warps
-      const int r0 = blk * kBlockM + lw;
-      int r1 = (blk + 1) * kBlockM;
-      if (r1 > M) r1 = M;
-      if (N == 768)
-        LnTail<6>::rows(xs, e.ldo, r0, r1, kNumLnWarps, N, e, lane, ring, ln_row_bar(lw, 0), slots, phases);
-      else if (N == 1024)
-        LnTail<8>::rows(xs, e.ldo, r0, r1, kNumLnWarps, N, e, lane, ring, ln_row_bar(lw, 0), slots, phases);
-      else
-        LnTail<0>::rows(xs, e.ldo, r0, r1, kNumLnWarps, N, e, lane, ring, ln_row_bar(lw, 0), slots, phases);
     }
   }
 
@@ -1346,18 +1104,11 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
 
 int g_force_ctas = 0;        // 0 = auto, 1 / 2 = forced (tests, A/B timing)
 int g_force_direct_epi = 0;  // 1 = never use the TMA-store epilogue (tests, A/B timing)
-// LayerNorm after a residual GEMM: 0 = a separate layernorm_fwd launch (default: measured faster,
-// see the note at kNumLnWarps), 1 = the in-kernel tail.  VITK_FUSED_LN=1 / gemm_set_fused_layernorm.
-int g_fused_ln = [] {
-  const char* v = getenv("VITK_FUSED_LN");
-  return (v != nullptr && v[0] == '1') ? 1 : 0;
-}();
 
-template <int BLOCK_N, int EPI, int CTAS, bool TMA_EPI, bool MN, bool LNF = false>
+template <int BLOCK_N, int EPI, int CTAS, bool TMA_EPI, bool MN>
 int launch(const GemmProblem& p, cudaStream_t stream) {
-  using C = Cfg<BLOCK_N, CTAS, LNF ? 1 : ((TMA_EPI && EPI == EPI_DGELU_BF16) ? 3 : 2),
-                LNF ? ln_ring_bytes(CTAS) : 0>;
-  auto kernel = gemm_tn_kernel<BLOCK_N, EPI, CTAS, TMA_EPI, MN, LNF>;
+  using C = Cfg<BLOCK_N, CTAS, (TMA_EPI && EPI == EPI_DGELU_BF16) ? 3 : 2>;
+  auto kernel = gemm_tn_kernel<BLOCK_N, EPI, CTAS, TMA_EPI, MN>;
   static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;
   std::call_once(once, [&] {
@@ -1407,25 +1158,23 @@ int launch(const GemmProblem& p, cudaStream_t stream) {
   if (num_tiles * CTAS < grid) grid = num_tiles * CTAS;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(LNF ? kNumThreadsLn : kNumThreads);
+  cfg.blockDim = dim3(kNumThreads);
   cfg.dynamicSmemBytes = C::kSmemBytes;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CTAS;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = CTAS;
+  attr.val.clusterDim.y = 1;
+  attr.val.clusterDim.z = 1;
+  cfg.attrs = &attr;
+  cfg.numAttrs = 1;
   ProfileScope prof(PROF_GEMM, 2.0 * p.M * p.N * p.K, stream);
   const int descending = sweep_next();
   cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, ta, tb, tc, tc2, p.M, p.N, p.K, kb_per_split,
                                       splits, descending, p.e);
   if (le != cudaSuccess)
     return set_error(VITK_ERR_CUDA, "launch of gemm_tn_kernel<%d,%d,%d,%d,%d> failed: %s", BLOCK_N,
-                     EPI, CTAS, (int)TMA_EPI, (int)LNF, cudaGetErrorString(le));
+                     EPI, CTAS, (int)TMA_EPI, (int)MN, cudaGetErrorString(le));
   VITK_CHECK_LAUNCH("gemm_tn_kernel");
   return VITK_OK;
 }
@@ -1472,20 +1221,6 @@ bool tma_epilogue_ok(const GemmProblem& p, bool honour_force = true) {
   }
 }
 
-// x += A W^T + b with the LayerNorm of the updated rows in the same launch (GemmEpilogue::ln_out).
-int dispatch_resid_ln(const GemmProblem& p, cudaStream_t stream) {
-  const int waste256 = ((p.N + 255) / 256) * 256 - p.N;
-  const int waste128 = ((p.N + 127) / 128) * 128 - p.N;
-  const bool n128 = waste128 < waste256;
-  int ctas = (p.M > kBlockM) ? 2 : 1;
-  if (g_force_ctas == 1 || g_force_ctas == 2) ctas = g_force_ctas;
-  if (ctas == 2)
-    return n128 ? launch<128, EPI_RESID_F32, 2, true, false, true>(p, stream)
-                : launch<256, EPI_RESID_F32, 2, true, false, true>(p, stream);
-  return n128 ? launch<128, EPI_RESID_F32, 1, true, false, true>(p, stream)
-              : launch<256, EPI_RESID_F32, 1, true, false, true>(p, stream);
-}
-
 template <int EPI>
 int dispatch(const GemmProblem& p, cudaStream_t stream) {
   if constexpr (EPI == EPI_DGELU_BF16) {
@@ -1522,7 +1257,6 @@ int gemm_debug_trace(long long* out, int n) {
 }
 void gemm_force_cta_group(int ctas) { g_force_ctas = ctas; }
 void gemm_force_direct_epilogue(int on) { g_force_direct_epi = on; }
-void gemm_set_fused_layernorm(int on) { g_fused_ln = on; }
 int gemm_stats_parts(int N) {
   // as dispatch_tile: 256-wide tiles unless they waste more than 128-wide ones; an epilogue warp
   // owns half a tile's columns
@@ -1578,21 +1312,6 @@ int gemm_bf16_tn(const GemmProblem& p, cudaStream_t stream) {
     case EPI_RELU_BF16: return dispatch<EPI_RELU_BF16>(p, stream);
     case EPI_RESID_F32:
       VITK_REQUIRE(p.e.resid != nullptr && p.e.ldr % 4 == 0, "gemm: residual epilogue needs resid");
-      if (p.e.ln_out != nullptr) {
-        VITK_REQUIRE(p.e.ln_gamma && p.e.ln_beta && p.e.rows_per_group == 0 && p.e.ldo == p.N &&
-                         p.e.ln_ldo % 4 == 0 && p.N % 4 == 0 && p.N <= 128 * kLnMaxVec,
-                     "gemm: LayerNorm tail needs gamma/beta, dense rows of at most %d features and "
-                     "no row remap", 128 * kLnMaxVec);
-        if (g_fused_ln && p.e.ln_counters != nullptr && tma_epilogue_ok(p))
-          return dispatch_resid_ln(p, stream);
-        // not expressible as the in-place TMA form: the same result in two launches
-        GemmProblem q = p;
-        q.e.ln_out = nullptr;
-        VITK_TRY(dispatch<EPI_RESID_F32>(q, stream));
-        return layernorm_fwd(static_cast<const float*>(p.e.out), p.e.ldo, p.e.ln_gamma, p.e.ln_beta,
-                             p.e.ln_out, 0, p.e.ln_ldo, p.e.ln_mean, p.e.ln_rstd, p.M, p.N,
-                             p.e.ln_eps, stream, p.e.ln_xcopy);
-      }
       return dispatch<EPI_RESID_F32>(p, stream);
     case EPI_F32: return dispatch<EPI_F32>(p, stream);
     case EPI_DGELU_BF16:

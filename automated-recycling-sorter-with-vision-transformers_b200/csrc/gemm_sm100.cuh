@@ -45,24 +45,6 @@ struct GemmEpilogue {
   //   EPI_GELU_*   : out = dropout(gelu(acc + bias))     (out2 keeps the undropped pre-activation)
   //   EPI_DGELU    : out = dropout_mask(acc) * gelu'(aux) (the backward of the above)
   DropParams drop;
-  // LayerNorm of the updated rows (EPI_RESID_F32; reference train.py:586-591: x = x + f(..);
-  // LN(x) feeds the next Linear): ln_out = LN(out) * ln_gamma + ln_beta as bf16.  By default a
-  // layernorm_fwd launch behind the GEMM.  With gemm_set_fused_layernorm(1), the in-place TMA
-  // reduce-add form and ln_counters != nullptr, one launch: every epilogue warp counts its
-  // finished column tile of a 128-row block in ln_counters[row / 128]; the CTA that completes the
-  // count fetches those rows of `out` (still L2-resident) into shared memory by bulk copies and
-  // its LayerNorm warps normalise them.  Same arithmetic, lane for lane, as layernorm_fwd_kernel:
-  // both forms produce the same bits.  ln_out == nullptr: no LayerNorm.
-  // ln_counters: zero-filled uint32[ceil(M / 128)], left zero-filled.
-  void* ln_out = nullptr;         // bf16 [M, ln_ldo]
-  const float* ln_gamma = nullptr;
-  const float* ln_beta = nullptr;
-  float* ln_mean = nullptr;       // optional [M]
-  float* ln_rstd = nullptr;       // optional [M]
-  float* ln_xcopy = nullptr;      // optional fp32 [M, N] copy of the updated rows (saved for backward)
-  unsigned int* ln_counters = nullptr;
-  int ln_ldo = 0;
-  float ln_eps = 1e-5f;
   // ---- LayerNorm folded into the two GEMMs around it (inference; DESIGN.md 3.9).
   // Producer (EPI_RESID_STATS_F32): every epilogue thread owns a row and 128 (BLOCK_N / 2) of its
   // columns, so the partial sums need no exchange: ln_part_out[(column group) * M + row] =
@@ -77,6 +59,7 @@ struct GemmEpilogue {
   const float2* ln_part = nullptr;
   int ln_nparts = 0;
   int ln_dim = 0;
+  float ln_eps = 1e-5f;
 };
 
 struct GemmProblem {
@@ -105,7 +88,4 @@ void gemm_force_direct_epilogue(int on);
 int gemm_debug_trace(long long* out, int n);
 // Column groups per row of EPI_RESID_STATS_F32's partial sums for an N-column output.
 int gemm_stats_parts(int N);
-// GemmEpilogue::ln_out: 0 (default) = residual GEMM, then a separate layernorm_fwd launch;
-// 1 = the LayerNorm tail inside the GEMM kernel.  Same bits either way.
-void gemm_set_fused_layernorm(int on);
 }  // namespace vitk

@@ -34,17 +34,6 @@ __device__ __forceinline__ bool elect_one_sync() {
   return pred != 0;
 }
 
-// Programmatic dependent launch (PDL): a kernel launched with the programmatic-serialization
-// attribute (common.h: launch_pdl) may start while its predecessor in the stream is still running;
-// pdl_wait() blocks until the predecessor grid has completed and its memory is visible, so a
-// kernel runs its prologue (barrier init, TMEM allocation, descriptor prefetch) early and calls
-// pdl_wait() before it first touches global memory.  pdl_launch_dependents() lets the successor
-// be scheduled before this grid has finished.  Both are no-ops for ordinary launches.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() {
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
 // Per-warpgroup register budget (all four warps of the warpgroup execute the same instruction).
 template <int REGS>
 __device__ __forceinline__ void setmaxnreg_inc() {
@@ -120,15 +109,6 @@ __device__ __forceinline__ void tma_load_2d_hint(uint32_t dst_smem, const void* 
       :
       : "r"(dst_smem), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar), "r"(c0), "r"(c1),
         "l"(hint)
-      : "memory");
-}
-// 1-D bulk copy global -> shared (16-byte aligned, size a multiple of 16), completion on an mbarrier.
-__device__ __forceinline__ void bulk_load_1d(uint32_t dst_smem, const void* src, uint32_t bytes,
-                                             uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      :
-      : "r"(dst_smem), "l"(reinterpret_cast<uint64_t>(src)), "r"(bytes), "r"(bar)
       : "memory");
 }
 // 2-D tiled store shared -> global (bulk async group).

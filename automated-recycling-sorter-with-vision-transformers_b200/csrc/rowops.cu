@@ -46,8 +46,6 @@ layernorm_fwd_kernel(const float* __restrict__ x, long long in_stride,
                      float eps, int descending) {
   int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  pdl_wait();
-  pdl_launch_dependents();
   if (warp >= rows) return;
   if (descending) warp = rows - 1 - warp;  // blocks are scheduled in index order
   const float* xr = x + static_cast<long long>(warp) * in_stride;
@@ -271,8 +269,6 @@ row_stats_kernel(const float* __restrict__ x, long long in_stride, __nv_bfloat16
                  long long out_stride, float2* __restrict__ part, int rows, int D, int descending) {
   int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  pdl_wait();
-  pdl_launch_dependents();
   if (warp >= rows) return;
   if (descending) warp = rows - 1 - warp;
   const float* xr = x + static_cast<long long>(warp) * in_stride;
@@ -354,13 +350,13 @@ int layernorm_fwd(const float* x, long long in_stride, const float* gamma, const
   ProfileScope prof(PROF_LN, static_cast<double>(rows) * D * (4.0 + (y_is_f32 ? 4.0 : 2.0)), stream);
   const int descending = sweep_next();
   if (y_is_f32)
-    launch_pdl(layernorm_fwd_kernel<float>, dim3(grid), dim3(block), 0, stream, x, in_stride, gamma,
-               beta, static_cast<float*>(y), out_stride, mean_out, rstd_out, x_copy, rows, D, eps,
-               descending);
+    layernorm_fwd_kernel<float><<<grid, block, 0, stream>>>(
+        x, in_stride, gamma, beta, static_cast<float*>(y), out_stride, mean_out, rstd_out, x_copy,
+        rows, D, eps, descending);
   else
-    launch_pdl(layernorm_fwd_kernel<__nv_bfloat16>, dim3(grid), dim3(block), 0, stream, x, in_stride,
-               gamma, beta, static_cast<__nv_bfloat16*>(y), out_stride, mean_out, rstd_out, x_copy,
-               rows, D, eps, descending);
+    layernorm_fwd_kernel<__nv_bfloat16><<<grid, block, 0, stream>>>(
+        x, in_stride, gamma, beta, static_cast<__nv_bfloat16*>(y), out_stride, mean_out, rstd_out,
+        x_copy, rows, D, eps, descending);
   VITK_CHECK_LAUNCH("layernorm_fwd_kernel");
   return VITK_OK;
 }
@@ -373,8 +369,8 @@ int row_stats(const float* x, long long in_stride, void* y_bf16, long long out_s
   VITK_REQUIRE(in_stride % 4 == 0 && out_stride % 4 == 0, "row_stats: strides must be multiples of 4");
   ProfileScope prof(PROF_LN, static_cast<double>(rows) * D * 6.0, stream);
   const int descending = sweep_next();
-  launch_pdl(row_stats_kernel, dim3((rows + 7) / 8), dim3(256), 0, stream, x, in_stride,
-             static_cast<__nv_bfloat16*>(y_bf16), out_stride, part, rows, D, descending);
+  row_stats_kernel<<<(rows + 7) / 8, 256, 0, stream>>>(
+      x, in_stride, static_cast<__nv_bfloat16*>(y_bf16), out_stride, part, rows, D, descending);
   VITK_CHECK_LAUNCH("row_stats_kernel");
   return VITK_OK;
 }

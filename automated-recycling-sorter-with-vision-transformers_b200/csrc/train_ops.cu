@@ -7,8 +7,6 @@
 
 #include <cuda_bf16.h>
 
-#include <cstdlib>
-
 #include "common.h"
 #include "ptx.cuh"
 
@@ -152,8 +150,6 @@ layernorm_bwd_fused_kernel(const DyT* __restrict__ dy, long long dy_stride,
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long gw = static_cast<long long>(blockIdx.x) * 8 + warp;
   const long long W = static_cast<long long>(gridDim.x) * 8;
-  pdl_wait();
-  pdl_launch_dependents();
   const float inv_d = 1.f / static_cast<float>(D);
   using RV = RawVec<DyT>;
   float4 ag[NVEC], ab[NVEC];
@@ -818,16 +814,16 @@ int layernorm_bwd(const void* dy, int dy_is_f32, long long dy_stride, const floa
   VITK_REQUIRE(!dropping || (dx_bf16 != nullptr && dxb_stride == D &&
                              static_cast<long long>(rows) * D < (1ll << 32)),
                "layernorm_bwd: the dropout mask applies to a dense bf16 output");
-  if (dgamma != nullptr && nv <= 6 && (dropping || std::getenv("VITK_LN_BWD_SPLIT") == nullptr)) {
+  if (dgamma != nullptr && nv <= 6) {
     // one pass: dx and the parameter gradients together
     ProfileScope prof(PROF_LN, static_cast<double>(rows) * D * (dy_is_f32 ? 14.0 : 12.0), stream);
     int fgrid = sm_count() * 2;
     if (fgrid > (rows + 7) / 8) fgrid = (rows + 7) / 8;
     __nv_bfloat16* dxb = static_cast<__nv_bfloat16*>(dx_bf16);
 #define VITK_LN_FUSED(T, PTR, NV)                                                                 \
-  launch_pdl(layernorm_bwd_fused_kernel<T, NV>, dim3(fgrid), dim3(block), 0, stream, PTR, dy_stride, \
-             x, x_stride, mean, rstd, gamma, dx_io, dx_stride, add_resid, dxb, dxb_stride, dgamma,  \
-             dbeta, dx_colsum, rows, D, dp)
+  layernorm_bwd_fused_kernel<T, NV><<<fgrid, block, 0, stream>>>(                                 \
+      PTR, dy_stride, x, x_stride, mean, rstd, gamma, dx_io, dx_stride, add_resid, dxb, dxb_stride, \
+      dgamma, dbeta, dx_colsum, rows, D, dp)
     if (dy_is_f32) {
       if (nv <= 2) VITK_LN_FUSED(float, dyf, 2);
       else if (nv <= 4) VITK_LN_FUSED(float, dyf, 4);

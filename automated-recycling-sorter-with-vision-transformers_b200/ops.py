@@ -70,8 +70,8 @@ def gemm(a: torch.Tensor, b: torch.Tensor, epilogue: int = _lib.EPI_BF16, *, bia
 
 def gemm_resid_layernorm(a: torch.Tensor, w: torch.Tensor, x: torch.Tensor, gamma: torch.Tensor,
                          beta: torch.Tensor, *, bias=None, eps: float = 1e-5,
-                         return_stats: bool = False, counters: torch.Tensor | None = None):
-    """x += a @ w.T + bias (in place, fp32) and LN(x) * gamma + beta as bf16, one launch
+                         return_stats: bool = False):
+    """x += a @ w.T + bias (in place, fp32) and LN(x) * gamma + beta as bf16, two launches
     (train.py:586-591).  Returns the bf16 LayerNorm output (and mean / rstd)."""
     _need_cuda(a, w, x)
     assert a.dtype == torch.bfloat16 and w.dtype == torch.bfloat16 and x.dtype == torch.float32
@@ -84,12 +84,10 @@ def gemm_resid_layernorm(a: torch.Tensor, w: torch.Tensor, x: torch.Tensor, gamm
     if return_stats:
         mean = torch.empty(M, dtype=torch.float32, device=x.device)
         rstd = torch.empty(M, dtype=torch.float32, device=x.device)
-    if counters is None:  # zero-filled scratch, handed back zero-filled
-        counters = torch.zeros((M + 127) // 128, dtype=torch.int32, device=x.device)
     check(lib().vitk_gemm_resid_layernorm(a.data_ptr(), a.stride(0), w.data_ptr(), w.stride(0), M,
                                           N, K, _ptr(bias), x.data_ptr(), gamma.data_ptr(),
                                           beta.data_ptr(), eps, y.data_ptr(), _ptr(mean),
-                                          _ptr(rstd), counters.data_ptr(), _stream()))
+                                          _ptr(rstd), _stream()))
     return (y, mean, rstd) if return_stats else y
 
 

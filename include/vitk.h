@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define VITK_ABI_VERSION 5
+#define VITK_ABI_VERSION 6
 
 #define VITK_OK 0
 #define VITK_ERR_INVALID 1
@@ -121,11 +121,6 @@ int vitk_gemm_set_direct_epilogue(int on);
  * [pair][{total, wait operands, wait accumulator, tiles}] of the last GEMM launch to HOST memory
  * (n entries).  Returns the entries written; 0 in a normal build. */
 int vitk_debug_gemm_trace(long long* out_host, int n);
-/* LayerNorm after a residual GEMM (vitk_gemm_resid_layernorm and the encoder's projection /
- * linear2 launches): 0 (default) = a separate LayerNorm launch, 1 = LayerNorm warps inside the
- * GEMM kernel (one launch; measured slower on B200, kept for A/B - DESIGN.md section 6).  Same
- * bits either way.  Initial value from the environment variable VITK_FUSED_LN. */
-int vitk_gemm_set_fused_layernorm(int on);
 /* vitk_forward with VitkBlockWeights::*_ln set: 1 (default) = LayerNorm folded into the GEMMs
  * around it, 0 = separate LayerNorm launches (A/B timing, tests).  Initial value from the
  * environment variable VITK_LN_FOLD. */
@@ -171,9 +166,6 @@ int vitk_linear_rows_backward(const float* x, long long row_stride, const float*
 /* Persistent kernels (GEMM, attention) launch one CTA per SM; keep `n` SMs out of their grids, e.g.
  * for the NCCL kernels of a gradient all-reduce that overlaps the backward pass. 0 restores all. */
 int vitk_reserve_sms(int n);
-/* Programmatic dependent launch of the library's kernels (off by default; VITK_PDL=1 or
- * vitk_set_pdl(1) turns it on; measured neutral on B200, tests/ab_pdl.py). */
-int vitk_set_pdl(int on);
 
 /* Attention kernel choice: 0 = automatic (tcgen05 single-key-block kernel when N <= 256, else the
  * flash kernel), 1 = flash (mma.sync, any N), 2 = tcgen05.  Tests and A/B timing. */
@@ -228,16 +220,12 @@ int vitk_gemm(const void* A, int lda, const void* B, int ldb, int M, int N, int 
 
 /* Residual update and the LayerNorm that follows it (train.py:586-591: x = x + f(..), then
  * layer_norm(x) feeds the next Linear): x[M,N] f32 += A[M,K] W[N,K]^T + bias (TMA reduce-add
- * epilogue) and ln_out bf16 [M,N] = LN(x) * gamma + beta (optionally mean / rstd f32 [M]).
- * Two launches by default; with vitk_gemm_set_fused_layernorm(1) one: as soon as all column
- * tiles of a 128-row block have landed, LayerNorm warps of the GEMM kernel fetch those rows from
- * L2 by bulk copies and normalise them.  counters: zero-filled uint32[ceil(M/128)] scratch for
- * the fused form, returned zero-filled (may be null: then always two launches).  Bit-identical
- * to vitk_gemm(VITK_EPI_RESID_F32) followed by vitk_layernorm in both forms. */
+ * epilogue) and ln_out bf16 [M,N] = LN(x) * gamma + beta (optionally mean / rstd f32 [M]), N <= 1024.
+ * Two launches: vitk_gemm(VITK_EPI_RESID_F32) followed by vitk_layernorm, with the same bits. */
 int vitk_gemm_resid_layernorm(const void* A, int lda, const void* W, int ldb, int M, int N, int K,
                               const float* bias, float* x_inout, const float* gamma,
                               const float* beta, float eps, void* ln_out, float* mean_out,
-                              float* rstd_out, unsigned int* counters, vitk_stream_t stream);
+                              float* rstd_out, vitk_stream_t stream);
 
 /* ---- LayerNorm folded into the two GEMMs around it (train.py:584-591: x = x + f(..);
  * Linear(layer_norm(x))).  Instead of a LayerNorm pass over the fp32 residual stream between two

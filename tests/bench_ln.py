@@ -1,7 +1,6 @@
-"""Not a pytest file: device-timed LayerNorm forward / backward (fused vs split) at the encoder's shapes.
+"""Not a pytest file: device-timed LayerNorm forward / backward at the encoder's shapes.
     python tests/bench_ln.py [batch]
 """
-import os
 import sys
 from pathlib import Path
 
@@ -38,12 +37,9 @@ ms = timeit(lambda: vitk.ops.layernorm(x, g, bta))
 print(f"layernorm fwd  rows={M}: {ms*1e3:7.1f} us  {M*D*6/ms/1e6:7.0f} GB/s")
 dx = torch.randn(M, D, device="cuda")
 dgam, dbet = torch.zeros(D, device="cuda"), torch.zeros(D, device="cuda")
-for mode in ("fused", "split"):
-    if mode == "split":
-        os.environ["VITK_LN_BWD_SPLIT"] = "1"
-    dxb = torch.empty(M, D, device="cuda", dtype=torch.bfloat16)
-    st = torch.cuda.current_stream().cuda_stream
-    ms = timeit(lambda: vitk._lib.check(vitk._lib.lib().vitk_layernorm_bwd(
-        dy.data_ptr(), 0, x.data_ptr(), mean.data_ptr(), rstd.data_ptr(), g.data_ptr(), dx.data_ptr(), 1,
-        dxb.data_ptr(), dgam.data_ptr(), dbet.data_ptr(), M, D, st)))
-    print(f"layernorm bwd {mode} rows={M}: {ms*1e3:7.1f} us  {M*D*16/ms/1e6:7.0f} GB/s (algorithmic 16 B/elem)")
+dxb = torch.empty(M, D, device="cuda", dtype=torch.bfloat16)
+st = torch.cuda.current_stream().cuda_stream
+ms = timeit(lambda: vitk._lib.check(vitk._lib.lib().vitk_layernorm_bwd(
+    dy.data_ptr(), 0, x.data_ptr(), mean.data_ptr(), rstd.data_ptr(), g.data_ptr(), dx.data_ptr(), 1,
+    dxb.data_ptr(), dgam.data_ptr(), dbet.data_ptr(), M, D, st)))
+print(f"layernorm bwd rows={M}: {ms*1e3:7.1f} us  {M*D*16/ms/1e6:7.0f} GB/s (algorithmic 16 B/elem)")

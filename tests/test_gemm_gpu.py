@@ -140,7 +140,7 @@ def test_gemm_wgrad_mn_major(vitk, T, O, I, split):
     torch.testing.assert_close(out2, 1.5 * ref, rtol=2e-4, atol=3e-3 * (T / 256) ** 0.5)
 
 
-# ---- residual GEMM with the fused LayerNorm tail (train.py:586-591) --------------------------
+# ---- residual GEMM followed by its LayerNorm (train.py:586-591) ------------------------------
 LN_SHAPES = [
     (15, 64, 64),          # tiny model of the smoke test: one partial row block, BLOCK_N = 128
     (128, 256, 256),       # exactly one row block
@@ -149,13 +149,14 @@ LN_SHAPES = [
     (197 * 8, 768, 3072),  # linear2 of ViT-B/16
     (197 * 4, 1024, 1024),  # ViT-L width: four column tiles, 8 float4 per lane
     (129, 768, 768),       # second CTA of the pair owns a single row
+    (197 * 256, 768, 768),  # configs[1] geometry: every CTA pair covers several row blocks
 ]
 
 
 @pytest.mark.parametrize("M,N,K", LN_SHAPES)
-def test_gemm_resid_layernorm_matches_two_launches(vitk, M, N, K, gemm_mode):
-    """One launch (GEMM + LayerNorm tail) == vitk_gemm(RESID_F32) followed by vitk_layernorm, bit
-    for bit, and both match fp32 PyTorch; the arrival counters come back zero-filled."""
+def test_gemm_resid_layernorm_matches_gemm_then_layernorm(vitk, M, N, K, gemm_mode):
+    """vitk_gemm_resid_layernorm == vitk_gemm(RESID_F32) followed by vitk_layernorm, bit for bit,
+    and both match fp32 PyTorch."""
     a, w, bias = _mk(M, N, K, seed=7)
     g = torch.Generator(device="cuda").manual_seed(8)
     x0 = torch.randn(M, N, generator=g, device="cuda")
@@ -166,19 +167,11 @@ def test_gemm_resid_layernorm_matches_two_launches(vitk, M, N, K, gemm_mode):
     vitk.ops.gemm(a, w, vitk._lib.EPI_RESID_F32, bias=bias, resid=x_ref, out=x_ref)
     y_ref, mean_ref, rstd_ref = vitk.ops.layernorm(x_ref, gamma, beta, return_stats=True)
 
-    vitk._lib.set_gemm_fused_layernorm(True)
-    for rep in range(2):  # the second call reuses the counters the first one handed back
-        x = x0.clone()
-        counters = torch.zeros((M + 127) // 128, dtype=torch.int32, device="cuda") if rep == 0 \
-            else counters
-        y, mean, rstd = vitk.ops.gemm_resid_layernorm(a, w, x, gamma, beta, bias=bias,
-                                                      return_stats=True, counters=counters)
-        torch.cuda.synchronize()
-        assert int(counters.abs().sum()) == 0
-        assert torch.equal(x, x_ref)
-        assert torch.equal(y, y_ref)
-        assert torch.equal(mean, mean_ref) and torch.equal(rstd, rstd_ref)
-    vitk._lib.set_gemm_fused_layernorm(False)
+    x = x0.clone()
+    y, mean, rstd = vitk.ops.gemm_resid_layernorm(a, w, x, gamma, beta, bias=bias, return_stats=True)
+    assert torch.equal(x, x_ref)
+    assert torch.equal(y, y_ref)
+    assert torch.equal(mean, mean_ref) and torch.equal(rstd, rstd_ref)
 
     xt = x0 + _ref(a, w) + bias
     torch.testing.assert_close(x, xt, rtol=1e-4, atol=2e-4)
@@ -186,23 +179,3 @@ def test_gemm_resid_layernorm_matches_two_launches(vitk, M, N, K, gemm_mode):
     torch.testing.assert_close(y.float(), yt, rtol=1e-2, atol=2e-2)
 
 
-def test_gemm_resid_layernorm_full_batch(vitk):
-    """configs[1] geometry (50 432 rows): every CTA pair completes several row blocks; the fused
-    and the two-launch forms give the same bits."""
-    vitk._lib.set_gemm_cta_group(0)
-    vitk._lib.set_gemm_direct_epilogue(False)
-    M, N, K = 197 * 256, 768, 768
-    a, w, bias = _mk(M, N, K, seed=9)
-    g = torch.Generator(device="cuda").manual_seed(10)
-    x0 = torch.randn(M, N, generator=g, device="cuda")
-    gamma = 1.0 + 0.1 * torch.randn(N, generator=g, device="cuda")
-    beta = 0.1 * torch.randn(N, generator=g, device="cuda")
-    outs = []
-    for fused in (False, True, True):
-        vitk._lib.set_gemm_fused_layernorm(fused)
-        x = x0.clone()
-        y = vitk.ops.gemm_resid_layernorm(a, w, x, gamma, beta, bias=bias)
-        outs.append((x, y))
-    vitk._lib.set_gemm_fused_layernorm(False)
-    for x, y in outs[1:]:
-        assert torch.equal(x, outs[0][0]) and torch.equal(y, outs[0][1])
