@@ -7,53 +7,13 @@
 #include <cstdlib>
 
 #include "common.h"
+#include "encoder.cuh"
 #include "fp32_mode.cuh"
 #include "gemm_sm100.cuh"
 #include "rowops.cuh"
 
 namespace vitk {
 namespace {
-
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-struct Dims {
-  int B, S, p, C, D, L, H, Mlp, prefix, P, N, Kp, hd;
-  long long M, Mp;
-};
-
-int check_config(const VitkConfig* cfg, int batch, Dims* d) {
-  VITK_REQUIRE(cfg != nullptr, "config is null");
-  VITK_REQUIRE(batch > 0, "batch must be positive (got %d)", batch);
-  VITK_REQUIRE(cfg->image_size > 0 && cfg->patch_size > 0 &&
-                   cfg->image_size % cfg->patch_size == 0,
-               "image_size %d must be a positive multiple of patch_size %d", cfg->image_size,
-               cfg->patch_size);
-  VITK_REQUIRE(cfg->embed_dim > 0 && cfg->num_heads > 0 && cfg->embed_dim % cfg->num_heads == 0,
-               "embed_dim %d must be divisible by num_heads %d", cfg->embed_dim, cfg->num_heads);
-  VITK_REQUIRE(cfg->n_prefix_tokens == 1 || cfg->n_prefix_tokens == 2,
-               "n_prefix_tokens must be 1 (ViT) or 2 (DeiT)");
-  VITK_REQUIRE(cfg->num_layers > 0 && cfg->mlp_dim > 0 && cfg->in_channels > 0, "bad layer sizes");
-  VITK_REQUIRE(cfg->embed_dim % 8 == 0 && cfg->mlp_dim % 8 == 0,
-               "embed_dim and mlp_dim must be multiples of 8");
-  d->B = batch;
-  d->S = cfg->image_size;
-  d->p = cfg->patch_size;
-  d->C = cfg->in_channels;
-  d->D = cfg->embed_dim;
-  d->L = cfg->num_layers;
-  d->H = cfg->num_heads;
-  d->Mlp = cfg->mlp_dim;
-  d->prefix = cfg->n_prefix_tokens;
-  const int gw = d->S / d->p;
-  d->P = gw * gw;
-  d->N = d->P + d->prefix;
-  d->Kp = d->C * d->p * d->p;
-  d->hd = d->D / d->H;
-  d->M = static_cast<long long>(batch) * d->N;
-  d->Mp = static_cast<long long>(batch) * d->P;
-  VITK_REQUIRE(d->M < (1ll << 31) / 4, "batch too large");
-  return VITK_OK;
-}
 
 struct Workspace {
   float* x;     // residual stream f32 [M, D]
@@ -71,100 +31,20 @@ struct Workspace {
 };
 
 Workspace carve(const Dims& d, void* base) {
+  Carver c(base);
   Workspace w;
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    void* p = base ? static_cast<char*>(base) + off : nullptr;
-    off += align_up(n, 1024);
-    return p;
-  };
-  w.x = static_cast<float*>(take(d.M * d.D * 4));
-  w.xn = take(d.M * d.D * 2);
-  w.qkv = take(d.M * 3 * d.D * 2);
-  w.ctx = take(d.M * d.D * 2);
-  w.h = take(d.M * d.Mlp * 2);
-  w.patch = take(d.Mp * d.Kp * 2);
-  w.c_x = static_cast<float*>(take(static_cast<size_t>(d.B) * d.D * 4));
-  w.c_b = take(static_cast<size_t>(d.B) * d.D * 2);
-  w.c_h = take(static_cast<size_t>(d.B) * d.Mlp * 2);
-  w.stats = static_cast<float2*>(take(static_cast<size_t>(gemm_stats_parts(d.D)) * d.M * 8));
-  w.bytes = off;
+  w.x = static_cast<float*>(c.take(d.M * d.D * 4));
+  w.xn = c.take(d.M * d.D * 2);
+  w.qkv = c.take(d.M * 3 * d.D * 2);
+  w.ctx = c.take(d.M * d.D * 2);
+  w.h = c.take(d.M * d.Mlp * 2);
+  w.patch = c.take(d.Mp * d.Kp * 2);
+  w.c_x = static_cast<float*>(c.take(static_cast<size_t>(d.B) * d.D * 4));
+  w.c_b = c.take(static_cast<size_t>(d.B) * d.D * 2);
+  w.c_h = c.take(static_cast<size_t>(d.B) * d.Mlp * 2);
+  w.stats = static_cast<float2*>(c.take(static_cast<size_t>(gemm_stats_parts(d.D)) * d.M * 8));
+  w.bytes = c.off;
   return w;
-}
-
-int linear(const void* A, int lda, const void* W, int M, int N, int K, GemmEpi epi,
-           const float* bias, const float* resid, int ldr, void* out, void* out2, int ldo,
-           cudaStream_t stream) {
-  GemmProblem p;
-  p.A = A;
-  p.lda = lda;
-  p.B = W;
-  p.ldb = K;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = epi;
-  p.e.bias = bias;
-  p.e.resid = resid;
-  p.e.ldr = ldr;
-  p.e.out = out;
-  p.e.out2 = out2;
-  p.e.ldo = ldo;
-  return gemm_bf16_tn(p, stream);
-}
-
-// x += A W^T + bias, then xn = LN(x) * gamma + beta as bf16: the residual GEMM and a layernorm_fwd
-// launch.  train.py:586-591.
-int linear_resid_ln(const void* A, int lda, const void* W, int M, int N, int K, const float* bias,
-                    float* x, const float* gamma, const float* beta, float eps, void* xn,
-                    cudaStream_t stream) {
-  VITK_TRY(linear(A, lda, W, M, N, K, EPI_RESID_F32, bias, x, N, x, nullptr, N, stream));
-  return layernorm_fwd(x, N, gamma, beta, xn, 0, N, nullptr, nullptr, M, N, eps, stream);
-}
-
-// x += A W^T + bias in place; xb = bf16(x); partial row statistics of the updated x.
-int linear_resid_stats(const void* A, int lda, const void* W, int M, int N, int K, const float* bias,
-                       float* x, void* xb, float2* stats, cudaStream_t stream) {
-  GemmProblem p;
-  p.A = A;
-  p.lda = lda;
-  p.B = W;
-  p.ldb = K;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = EPI_RESID_STATS_F32;
-  p.e.bias = bias;
-  p.e.resid = x;
-  p.e.ldr = N;
-  p.e.out = x;
-  p.e.out2 = xb;
-  p.e.ldo = N;
-  p.e.ln_part_out = stats;
-  return gemm_bf16_tn(p, stream);
-}
-
-// out = epilogue(Linear(LayerNorm(x))) from bf16(x), W * gamma and the row statistics.
-int linear_ln(const void* xb, int K, const void* w_ln, int M, int N, GemmEpi epi,
-              const float* b_ln, const float2* stats, int nparts, float eps, void* out, int ldo,
-              cudaStream_t stream) {
-  GemmProblem p;
-  p.A = xb;
-  p.lda = K;
-  p.B = w_ln;
-  p.ldb = K;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = epi;
-  p.e.bias = b_ln;
-  p.e.out = out;
-  p.e.ldo = ldo;
-  p.e.ln_part = stats;
-  p.e.ln_nparts = nparts;
-  p.e.ln_dim = K;
-  p.e.ln_eps = eps;
-  return gemm_bf16_tn(p, stream);
 }
 
 // LayerNorm folding in vitk_forward: on when every block carries folded weights, unless
@@ -198,16 +78,30 @@ int cls_tail(const VitkConfig* cfg, const VitkWeights* w, const Dims& d, const W
   else
     VITK_TRY(attention_x(qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D, ws.c_b, D, D, d.B, 1,
                          d.N, d.H, d.hd, stream));
-  VITK_TRY(linear(ws.c_b, D, bw.proj_w, d.B, D, D, EPI_RESID_F32, bw.proj_b, ws.x, d.N * D, ws.c_x,
-                  nullptr, D, stream));
+  VITK_TRY(linear_fwd(ws.c_b, D, bw.proj_w, d.B, D, D, EPI_RESID_F32, bw.proj_b, ws.x, d.N * D,
+                      ws.c_x, nullptr, D, stream));
   VITK_TRY(layernorm_fwd(ws.c_x, D, bw.ln2_w, bw.ln2_b, ws.c_b, 0, D, nullptr, nullptr, d.B, D,
                          cfg->ln_eps, stream));
-  VITK_TRY(linear(ws.c_b, D, bw.fc1_w, d.B, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b, nullptr, 0,
-                  ws.c_h, nullptr, d.Mlp, stream));
-  VITK_TRY(linear(ws.c_h, d.Mlp, bw.fc2_w, d.B, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.c_x, D, ws.c_x,
-                  nullptr, D, stream));
+  VITK_TRY(linear_fwd(ws.c_b, D, bw.fc1_w, d.B, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b, nullptr, 0,
+                      ws.c_h, nullptr, d.Mlp, stream));
+  VITK_TRY(linear_fwd(ws.c_h, d.Mlp, bw.fc2_w, d.B, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.c_x, D,
+                      ws.c_x, nullptr, D, stream));
   return cls_head(ws.c_x, D, w->ln_f_w, w->ln_f_b, w->head_w, w->head_b, nullptr, logits_out, d.B,
                   D, cfg->n_classes, cfg->ln_eps, stream);
+}
+
+// Final LayerNorm of the residual stream x: over every token into tokens_out (the backbone
+// contract), and on the CLS rows with the classifier into logits_out; either may be null.
+int encoder_tail(const VitkConfig* cfg, const VitkWeights* w, const Dims& d, const float* x,
+                 float* tokens_out, float* logits_out, cudaStream_t stream) {
+  const int D = d.D;
+  if (tokens_out)
+    VITK_TRY(layernorm_fwd(x, D, w->ln_f_w, w->ln_f_b, tokens_out, 1, D, nullptr, nullptr,
+                           static_cast<int>(d.M), D, cfg->ln_eps, stream));
+  if (logits_out)
+    VITK_TRY(cls_head(x, static_cast<long long>(d.N) * D, w->ln_f_w, w->ln_f_b, w->head_w,
+                      w->head_b, nullptr, logits_out, d.B, D, cfg->n_classes, cfg->ln_eps, stream));
+  return VITK_OK;
 }
 
 struct U8Input {
@@ -229,26 +123,8 @@ int forward_bf16(const VitkConfig* cfg, const VitkWeights* w, const float* image
     VITK_TRY(patchify(images, ws.patch, d.B, d.C, d.S, d.p, stream));
   VITK_TRY(prefix_tokens(ws.x, w->cls_token, w->dist_token, w->pos_embed, d.B, d.N, D, d.prefix,
                          stream));
-  {
-    GemmProblem p;
-    p.A = ws.patch;
-    p.lda = d.Kp;
-    p.B = w->patch_w;
-    p.ldb = d.Kp;
-    p.M = static_cast<int>(d.Mp);
-    p.N = D;
-    p.K = d.Kp;
-    p.epi = EPI_RESID_F32;
-    p.e.bias = w->patch_b;
-    p.e.resid = w->pos_embed;
-    p.e.ldr = D;
-    p.e.out = ws.x;
-    p.e.ldo = D;
-    p.e.rows_per_group = d.P;
-    p.e.group_stride = d.N;
-    p.e.group_offset = d.prefix;
-    VITK_TRY(gemm_bf16_tn(p, stream));
-  }
+  VITK_TRY(patch_embed(ws.patch, w->patch_w, d.B, d.P, d.Kp, D, d.N, d.prefix, w->patch_b,
+                       w->pos_embed, ws.x, stream));
   if (g_ln_fold && folded_weights_present(w, d.L)) {
     // -- encoder blocks with every LayerNorm folded into the GEMMs around it: 5 launches per
     //    block, no pass over the fp32 residual stream other than the residual GEMMs' own update
@@ -258,65 +134,51 @@ int forward_bf16(const VitkConfig* cfg, const VitkWeights* w, const float* image
     for (int l = 0; l < d.L; ++l) {
       const VitkBlockWeights& bw = w->blocks[l];
       const bool last = (l == d.L - 1);
-      VITK_TRY(linear_ln(ws.xn, D, bw.qkv_w_ln, M, 3 * D, EPI_BF16, bw.qkv_b_ln, ws.stats, nparts,
-                         cfg->ln_eps, ws.qkv, 3 * D, stream));
-      if (cls_only_tail && last) break;  // the row-wise tail below finishes the block
+      VITK_TRY(linear_ln(ws.xn, D, bw.qkv_w_ln, D, M, 3 * D, D, EPI_BF16, bw.qkv_b_ln, ws.stats,
+                         nparts, cfg->ln_eps, ws.qkv, 3 * D, stream));
+      if (cls_only_tail && last) break;  // cls_tail finishes the block
       VITK_TRY(attention_fwd(ws.qkv, ws.ctx, nullptr, d.B, d.N, d.H, d.hd, stream));
-      VITK_TRY(linear_resid_stats(ws.ctx, D, bw.proj_w, M, D, D, bw.proj_b, ws.x, ws.xn, ws.stats,
-                                  stream));
+      VITK_TRY(linear_resid_stats(ws.ctx, D, bw.proj_w, D, M, D, D, bw.proj_b, ws.x, ws.xn,
+                                  ws.stats, stream));
       nparts = parts;
-      VITK_TRY(linear_ln(ws.xn, D, bw.fc1_w_ln, M, d.Mlp, EPI_GELU_TANH_BF16, bw.fc1_b_ln, ws.stats,
-                         nparts, cfg->ln_eps, ws.h, d.Mlp, stream));
+      VITK_TRY(linear_ln(ws.xn, D, bw.fc1_w_ln, D, M, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b_ln,
+                         ws.stats, nparts, cfg->ln_eps, ws.h, d.Mlp, stream));
       if (!last)
-        VITK_TRY(linear_resid_stats(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, bw.fc2_b, ws.x, ws.xn,
-                                    ws.stats, stream));
+        VITK_TRY(linear_resid_stats(ws.h, d.Mlp, bw.fc2_w, d.Mlp, M, D, d.Mlp, bw.fc2_b, ws.x,
+                                    ws.xn, ws.stats, stream));
       else
-        VITK_TRY(linear(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.x, D, ws.x,
-                        nullptr, D, stream));
+        VITK_TRY(linear_fwd(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.x, D,
+                            ws.x, nullptr, D, stream));
     }
-    if (cls_only_tail)
-      return cls_tail(cfg, w, d, ws, logits_out, stream);
-    if (tokens_out)
-      VITK_TRY(layernorm_fwd(ws.x, D, w->ln_f_w, w->ln_f_b, tokens_out, 1, D, nullptr, nullptr, M, D,
-                             cfg->ln_eps, stream));
-    if (logits_out)
-      VITK_TRY(cls_head(ws.x, static_cast<long long>(d.N) * D, w->ln_f_w, w->ln_f_b, w->head_w,
-                        w->head_b, nullptr, logits_out, d.B, D, cfg->n_classes, cfg->ln_eps, stream));
-    return VITK_OK;
-  }
-  // -- encoder blocks (train.py:584-593)
-  // LayerNorm 1 of block 0 runs on its own; every later one follows the residual GEMM that
-  // produces its input in linear_resid_ln (projection -> LN2, linear2 -> LN1 of the next
-  // block)
-  VITK_TRY(layernorm_fwd(ws.x, D, w->blocks[0].ln1_w, w->blocks[0].ln1_b, ws.xn, 0, D, nullptr,
-                         nullptr, M, D, cfg->ln_eps, stream));
-  for (int l = 0; l < d.L; ++l) {
-    const VitkBlockWeights& bw = w->blocks[l];
-    VITK_TRY(linear(ws.xn, D, bw.qkv_w, M, 3 * D, D, EPI_BF16, bw.qkv_b, nullptr, 0, ws.qkv,
-                    nullptr, 3 * D, stream));
-    if (cls_only_tail && l == d.L - 1) return cls_tail(cfg, w, d, ws, logits_out, stream);
-    VITK_TRY(attention_fwd(ws.qkv, ws.ctx, nullptr, d.B, d.N, d.H, d.hd, stream));
-    VITK_TRY(linear_resid_ln(ws.ctx, D, bw.proj_w, M, D, D, bw.proj_b, ws.x, bw.ln2_w, bw.ln2_b,
-                             cfg->ln_eps, ws.xn, stream));
-    VITK_TRY(linear(ws.xn, D, bw.fc1_w, M, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b, nullptr, 0, ws.h,
-                    nullptr, d.Mlp, stream));
-    if (l + 1 < d.L) {
-      const VitkBlockWeights& nx = w->blocks[l + 1];
-      VITK_TRY(linear_resid_ln(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, bw.fc2_b, ws.x, nx.ln1_w,
-                               nx.ln1_b, cfg->ln_eps, ws.xn, stream));
-    } else {
-      VITK_TRY(linear(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.x, D, ws.x,
-                      nullptr, D, stream));
+  } else {
+    // -- encoder blocks (train.py:584-593)
+    // LayerNorm 1 of block 0 runs on its own; every later one follows the residual GEMM that
+    // produces its input in linear_resid_ln (projection -> LN2, linear2 -> LN1 of the next
+    // block)
+    VITK_TRY(layernorm_fwd(ws.x, D, w->blocks[0].ln1_w, w->blocks[0].ln1_b, ws.xn, 0, D, nullptr,
+                           nullptr, M, D, cfg->ln_eps, stream));
+    for (int l = 0; l < d.L; ++l) {
+      const VitkBlockWeights& bw = w->blocks[l];
+      VITK_TRY(linear_fwd(ws.xn, D, bw.qkv_w, M, 3 * D, D, EPI_BF16, bw.qkv_b, nullptr, 0, ws.qkv,
+                          nullptr, 3 * D, stream));
+      if (cls_only_tail && l == d.L - 1) break;  // cls_tail finishes the block
+      VITK_TRY(attention_fwd(ws.qkv, ws.ctx, nullptr, d.B, d.N, d.H, d.hd, stream));
+      VITK_TRY(linear_resid_ln(ws.ctx, D, bw.proj_w, D, M, D, D, bw.proj_b, ws.x, bw.ln2_w,
+                               bw.ln2_b, cfg->ln_eps, ws.xn, nullptr, nullptr, stream));
+      VITK_TRY(linear_fwd(ws.xn, D, bw.fc1_w, M, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b, nullptr, 0,
+                          ws.h, nullptr, d.Mlp, stream));
+      if (l + 1 < d.L) {
+        const VitkBlockWeights& nx = w->blocks[l + 1];
+        VITK_TRY(linear_resid_ln(ws.h, d.Mlp, bw.fc2_w, d.Mlp, M, D, d.Mlp, bw.fc2_b, ws.x,
+                                 nx.ln1_w, nx.ln1_b, cfg->ln_eps, ws.xn, nullptr, nullptr, stream));
+      } else {
+        VITK_TRY(linear_fwd(ws.h, d.Mlp, bw.fc2_w, M, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.x, D,
+                            ws.x, nullptr, D, stream));
+      }
     }
   }
-  // -- final LayerNorm: all tokens for the backbone contract, CLS row only for the classifier
-  if (tokens_out)
-    VITK_TRY(layernorm_fwd(ws.x, D, w->ln_f_w, w->ln_f_b, tokens_out, 1, D, nullptr, nullptr, M, D,
-                           cfg->ln_eps, stream));
-  if (logits_out)
-    VITK_TRY(cls_head(ws.x, static_cast<long long>(d.N) * D, w->ln_f_w, w->ln_f_b, w->head_w,
-                      w->head_b, nullptr, logits_out, d.B, D, cfg->n_classes, cfg->ln_eps, stream));
-  return VITK_OK;
+  if (cls_only_tail) return cls_tail(cfg, w, d, ws, logits_out, stream);
+  return encoder_tail(cfg, w, d, ws.x, tokens_out, logits_out, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -336,23 +198,18 @@ struct WorkspaceF32 {
 };
 
 WorkspaceF32 carve_f32(const Dims& d, void* base) {
+  Carver c(base);
   WorkspaceF32 w;
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    void* p = base ? static_cast<char*>(base) + off : nullptr;
-    off += align_up(n, 1024);
-    return p;
-  };
   int kmax = d.D > d.Mlp ? d.D : d.Mlp;
   if (d.Kp > kmax) kmax = d.Kp;
-  w.x = static_cast<float*>(take(d.M * d.D * 4));
-  w.xn = static_cast<float*>(take(d.M * d.D * 4));
-  w.qkv = static_cast<float*>(take(d.M * 3 * d.D * 4));
-  w.ctx = static_cast<float*>(take(d.M * d.D * 4));
-  w.h = static_cast<float*>(take(d.M * d.Mlp * 4));
-  w.patch = static_cast<float*>(take(d.Mp * d.Kp * 4));
-  w.a6 = take(d.M * 6 * static_cast<size_t>(kmax) * 2);
-  w.bytes = off;
+  w.x = static_cast<float*>(c.take(d.M * d.D * 4));
+  w.xn = static_cast<float*>(c.take(d.M * d.D * 4));
+  w.qkv = static_cast<float*>(c.take(d.M * 3 * d.D * 4));
+  w.ctx = static_cast<float*>(c.take(d.M * d.D * 4));
+  w.h = static_cast<float*>(c.take(d.M * d.Mlp * 4));
+  w.patch = static_cast<float*>(c.take(d.Mp * d.Kp * 4));
+  w.a6 = c.take(d.M * 6 * static_cast<size_t>(kmax) * 2);
+  w.bytes = c.off;
   return w;
 }
 
@@ -360,21 +217,8 @@ WorkspaceF32 carve_f32(const Dims& d, void* base) {
 int linear_f32(const float* A, int K, const void* W6, int M, int N, GemmEpi epi, const float* bias,
                float* resid_out, float* out, int apply_gelu_to_a, void* a6, cudaStream_t stream) {
   VITK_TRY(split3(A, K, a6, M, K, 0, apply_gelu_to_a, stream));
-  GemmProblem p;
-  p.A = a6;
-  p.lda = 6 * K;
-  p.B = W6;
-  p.ldb = 6 * K;
-  p.M = M;
-  p.N = N;
-  p.K = 6 * K;
-  p.epi = epi;
-  p.e.bias = bias;
-  p.e.resid = resid_out;
-  p.e.ldr = N;
-  p.e.out = (epi == EPI_RESID_F32) ? resid_out : out;
-  p.e.ldo = N;
-  return gemm_bf16_tn(p, stream);
+  return linear_fwd(a6, 6 * K, W6, M, N, 6 * K, epi, bias, resid_out, N,
+                    (epi == EPI_RESID_F32) ? resid_out : out, nullptr, N, stream);
 }
 
 int forward_f32(const VitkConfig* cfg, const VitkWeights* w, const float* images, const Dims& d,
@@ -383,27 +227,9 @@ int forward_f32(const VitkConfig* cfg, const VitkWeights* w, const float* images
   VITK_TRY(patchify_f32(images, ws.patch, d.B, d.C, d.S, d.p, stream));
   VITK_TRY(prefix_tokens(ws.x, w->cls_token, w->dist_token, w->pos_embed, d.B, d.N, D, d.prefix,
                          stream));
-  {
-    VITK_TRY(split3(ws.patch, d.Kp, ws.a6, d.Mp, d.Kp, 0, 0, stream));
-    GemmProblem p;
-    p.A = ws.a6;
-    p.lda = 6 * d.Kp;
-    p.B = w->patch_w;
-    p.ldb = 6 * d.Kp;
-    p.M = static_cast<int>(d.Mp);
-    p.N = D;
-    p.K = 6 * d.Kp;
-    p.epi = EPI_RESID_F32;
-    p.e.bias = w->patch_b;
-    p.e.resid = w->pos_embed;
-    p.e.ldr = D;
-    p.e.out = ws.x;
-    p.e.ldo = D;
-    p.e.rows_per_group = d.P;
-    p.e.group_stride = d.N;
-    p.e.group_offset = d.prefix;
-    VITK_TRY(gemm_bf16_tn(p, stream));
-  }
+  VITK_TRY(split3(ws.patch, d.Kp, ws.a6, d.Mp, d.Kp, 0, 0, stream));
+  VITK_TRY(patch_embed(ws.a6, w->patch_w, d.B, d.P, 6 * d.Kp, D, d.N, d.prefix, w->patch_b,
+                       w->pos_embed, ws.x, stream));
   for (int l = 0; l < d.L; ++l) {
     const VitkBlockWeights& bw = w->blocks[l];
     VITK_TRY(layernorm_fwd(ws.x, D, bw.ln1_w, bw.ln1_b, ws.xn, 1, D, nullptr, nullptr, M, D,
@@ -421,12 +247,34 @@ int forward_f32(const VitkConfig* cfg, const VitkWeights* w, const float* images
     VITK_TRY(linear_f32(ws.h, d.Mlp, bw.fc2_w, M, D, EPI_RESID_F32, bw.fc2_b, ws.x, nullptr, 1,
                         ws.a6, stream));
   }
-  if (tokens_out)
-    VITK_TRY(layernorm_fwd(ws.x, D, w->ln_f_w, w->ln_f_b, tokens_out, 1, D, nullptr, nullptr, M, D,
-                           cfg->ln_eps, stream));
+  return encoder_tail(cfg, w, d, ws.x, tokens_out, logits_out, stream);
+}
+
+size_t workspace_size(const VitkConfig* cfg, const Dims& d) {
+  return (cfg->precision == 1) ? carve_f32(d, nullptr).bytes : carve(d, nullptr).bytes;
+}
+
+// Argument checks shared by the inference entry points, run after each one's own: the weights,
+// the classifier head when logits are requested, and the workspace.
+int check_forward_args(const VitkConfig* cfg, const VitkWeights* w, const Dims& d,
+                       const float* tokens_out, const float* logits_out, const void* workspace,
+                       size_t workspace_bytes) {
+  VITK_REQUIRE(w != nullptr && workspace != nullptr, "null argument");
+  VITK_REQUIRE(tokens_out != nullptr || logits_out != nullptr,
+               "at least one of tokens_out / logits_out must be non-null");
+  VITK_REQUIRE(w->blocks != nullptr && w->patch_w && w->patch_b && w->cls_token && w->pos_embed &&
+                   w->ln_f_w && w->ln_f_b,
+               "weights struct has null members");
+  VITK_REQUIRE(d.prefix == 1 || w->dist_token != nullptr, "DeiT needs dist_token");
   if (logits_out)
-    VITK_TRY(cls_head(ws.x, static_cast<long long>(d.N) * D, w->ln_f_w, w->ln_f_b, w->head_w,
-                      w->head_b, nullptr, logits_out, d.B, D, cfg->n_classes, cfg->ln_eps, stream));
+    VITK_REQUIRE(cfg->n_classes > 0 && w->head_w && w->head_b,
+                 "logits requested but no classifier head configured");
+  VITK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0,
+               "workspace must be 1024-byte aligned");
+  const size_t need = workspace_size(cfg, d);
+  if (need > workspace_bytes)
+    return set_error(VITK_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need,
+                     workspace_bytes);
   return VITK_OK;
 }
 
@@ -471,45 +319,16 @@ int vitk_gemm_resid_stats(const void* A, int lda, const void* W, int ldb, int M,
                           const float* bias, float* x_inout, void* x_bf16, float* stats,
                           vitk_stream_t stream) {
   VITK_REQUIRE(x_inout && x_bf16 && stats, "gemm_resid_stats: null output");
-  GemmProblem p;
-  p.A = A;
-  p.lda = lda;
-  p.B = W;
-  p.ldb = ldb;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = EPI_RESID_STATS_F32;
-  p.e.bias = bias;
-  p.e.resid = x_inout;
-  p.e.ldr = N;
-  p.e.out = x_inout;
-  p.e.out2 = x_bf16;
-  p.e.ldo = N;
-  p.e.ln_part_out = reinterpret_cast<float2*>(stats);
-  return gemm_bf16_tn(p, static_cast<cudaStream_t>(stream));
+  return linear_resid_stats(A, lda, W, ldb, M, N, K, bias, x_inout, x_bf16,
+                            reinterpret_cast<float2*>(stats), static_cast<cudaStream_t>(stream));
 }
 int vitk_gemm_layernorm_folded(const void* x_bf16, int lda, const void* w_ln, int ldb, int M, int N,
                                int K, int epilogue, const float* b_ln, const float* stats,
                                int n_parts, float eps, void* out, int ldo, vitk_stream_t stream) {
   VITK_REQUIRE(stats != nullptr, "gemm_layernorm_folded: null statistics");
-  GemmProblem p;
-  p.A = x_bf16;
-  p.lda = lda;
-  p.B = w_ln;
-  p.ldb = ldb;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = static_cast<GemmEpi>(epilogue);
-  p.e.bias = b_ln;
-  p.e.out = out;
-  p.e.ldo = ldo;
-  p.e.ln_part = reinterpret_cast<const float2*>(stats);
-  p.e.ln_nparts = n_parts;
-  p.e.ln_dim = K;
-  p.e.ln_eps = eps;
-  return gemm_bf16_tn(p, static_cast<cudaStream_t>(stream));
+  return linear_ln(x_bf16, lda, w_ln, ldb, M, N, K, static_cast<GemmEpi>(epilogue), b_ln,
+                   reinterpret_cast<const float2*>(stats), n_parts, eps, out, ldo,
+                   static_cast<cudaStream_t>(stream));
 }
 int vitk_postprocess_scores(const float* logits, int rows, int n_classes, int exclude_last,
                             float* scores_out, long long* labels_out, float* probs_out,
@@ -562,7 +381,7 @@ int vitk_workspace_bytes(const VitkConfig* cfg, int batch, size_t* out_bytes) {
   Dims d;
   VITK_TRY(check_config(cfg, batch, &d));
   VITK_REQUIRE(out_bytes != nullptr, "out_bytes is null");
-  *out_bytes = (cfg->precision == 1) ? carve_f32(d, nullptr).bytes : carve(d, nullptr).bytes;
+  *out_bytes = workspace_size(cfg, d);
   return VITK_OK;
 }
 
@@ -571,35 +390,16 @@ int vitk_forward(const VitkConfig* cfg, const VitkWeights* w, const float* image
                  vitk_stream_t stream) {
   Dims d;
   VITK_TRY(check_config(cfg, batch, &d));
-  VITK_REQUIRE(w != nullptr && images != nullptr && workspace != nullptr, "null argument");
-  VITK_REQUIRE(tokens_out != nullptr || logits_out != nullptr,
-               "at least one of tokens_out / logits_out must be non-null");
-  VITK_REQUIRE(w->blocks != nullptr && w->patch_w && w->patch_b && w->cls_token && w->pos_embed &&
-                   w->ln_f_w && w->ln_f_b,
-               "weights struct has null members");
-  VITK_REQUIRE(d.prefix == 1 || w->dist_token != nullptr, "DeiT needs dist_token");
-  if (logits_out)
-    VITK_REQUIRE(cfg->n_classes > 0 && w->head_w && w->head_b,
-                 "logits requested but no classifier head configured");
-  VITK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0,
-               "workspace must be 1024-byte aligned");
+  VITK_REQUIRE(images != nullptr, "null argument");
   VITK_REQUIRE(cfg->precision == 0 || cfg->precision == 1, "unknown precision mode %d",
                cfg->precision);
   VITK_REQUIRE(d.hd == 64 || (cfg->precision == 0 && d.hd >= 8 && d.hd <= 128 && d.hd % 8 == 0),
                "head_dim %d unsupported (bf16: 8..128 in steps of 8; fp32-parity mode: 64)", d.hd);
-  if (cfg->precision == 1) {
-    const WorkspaceF32 wf = carve_f32(d, workspace);
-    if (wf.bytes > workspace_bytes)
-      return set_error(VITK_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", wf.bytes,
-                       workspace_bytes);
-    return forward_f32(cfg, w, images, d, tokens_out, logits_out, wf,
+  VITK_TRY(check_forward_args(cfg, w, d, tokens_out, logits_out, workspace, workspace_bytes));
+  if (cfg->precision == 1)
+    return forward_f32(cfg, w, images, d, tokens_out, logits_out, carve_f32(d, workspace),
                        static_cast<cudaStream_t>(stream));
-  }
-  const Workspace ws = carve(d, workspace);
-  if (ws.bytes > workspace_bytes)
-    return set_error(VITK_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", ws.bytes,
-                     workspace_bytes);
-  return forward_bf16(cfg, w, images, d, tokens_out, logits_out, ws,
+  return forward_bf16(cfg, w, images, d, tokens_out, logits_out, carve(d, workspace),
                       static_cast<cudaStream_t>(stream));
 }
 
@@ -608,24 +408,13 @@ int vitk_forward_cls(const VitkConfig* cfg, const VitkWeights* w, const float* i
                      vitk_stream_t stream) {
   Dims d;
   VITK_TRY(check_config(cfg, batch, &d));
-  VITK_REQUIRE(w != nullptr && images != nullptr && workspace != nullptr && logits_out != nullptr,
-               "null argument");
-  VITK_REQUIRE(w->blocks != nullptr && w->patch_w && w->patch_b && w->cls_token && w->pos_embed &&
-                   w->ln_f_w && w->ln_f_b,
-               "weights struct has null members");
-  VITK_REQUIRE(d.prefix == 1 || w->dist_token != nullptr, "DeiT needs dist_token");
-  VITK_REQUIRE(cfg->n_classes > 0 && w->head_w && w->head_b, "no classifier head configured");
-  VITK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0,
-               "workspace must be 1024-byte aligned");
+  VITK_REQUIRE(images != nullptr && logits_out != nullptr, "null argument");
   VITK_REQUIRE(cfg->precision == 0, "the CLS-only tail is implemented for the bf16 path");
   VITK_REQUIRE(d.hd == 32 || d.hd == 64 || d.hd == 96 || d.hd == 128,
                "head_dim %d unsupported (32, 64, 96 or 128)", d.hd);
-  const Workspace ws = carve(d, workspace);
-  if (ws.bytes > workspace_bytes)
-    return set_error(VITK_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", ws.bytes,
-                     workspace_bytes);
-  return forward_bf16(cfg, w, images, d, nullptr, logits_out, ws, static_cast<cudaStream_t>(stream),
-                      nullptr, true);
+  VITK_TRY(check_forward_args(cfg, w, d, nullptr, logits_out, workspace, workspace_bytes));
+  return forward_bf16(cfg, w, images, d, nullptr, logits_out, carve(d, workspace),
+                      static_cast<cudaStream_t>(stream), nullptr, true);
 }
 
 int vitk_forward_u8(const VitkConfig* cfg, const VitkWeights* w, const unsigned char* images_hwc,
@@ -634,29 +423,14 @@ int vitk_forward_u8(const VitkConfig* cfg, const VitkWeights* w, const unsigned 
                     vitk_stream_t stream) {
   Dims d;
   VITK_TRY(check_config(cfg, batch, &d));
-  VITK_REQUIRE(w != nullptr && images_hwc != nullptr && mean != nullptr && stddev != nullptr &&
-                   workspace != nullptr, "null argument");
-  VITK_REQUIRE(tokens_out != nullptr || logits_out != nullptr,
-               "at least one of tokens_out / logits_out must be non-null");
-  VITK_REQUIRE(w->blocks != nullptr && w->patch_w && w->patch_b && w->cls_token && w->pos_embed &&
-                   w->ln_f_w && w->ln_f_b,
-               "weights struct has null members");
-  VITK_REQUIRE(d.prefix == 1 || w->dist_token != nullptr, "DeiT needs dist_token");
-  if (logits_out)
-    VITK_REQUIRE(cfg->n_classes > 0 && w->head_w && w->head_b,
-                 "logits requested but no classifier head configured");
-  VITK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0,
-               "workspace must be 1024-byte aligned");
+  VITK_REQUIRE(images_hwc != nullptr && mean != nullptr && stddev != nullptr, "null argument");
   VITK_REQUIRE(cfg->precision == 0, "the 8-bit input edge feeds the bf16 path only");
   VITK_REQUIRE(d.C == 3, "the 8-bit input edge needs RGB images");
   VITK_REQUIRE(d.hd >= 8 && d.hd <= 128 && d.hd % 8 == 0,
                "head_dim %d unsupported (8..128 in steps of 8)", d.hd);
-  const Workspace ws = carve(d, workspace);
-  if (ws.bytes > workspace_bytes)
-    return set_error(VITK_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", ws.bytes,
-                     workspace_bytes);
+  VITK_TRY(check_forward_args(cfg, w, d, tokens_out, logits_out, workspace, workspace_bytes));
   const U8Input u8{images_hwc, mean, stddev};
-  return forward_bf16(cfg, w, nullptr, d, tokens_out, logits_out, ws,
+  return forward_bf16(cfg, w, nullptr, d, tokens_out, logits_out, carve(d, workspace),
                       static_cast<cudaStream_t>(stream), &u8);
 }
 
@@ -696,43 +470,14 @@ int vitk_gemm_resid_layernorm(const void* A, int lda, const void* W, int ldb, in
   // checked before the GEMM updates x: layernorm_fwd takes rows of at most 1024 features
   VITK_REQUIRE(ln_out && x_inout && gamma && beta && N <= 1024,
                "gemm_resid_layernorm: null operand or N > 1024");
-  GemmProblem p;
-  p.A = A;
-  p.lda = lda;
-  p.B = W;
-  p.ldb = ldb;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = EPI_RESID_F32;
-  p.e.bias = bias;
-  p.e.resid = x_inout;
-  p.e.ldr = N;
-  p.e.out = x_inout;
-  p.e.ldo = N;
-  const cudaStream_t st = static_cast<cudaStream_t>(stream);
-  VITK_TRY(gemm_bf16_tn(p, st));
-  return layernorm_fwd(x_inout, N, gamma, beta, ln_out, 0, N, mean_out, rstd_out, M, N, eps, st);
+  return linear_resid_ln(A, lda, W, ldb, M, N, K, bias, x_inout, gamma, beta, eps, ln_out, mean_out,
+                         rstd_out, static_cast<cudaStream_t>(stream));
 }
 
 int vitk_gemm_wgrad(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* out,
                     int ldo, float alpha, float beta, int split_k, vitk_stream_t stream) {
-  GemmProblem p;
-  p.A = A;
-  p.lda = lda;
-  p.B = B;
-  p.ldb = ldb;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = EPI_F32;
-  p.mn_major = true;
-  p.split_k = split_k;
-  p.e.out = out;
-  p.e.ldo = ldo;
-  p.e.alpha = alpha;
-  p.e.beta = beta;
-  return gemm_bf16_tn(p, static_cast<cudaStream_t>(stream));
+  return gemm_wgrad(A, lda, B, ldb, M, N, K, out, ldo, alpha, beta, split_k,
+                    static_cast<cudaStream_t>(stream));
 }
 
 int vitk_layernorm(const float* x, long long in_stride, const float* gamma, const float* beta,

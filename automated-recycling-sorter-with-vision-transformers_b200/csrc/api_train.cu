@@ -5,6 +5,7 @@
 #include "../../include/vitk.h"
 
 #include "common.h"
+#include "encoder.cuh"
 #include "gemm_sm100.cuh"
 #include "rowops.cuh"
 #include "train_ops.cuh"
@@ -12,49 +13,17 @@
 namespace vitk {
 namespace {
 
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-struct TDims {
-  int B, S, p, C, D, L, H, Mlp, prefix, P, N, Kp, hd, ncls;
-  long long M, Mp;
-};
-
-int check_train_config(const VitkConfig* cfg, int batch, TDims* d) {
-  VITK_REQUIRE(cfg != nullptr && batch > 0, "bad config / batch");
-  VITK_REQUIRE(cfg->image_size > 0 && cfg->patch_size > 0 &&
-                   cfg->image_size % cfg->patch_size == 0,
-               "image_size must be a positive multiple of patch_size");
-  VITK_REQUIRE(cfg->embed_dim > 0 && cfg->num_heads > 0 && cfg->embed_dim % cfg->num_heads == 0,
-               "embed_dim must be divisible by num_heads");
-  VITK_REQUIRE(cfg->n_prefix_tokens == 1 || cfg->n_prefix_tokens == 2, "n_prefix_tokens in {1,2}");
-  VITK_REQUIRE(cfg->embed_dim % 8 == 0 && cfg->mlp_dim % 8 == 0 && cfg->num_layers > 0,
-               "bad layer sizes");
+// The shared encoder checks, then what training adds to them.
+int check_train_config(const VitkConfig* cfg, int batch, Dims* d) {
+  VITK_TRY(check_config(cfg, batch, d));
   VITK_REQUIRE(cfg->precision == 0, "training runs in the bf16 mode only");
   VITK_REQUIRE(cfg->dropout_p >= 0.f && cfg->dropout_p < 1.f, "dropout_p must be in [0, 1)");
-  d->B = batch;
-  d->S = cfg->image_size;
-  d->p = cfg->patch_size;
-  d->C = cfg->in_channels;
-  d->D = cfg->embed_dim;
-  d->L = cfg->num_layers;
-  d->H = cfg->num_heads;
-  d->Mlp = cfg->mlp_dim;
-  d->prefix = cfg->n_prefix_tokens;
-  const int gw = d->S / d->p;
-  d->P = gw * gw;
-  d->N = d->P + d->prefix;
-  d->Kp = d->C * d->p * d->p;
-  d->hd = d->D / d->H;
-  d->ncls = cfg->n_classes;
-  d->M = static_cast<long long>(batch) * d->N;
-  d->Mp = static_cast<long long>(batch) * d->P;
   // head_dim 64 up to 256 tokens: tcgen05 attention kernels; every other shape (train.py's own
   // Config has head_dim 16; a 384 px fine-tune 577 tokens): the CUDA-core kernels of
   // attention_gen.cu, as far as one head's operands fit in shared memory
   VITK_REQUIRE((d->hd == 64 && d->N <= 256) || attention_gen_fits(d->N, d->hd),
                "training: head_dim %d with %d tokens is not covered (head_dim 8..128 in steps of 8, "
                "and tokens * head_dim within shared memory)", d->hd, d->N);
-  VITK_REQUIRE(d->M < (1ll << 31) / 4, "batch too large");
   VITK_REQUIRE(cfg->dropout_p == 0.f || d->M * d->Mlp < (1ll << 32),
                "dropout_p > 0 needs batch * tokens * mlp_dim < 2^32");
   return VITK_OK;
@@ -93,18 +62,7 @@ struct Saved {
   size_t bytes;
 };
 
-struct Carver {
-  char* base;
-  size_t off = 0;
-  explicit Carver(void* b) : base(static_cast<char*>(b)) {}
-  void* take(size_t n) {
-    void* p = base ? base + off : nullptr;
-    off += align_up(n, 1024);
-    return p;
-  }
-};
-
-SavedBlock carve_block(const TDims& d, void* base, size_t* bytes) {
+SavedBlock carve_block(const Dims& d, void* base, size_t* bytes) {
   Carver c(base);
   SavedBlock s;
   s.x1 = static_cast<float*>(c.take(d.M * d.D * 4));
@@ -124,7 +82,7 @@ SavedBlock carve_block(const TDims& d, void* base, size_t* bytes) {
   return s;
 }
 
-Saved carve_saved(const TDims& d, void* base) {
+Saved carve_saved(const Dims& d, void* base) {
   Carver c(base);
   Saved s;
   s.patches = c.take(d.Mp * d.Kp * 2);
@@ -150,7 +108,7 @@ struct TrainWs {
   size_t bytes;
 };
 
-TrainWs carve_ws(const TDims& d, void* base) {
+TrainWs carve_ws(const Dims& d, void* base) {
   Carver c(base);
   TrainWs w;
   w.x = static_cast<float*>(c.take(d.M * d.D * 4));
@@ -167,102 +125,14 @@ TrainWs carve_ws(const TDims& d, void* base) {
   return w;
 }
 
-int linear_fwd(const void* A, int lda, const void* W, int M, int N, int K, GemmEpi epi,
-               const float* bias, const float* resid, void* out, void* out2, int ldo,
-               cudaStream_t stream, const DropParams& drop = DropParams()) {
-  GemmProblem p;
-  p.e.drop = drop;
-  p.A = A;
-  p.lda = lda;
-  p.B = W;
-  p.ldb = K;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = epi;
-  p.e.bias = bias;
-  p.e.resid = resid;
-  p.e.ldr = ldo;
-  p.e.out = out;
-  p.e.out2 = out2;
-  p.e.ldo = ldo;
-  return gemm_bf16_tn(p, stream);
-}
-
-// dX[M, in] = dY[M, out] * W[out, in]  with W^T [in, out] as the K-major B operand.
-int linear_dgrad(const void* dY, int out_f, const void* Wt, int M, int in_f, GemmEpi epi,
-                 const void* aux, void* dX, cudaStream_t stream,
-                 const DropParams& drop = DropParams()) {
-  GemmProblem p;
-  p.e.drop = drop;
-  p.A = dY;
-  p.lda = out_f;
-  p.B = Wt;
-  p.ldb = out_f;
-  p.M = M;
-  p.N = in_f;
-  p.K = out_f;
-  p.epi = epi;
-  p.e.aux = aux;
-  p.e.out = dX;
-  p.e.ldo = in_f;
-  return gemm_bf16_tn(p, stream);
-}
-
-// dW[out, in] += dY[tokens, out]^T * X[tokens, in]   and   db[out] += column sums of dY
-int linear_wgrad(const void* dY, int out_f, const void* X, int in_f, int tokens, float* dW,
-                 float* db, cudaStream_t stream) {
-  GemmProblem p;
-  p.A = dY;
-  p.lda = out_f;
-  p.B = X;
-  p.ldb = in_f;
-  p.M = out_f;
-  p.N = in_f;
-  p.K = tokens;
-  p.epi = EPI_F32;
-  p.mn_major = true;
-  p.e.out = dW;
-  p.e.ldo = in_f;
-  p.e.beta = 1.f;
-  // enough K splits to give every CTA pair about two work items
-  const int tiles = ((out_f + 255) / 256) * ((in_f + 255) / 256);
-  int split = (sm_count() / 2 * 2) / (tiles > 0 ? tiles : 1);
-  if (split < 1) split = 1;
-  const int num_kb = (tokens + 63) / 64;
-  if (split > num_kb / 4) split = num_kb / 4 > 0 ? num_kb / 4 : 1;
-  p.split_k = split;
-  VITK_TRY(gemm_bf16_tn(p, stream));
-  if (db != nullptr) VITK_TRY(colsum_bf16(dY, out_f, tokens, out_f, db, stream));
-  return VITK_OK;
-}
-
-int forward_train(const VitkConfig* cfg, const VitkWeights* w, const float* images, const TDims& d,
+int forward_train(const VitkConfig* cfg, const VitkWeights* w, const float* images, const Dims& d,
                   float* tokens_out, const Saved& sv, const TrainWs& ws, cudaStream_t stream) {
   const int M = static_cast<int>(d.M), D = d.D;
   VITK_TRY(patchify(images, sv.patches, d.B, d.C, d.S, d.p, stream));
   VITK_TRY(prefix_tokens(ws.x, w->cls_token, w->dist_token, w->pos_embed, d.B, d.N, D, d.prefix,
                          stream));
-  {
-    GemmProblem p;
-    p.A = sv.patches;
-    p.lda = d.Kp;
-    p.B = w->patch_w;
-    p.ldb = d.Kp;
-    p.M = static_cast<int>(d.Mp);
-    p.N = D;
-    p.K = d.Kp;
-    p.epi = EPI_RESID_F32;
-    p.e.bias = w->patch_b;
-    p.e.resid = w->pos_embed;
-    p.e.ldr = D;
-    p.e.out = ws.x;
-    p.e.ldo = D;
-    p.e.rows_per_group = d.P;
-    p.e.group_stride = d.N;
-    p.e.group_offset = d.prefix;
-    VITK_TRY(gemm_bf16_tn(p, stream));
-  }
+  VITK_TRY(patch_embed(sv.patches, w->patch_w, d.B, d.P, d.Kp, D, d.N, d.prefix, w->patch_b,
+                       w->pos_embed, ws.x, stream));
   const DropSet drop{cfg->dropout_p, static_cast<uint32_t>(cfg->seed)};
   if (drop.p > 0.f)   // nn.Dropout on tokens + position embedding (train.py:681)
     VITK_TRY(dropout_f32_inplace(ws.x, d.M * D, drop.at(DROP_EMBED, 0), stream));
@@ -272,17 +142,17 @@ int forward_train(const VitkConfig* cfg, const VitkWeights* w, const float* imag
     const DropParams drop_a = drop.at(DROP_ATTN, l);
     VITK_TRY(layernorm_fwd(ws.x, D, bw.ln1_w, bw.ln1_b, sb.xn1, 0, D, sb.mean1, sb.rstd1, M, D,
                            cfg->ln_eps, stream, sb.x1));
-    VITK_TRY(linear_fwd(sb.xn1, D, bw.qkv_w, M, 3 * D, D, EPI_BF16, bw.qkv_b, nullptr, sb.qkv,
+    VITK_TRY(linear_fwd(sb.xn1, D, bw.qkv_w, M, 3 * D, D, EPI_BF16, bw.qkv_b, nullptr, 0, sb.qkv,
                         nullptr, 3 * D, stream));
     VITK_TRY(attention_fwd(sb.qkv, sb.ctx, sb.lse, d.B, d.N, d.H, d.hd, stream, &drop_a));
-    VITK_TRY(linear_fwd(sb.ctx, D, bw.proj_w, M, D, D, EPI_RESID_F32, bw.proj_b, ws.x, ws.x,
+    VITK_TRY(linear_fwd(sb.ctx, D, bw.proj_w, M, D, D, EPI_RESID_F32, bw.proj_b, ws.x, D, ws.x,
                         nullptr, D, stream, drop.at(DROP_PROJ, l)));
     VITK_TRY(layernorm_fwd(ws.x, D, bw.ln2_w, bw.ln2_b, sb.xn2, 0, D, sb.mean2, sb.rstd2, M, D,
                            cfg->ln_eps, stream, sb.x2));
-    VITK_TRY(linear_fwd(sb.xn2, D, bw.fc1_w, M, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b, nullptr, sb.hact,
-                        sb.hpre, d.Mlp, stream, drop.at(DROP_GELU, l)));
-    VITK_TRY(linear_fwd(sb.hact, d.Mlp, bw.fc2_w, M, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.x, ws.x,
-                        nullptr, D, stream, drop.at(DROP_FC2, l)));
+    VITK_TRY(linear_fwd(sb.xn2, D, bw.fc1_w, M, d.Mlp, D, EPI_GELU_TANH_BF16, bw.fc1_b, nullptr, 0,
+                        sb.hact, sb.hpre, d.Mlp, stream, drop.at(DROP_GELU, l)));
+    VITK_TRY(linear_fwd(sb.hact, d.Mlp, bw.fc2_w, M, D, d.Mlp, EPI_RESID_F32, bw.fc2_b, ws.x, D,
+                        ws.x, nullptr, D, stream, drop.at(DROP_FC2, l)));
   }
   if (tokens_out)
     VITK_TRY(layernorm_fwd(ws.x, D, w->ln_f_w, w->ln_f_b, tokens_out, 1, D, sv.mean_f, sv.rstd_f, M,
@@ -293,7 +163,7 @@ int forward_train(const VitkConfig* cfg, const VitkWeights* w, const float* imag
 // Backward through the blocks and the patch embedding. On entry ws.dx (f32) / ws.dxb (bf16) hold
 // the gradient w.r.t. the residual stream after the last block.
 int backward_blocks(const VitkConfig* cfg, const VitkWeights* w, const VitkWeightsT* wt,
-                    const VitkGrads* g, const TDims& d, const Saved& sv, const TrainWs& ws,
+                    const VitkGrads* g, const Dims& d, const Saved& sv, const TrainWs& ws,
                     cudaStream_t stream, const vitk_event_t* bucket_events = nullptr) {
   const int M = static_cast<int>(d.M), D = d.D, Mlp = d.Mlp;
   const DropSet drop{cfg->dropout_p, static_cast<uint32_t>(cfg->seed)};
@@ -313,24 +183,24 @@ int backward_blocks(const VitkConfig* cfg, const VitkWeights* w, const VitkWeigh
     // of the block above (below), or here for the top block whose dxb came from the loss
     if (drop.p > 0.f && l == d.L - 1)
       VITK_TRY(dropout_cast_bf16(ws.dx, ws.dxb, d.M * D, drop.at(DROP_FC2, l), stream));
-    VITK_TRY(linear_dgrad(ws.dxb, D, bt.fc2_wt, M, Mlp, EPI_DGELU_BF16, sb.hpre, ws.dh, stream,
+    VITK_TRY(linear_dgrad(ws.dxb, D, bt.fc2_wt, M, Mlp, EPI_DGELU_BF16, sb.hpre, ws.dh, 0.f, stream,
                           drop.at(DROP_GELU, l)));
     // the bias gradient (column sums of ws.dxb) was produced together with ws.dxb by the
     // LayerNorm backward of the block above, unless dropout re-masked it or this is the top block
     VITK_TRY(linear_wgrad(ws.dxb, D, sb.hact, Mlp, M, bg.fc2_w, l == d.L - 1 ? bg.fc2_b : nullptr,
                           stream));
-    VITK_TRY(linear_dgrad(ws.dh, Mlp, bt.fc1_wt, M, D, EPI_BF16, nullptr, ws.dxn, stream));
+    VITK_TRY(linear_dgrad(ws.dh, Mlp, bt.fc1_wt, M, D, EPI_BF16, nullptr, ws.dxn, 0.f, stream));
     VITK_TRY(linear_wgrad(ws.dh, Mlp, sb.xn2, D, M, bg.fc1_w, bg.fc1_b, stream));
     const DropParams drop_p = drop.at(DROP_PROJ, l);   // ws.dxb enters the dropped projection output
     VITK_TRY(layernorm_bwd(ws.dxn, 0, D, sb.x2, D, sb.mean2, sb.rstd2, bw.ln2_w, ws.dx, D, 1, ws.dxb,
                            D, bg.ln2_w, bg.ln2_b, M, D, stream, bg.proj_b, &drop_p));
     // ---- attention branch: x2 = x1 + drop(proj(attn(qkv(LN1(x1)))))      (train.py:552-553,586-587)
-    VITK_TRY(linear_dgrad(ws.dxb, D, bt.proj_wt, M, D, EPI_BF16, nullptr, ws.dctx, stream));
+    VITK_TRY(linear_dgrad(ws.dxb, D, bt.proj_wt, M, D, EPI_BF16, nullptr, ws.dctx, 0.f, stream));
     VITK_TRY(linear_wgrad(ws.dxb, D, sb.ctx, D, M, bg.proj_w, nullptr, stream));
     const DropParams drop_a = drop.at(DROP_ATTN, l);
     VITK_TRY(attention_bwd(sb.qkv, sb.ctx, ws.dctx, sb.lse, ws.dqkv, d.B, d.N, d.H, d.hd, stream,
                            &drop_a, bg.qkv_b));   // also accumulates the qkv bias gradient
-    VITK_TRY(linear_dgrad(ws.dqkv, 3 * D, bt.qkv_wt, M, D, EPI_BF16, nullptr, ws.dxn, stream));
+    VITK_TRY(linear_dgrad(ws.dqkv, 3 * D, bt.qkv_wt, M, D, EPI_BF16, nullptr, ws.dxn, 0.f, stream));
     VITK_TRY(linear_wgrad(ws.dqkv, 3 * D, sb.xn1, D, M, bg.qkv_w, nullptr, stream));
     // ws.dxb next enters the (dropped) linear2 output of the block below
     const DropParams drop_f = l > 0 ? drop.at(DROP_FC2, l - 1) : DropParams();
@@ -350,7 +220,7 @@ int backward_blocks(const VitkConfig* cfg, const VitkWeights* w, const VitkWeigh
 }
 
 int check_train_ptrs(const VitkWeights* w, const VitkWeightsT* wt, const VitkGrads* g,
-                     const TDims& d) {
+                     const Dims& d) {
   VITK_REQUIRE(w && wt && g, "null weights / grads");
   VITK_REQUIRE(w->blocks && wt->blocks && g->blocks, "null block arrays");
   VITK_REQUIRE(g->patch_w && g->patch_b && g->cls_token && g->pos_embed && g->ln_f_w && g->ln_f_b,
@@ -376,7 +246,7 @@ int vitk_dropout_keep_mask(float p, unsigned int seed, int site, int layer, long
 
 int vitk_train_workspace_bytes(const VitkConfig* cfg, int batch, size_t* saved_bytes,
                                size_t* workspace_bytes) {
-  TDims d;
+  Dims d;
   VITK_TRY(check_train_config(cfg, batch, &d));
   VITK_REQUIRE(saved_bytes && workspace_bytes, "null output");
   *saved_bytes = carve_saved(d, nullptr).bytes;
@@ -387,7 +257,7 @@ int vitk_train_workspace_bytes(const VitkConfig* cfg, int batch, size_t* saved_b
 int vitk_forward_train(const VitkConfig* cfg, const VitkWeights* w, const float* images, int batch,
                        float* tokens_out, void* saved, size_t saved_bytes, void* workspace,
                        size_t workspace_bytes, vitk_stream_t stream) {
-  TDims d;
+  Dims d;
   VITK_TRY(check_train_config(cfg, batch, &d));
   VITK_REQUIRE(w && images && saved && workspace && w->blocks, "null argument");
   VITK_REQUIRE((reinterpret_cast<uintptr_t>(saved) & 1023) == 0 &&
@@ -416,7 +286,7 @@ int vitk_classifier_loss_backward_ev(const VitkConfig* cfg, const VitkWeights* w
                                      float* logits_out, float* loss_out, void* saved,
                                      void* workspace, const vitk_event_t* bucket_events,
                                      int n_events, vitk_stream_t stream_) {
-  TDims d;
+  Dims d;
   VITK_TRY(check_train_config(cfg, batch, &d));
   VITK_REQUIRE(bucket_events == nullptr || n_events == d.L + 2,
                "bucket_events needs num_layers + 2 = %d entries (got %d)", d.L + 2, n_events);
@@ -440,7 +310,7 @@ int vitk_classifier_loss_backward_ev(const VitkConfig* cfg, const VitkWeights* w
 int vitk_backward_tokens(const VitkConfig* cfg, const VitkWeights* w, const VitkWeightsT* wt,
                          const VitkGrads* g, const float* d_tokens, int batch, void* saved,
                          void* workspace, vitk_stream_t stream_) {
-  TDims d;
+  Dims d;
   VITK_TRY(check_train_config(cfg, batch, &d));
   VITK_TRY(check_train_ptrs(w, wt, g, d));
   VITK_REQUIRE(d_tokens && saved && workspace, "null argument");

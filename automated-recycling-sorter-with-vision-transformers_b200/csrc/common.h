@@ -1,6 +1,8 @@
 // Host-side plumbing shared by every translation unit of libvitk: error reporting that never
-// throws across the C ABI, launch accounting, device properties, TMA descriptor encoding.
+// throws across the C ABI, launch accounting, device properties, TMA descriptor encoding,
+// workspace carving.
 #pragma once
+#include <cstddef>
 #include <cstdint>
 #include <cstdio>
 #include <cuda.h>
@@ -46,6 +48,22 @@ const char* last_error();
 
 void count_launch();
 long long launch_count();
+
+inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Lays buffers out in a caller-provided workspace, one after the other in the order they are
+// taken, each at a 1024-byte aligned offset.  A null base hands out null pointers and only counts
+// the bytes (the workspace-size queries).
+struct Carver {
+  char* base;
+  size_t off = 0;
+  explicit Carver(void* b) : base(static_cast<char*>(b)) {}
+  void* take(size_t n) {
+    void* p = base ? base + off : nullptr;
+    off += align_up(n, 1024);
+    return p;
+  }
+};
 
 // Optional per-kernel-class timing (bench.py's roofline leg): when enabled, every launcher brackets
 // its kernel with CUDA events on the launching stream.  Off by default (zero overhead).

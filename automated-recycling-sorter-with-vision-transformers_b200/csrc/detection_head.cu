@@ -32,8 +32,6 @@ using namespace ptx;
 
 namespace {
 
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
 // ---------------------------------------------------------------------------------------------
 // Post-norm LayerNorm: y = LN(in[r % in_rows]) written twice, fp32 (the residual stream the next
 // GEMM reduce-adds into; may alias `in`) and bf16 (the next GEMM's operand).  in_rows < rows
@@ -180,24 +178,19 @@ struct HeadWorkspace {
 };
 
 HeadWorkspace carve(const HeadDims& d, void* base) {
+  Carver c(base);
   HeadWorkspace w;
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    void* p = base ? static_cast<char*>(base) + off : nullptr;
-    off += align_up(n, 1024);
-    return p;
-  };
   const size_t D = d.D;
-  w.x = static_cast<float*>(take(d.M * D * 4));
-  w.xb = take(d.M * D * 2);
-  w.qkv = take(d.M * 3 * D * 2);
-  w.ctx = take(d.M * D * 2);
-  w.h = take(d.M * static_cast<size_t>(d.F) * 2);
-  w.mem = take(d.Mm * D * 2);
-  w.kv = take(d.Mm * static_cast<size_t>(d.L) * 2 * D * 2);
-  w.xq = static_cast<float*>(take(static_cast<size_t>(d.Q) * D * 4));
-  w.xqb = take(static_cast<size_t>(d.Q) * D * 2);
-  w.bytes = off;
+  w.x = static_cast<float*>(c.take(d.M * D * 4));
+  w.xb = c.take(d.M * D * 2);
+  w.qkv = c.take(d.M * 3 * D * 2);
+  w.ctx = c.take(d.M * D * 2);
+  w.h = c.take(d.M * static_cast<size_t>(d.F) * 2);
+  w.mem = c.take(d.Mm * D * 2);
+  w.kv = c.take(d.Mm * static_cast<size_t>(d.L) * 2 * D * 2);
+  w.xq = static_cast<float*>(c.take(static_cast<size_t>(d.Q) * D * 4));
+  w.xqb = c.take(static_cast<size_t>(d.Q) * D * 2);
+  w.bytes = c.off;
   return w;
 }
 
@@ -237,27 +230,6 @@ int check(const VitkDetectionHeadConfig* cfg, int batch, int n_tokens, int skip,
   return VITK_OK;
 }
 
-int linear(const void* A, int lda, const void* W, int M, int N, int K, GemmEpi epi,
-           const float* bias, float* resid_out, void* out, int ldo, cudaStream_t stream,
-           const DropParams& drop = DropParams()) {
-  GemmProblem p;
-  p.e.drop = drop;
-  p.A = A;
-  p.lda = lda;
-  p.B = W;
-  p.ldb = K;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.epi = epi;
-  p.e.bias = bias;
-  p.e.resid = resid_out;
-  p.e.ldr = N;
-  p.e.out = (epi == EPI_RESID_F32) ? static_cast<void*>(resid_out) : out;
-  p.e.ldo = ldo;
-  return gemm_bf16_tn(p, stream);
-}
-
 int attn_x(const HeadDims& d, int B, const void* q, long long q_img, int ldq, const void* k,
            const void* v, long long kv_img, int ldkv, int Nk, void* ctx, cudaStream_t stream) {
   const long long ctx_img = static_cast<long long>(d.Q) * d.D;
@@ -281,8 +253,8 @@ int head_forward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWeig
   //    layer's multihead_attn in one GEMM (rows of the skipped prefix tokens are computed and
   //    never read)
   VITK_TRY(cast_f32_to_bf16(tokens, ws.mem, d.Mm * D, stream));
-  VITK_TRY(linear(ws.mem, D, w->ca_kv_w, static_cast<int>(d.Mm), ldkv, D, EPI_BF16, w->ca_kv_b,
-                  nullptr, ws.kv, ldkv, stream));
+  VITK_TRY(linear_fwd(ws.mem, D, w->ca_kv_w, static_cast<int>(d.Mm), ldkv, D, EPI_BF16, w->ca_kv_b,
+                      nullptr, 0, ws.kv, nullptr, ldkv, stream));
   for (int l = 0; l < d.L; ++l) {
     const VitkDecoderLayerWeights& lw = w->layers[l];
     // ---- x = norm1(x + self_attn(x, x, x))
@@ -292,36 +264,37 @@ int head_forward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWeig
       VITK_CHECK_CUDA(cudaMemcpyAsync(ws.xq, w->object_queries, static_cast<size_t>(Q) * D * 4,
                                       cudaMemcpyDeviceToDevice, stream));
       VITK_TRY(cast_f32_to_bf16(w->object_queries, ws.xqb, static_cast<long long>(Q) * D, stream));
-      VITK_TRY(linear(ws.xqb, D, lw.sa_in_w, Q, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, ws.qkv,
-                      3 * D, stream));
+      VITK_TRY(linear_fwd(ws.xqb, D, lw.sa_in_w, Q, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, 0,
+                          ws.qkv, nullptr, 3 * D, stream));
       VITK_TRY(attn_x(d, 1, qkv, 0, 3 * D, qkv + D, qkv + 2 * D, 0, 3 * D, Q, ws.ctx, stream));
-      VITK_TRY(linear(ws.ctx, D, lw.sa_out_w, Q, D, D, EPI_RESID_F32, lw.sa_out_b, ws.xq, nullptr,
-                      D, stream));
+      VITK_TRY(linear_fwd(ws.ctx, D, lw.sa_out_w, Q, D, D, EPI_RESID_F32, lw.sa_out_b, ws.xq, D,
+                          ws.xq, nullptr, D, stream));
       VITK_TRY(ln_post(ws.xq, Q, lw.norm1_w, lw.norm1_b, ws.x, ws.xb, M, D, cfg->ln_eps, stream));
     } else {
-      VITK_TRY(linear(ws.xb, D, lw.sa_in_w, M, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, ws.qkv,
-                      3 * D, stream));
+      VITK_TRY(linear_fwd(ws.xb, D, lw.sa_in_w, M, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, 0,
+                          ws.qkv, nullptr, 3 * D, stream));
       const long long img = static_cast<long long>(Q) * 3 * D;
       VITK_TRY(attn_x(d, d.B, qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D, Q, ws.ctx, stream));
-      VITK_TRY(linear(ws.ctx, D, lw.sa_out_w, M, D, D, EPI_RESID_F32, lw.sa_out_b, ws.x, nullptr, D,
-                      stream));
+      VITK_TRY(linear_fwd(ws.ctx, D, lw.sa_out_w, M, D, D, EPI_RESID_F32, lw.sa_out_b, ws.x, D,
+                          ws.x, nullptr, D, stream));
       VITK_TRY(ln_post(ws.x, M, lw.norm1_w, lw.norm1_b, ws.x, ws.xb, M, D, cfg->ln_eps, stream));
     }
     // ---- x = norm2(x + multihead_attn(x, memory, memory))
-    VITK_TRY(linear(ws.xb, D, lw.ca_q_w, M, D, D, EPI_BF16, lw.ca_q_b, nullptr, ws.qkv, D, stream));
+    VITK_TRY(linear_fwd(ws.xb, D, lw.ca_q_w, M, D, D, EPI_BF16, lw.ca_q_b, nullptr, 0, ws.qkv,
+                        nullptr, D, stream));
     {
       const __nv_bfloat16* kl = kv + static_cast<size_t>(d.skip) * ldkv + static_cast<size_t>(l) * 2 * D;
       VITK_TRY(attn_x(d, d.B, qkv, static_cast<long long>(Q) * D, D, kl, kl + D,
                       static_cast<long long>(d.Ntok) * ldkv, ldkv, d.P, ws.ctx, stream));
     }
-    VITK_TRY(linear(ws.ctx, D, lw.ca_out_w, M, D, D, EPI_RESID_F32, lw.ca_out_b, ws.x, nullptr, D,
-                    stream));
+    VITK_TRY(linear_fwd(ws.ctx, D, lw.ca_out_w, M, D, D, EPI_RESID_F32, lw.ca_out_b, ws.x, D, ws.x,
+                        nullptr, D, stream));
     VITK_TRY(ln_post(ws.x, M, lw.norm2_w, lw.norm2_b, ws.x, ws.xb, M, D, cfg->ln_eps, stream));
     // ---- x = norm3(x + linear2(relu(linear1(x))))
-    VITK_TRY(linear(ws.xb, D, lw.ff1_w, M, d.F, D, EPI_RELU_BF16, lw.ff1_b, nullptr, ws.h, d.F,
-                    stream));
-    VITK_TRY(linear(ws.h, d.F, lw.ff2_w, M, D, d.F, EPI_RESID_F32, lw.ff2_b, ws.x, nullptr, D,
-                    stream));
+    VITK_TRY(linear_fwd(ws.xb, D, lw.ff1_w, M, d.F, D, EPI_RELU_BF16, lw.ff1_b, nullptr, 0, ws.h,
+                        nullptr, d.F, stream));
+    VITK_TRY(linear_fwd(ws.h, d.F, lw.ff2_w, M, D, d.F, EPI_RESID_F32, lw.ff2_b, ws.x, D, ws.x,
+                        nullptr, D, stream));
     VITK_TRY(ln_post(ws.x, M, lw.norm3_w, lw.norm3_b, ws.x, ws.xb, M, D, cfg->ln_eps, stream));
   }
   {
@@ -359,55 +332,45 @@ struct SavedHead {
 };
 
 SavedLayer carve_layer(const HeadDims& d, int l, char* base, size_t* bytes) {
+  Carver c(base);
   SavedLayer s;
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    void* p = base ? base + off : nullptr;
-    off += align_up(n, 1024);
-    return p;
-  };
   // every layer gets the same (largest) layout so that layer_bytes is one number
   (void)l;
   const size_t M = d.M, D = d.D, F = d.F;
-  s.xb_in = take(M * D * 2);
-  s.qkv = take(M * 3 * D * 2);
-  s.ctx_sa = take(M * D * 2);
-  s.lse_sa = static_cast<float*>(take(static_cast<size_t>(d.B) * d.H * d.Q * 4));
-  s.r1 = static_cast<float*>(take(M * D * 4));
-  s.mean1 = static_cast<float*>(take(M * 4));
-  s.rstd1 = static_cast<float*>(take(M * 4));
-  s.xb1 = take(M * D * 2);
-  s.qc = take(M * D * 2);
-  s.ctx_ca = take(M * D * 2);
-  s.lse_ca = static_cast<float*>(take(static_cast<size_t>(d.B) * d.H * d.Q * 4));
-  s.r2 = static_cast<float*>(take(M * D * 4));
-  s.mean2 = static_cast<float*>(take(M * 4));
-  s.rstd2 = static_cast<float*>(take(M * 4));
-  s.xb2 = take(M * D * 2);
-  s.h = take(M * F * 2);
-  s.r3 = static_cast<float*>(take(M * D * 4));
-  s.mean3 = static_cast<float*>(take(M * 4));
-  s.rstd3 = static_cast<float*>(take(M * 4));
-  if (bytes) *bytes = off;
+  s.xb_in = c.take(M * D * 2);
+  s.qkv = c.take(M * 3 * D * 2);
+  s.ctx_sa = c.take(M * D * 2);
+  s.lse_sa = static_cast<float*>(c.take(static_cast<size_t>(d.B) * d.H * d.Q * 4));
+  s.r1 = static_cast<float*>(c.take(M * D * 4));
+  s.mean1 = static_cast<float*>(c.take(M * 4));
+  s.rstd1 = static_cast<float*>(c.take(M * 4));
+  s.xb1 = c.take(M * D * 2);
+  s.qc = c.take(M * D * 2);
+  s.ctx_ca = c.take(M * D * 2);
+  s.lse_ca = static_cast<float*>(c.take(static_cast<size_t>(d.B) * d.H * d.Q * 4));
+  s.r2 = static_cast<float*>(c.take(M * D * 4));
+  s.mean2 = static_cast<float*>(c.take(M * 4));
+  s.rstd2 = static_cast<float*>(c.take(M * 4));
+  s.xb2 = c.take(M * D * 2);
+  s.h = c.take(M * F * 2);
+  s.r3 = static_cast<float*>(c.take(M * D * 4));
+  s.mean3 = static_cast<float*>(c.take(M * 4));
+  s.rstd3 = static_cast<float*>(c.take(M * 4));
+  if (bytes) *bytes = c.off;
   return s;
 }
 
 SavedHead carve_saved(const HeadDims& d, void* base) {
+  Carver c(base);
   SavedHead s;
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    void* p = base ? static_cast<char*>(base) + off : nullptr;
-    off += align_up(n, 1024);
-    return p;
-  };
   const size_t D = d.D;
-  s.mem = take(d.Mm * D * 2);
-  s.kv = take(d.Mm * static_cast<size_t>(d.L) * 2 * D * 2);
-  s.xfinal = static_cast<float*>(take(d.M * D * 4));
-  s.xb_last = take(d.M * D * 2);
+  s.mem = c.take(d.Mm * D * 2);
+  s.kv = c.take(d.Mm * static_cast<size_t>(d.L) * 2 * D * 2);
+  s.xfinal = static_cast<float*>(c.take(d.M * D * 4));
+  s.xb_last = c.take(d.M * D * 2);
   carve_layer(d, 0, nullptr, &s.layer_bytes);
-  s.layers = static_cast<char*>(take(s.layer_bytes * d.L));
-  s.bytes = off;
+  s.layers = static_cast<char*>(c.take(s.layer_bytes * d.L));
+  s.bytes = c.off;
   return s;
 }
 
@@ -425,24 +388,19 @@ struct HeadTrainWs {
 };
 
 HeadTrainWs carve_train_ws(const HeadDims& d, void* base) {
+  Carver c(base);
   HeadTrainWs w;
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    void* p = base ? static_cast<char*>(base) + off : nullptr;
-    off += align_up(n, 1024);
-    return p;
-  };
   const size_t D = d.D;
-  w.x = static_cast<float*>(take(d.M * D * 4));
-  w.xq = static_cast<float*>(take(static_cast<size_t>(d.Q) * D * 4));
-  w.dxb = take(d.M * D * 2);
-  w.dh = take(d.M * static_cast<size_t>(d.F) * 2);
-  w.dctx = take(d.M * D * 2);
-  w.dqkv = take(d.M * 3 * D * 2);
-  w.dkv = take(d.Mm * static_cast<size_t>(d.L) * 2 * D * 2);
-  w.dsumb = take(static_cast<size_t>(d.Q) * D * 2);
-  w.dz = static_cast<float*>(take(d.M * static_cast<size_t>(d.C + 4) * 4));
-  w.bytes = off;
+  w.x = static_cast<float*>(c.take(d.M * D * 4));
+  w.xq = static_cast<float*>(c.take(static_cast<size_t>(d.Q) * D * 4));
+  w.dxb = c.take(d.M * D * 2);
+  w.dh = c.take(d.M * static_cast<size_t>(d.F) * 2);
+  w.dctx = c.take(d.M * D * 2);
+  w.dqkv = c.take(d.M * 3 * D * 2);
+  w.dkv = c.take(d.Mm * static_cast<size_t>(d.L) * 2 * D * 2);
+  w.dsumb = c.take(static_cast<size_t>(d.Q) * D * 2);
+  w.dz = static_cast<float*>(c.take(d.M * static_cast<size_t>(d.C + 4) * 4));
+  w.bytes = c.off;
   return w;
 }
 
@@ -492,8 +450,8 @@ int head_forward_train(const VitkDetectionHeadConfig* cfg, const VitkDetectionHe
   const __nv_bfloat16* kv = static_cast<const __nv_bfloat16*>(sv.kv);
   const int ldkv = d.L * 2 * D;
   VITK_TRY(cast_f32_to_bf16(tokens, sv.mem, d.Mm * D, stream));
-  VITK_TRY(linear(sv.mem, D, w->ca_kv_w, static_cast<int>(d.Mm), ldkv, D, EPI_BF16, w->ca_kv_b,
-                  nullptr, sv.kv, ldkv, stream));
+  VITK_TRY(linear_fwd(sv.mem, D, w->ca_kv_w, static_cast<int>(d.Mm), ldkv, D, EPI_BF16, w->ca_kv_b,
+                      nullptr, 0, sv.kv, nullptr, ldkv, stream));
   for (int l = 0; l < d.L; ++l) {
     const VitkDecoderLayerWeights& lw = w->layers[l];
     const SavedLayer sl = carve_layer(d, l, sv.layers + l * sv.layer_bytes, nullptr);
@@ -507,28 +465,29 @@ int head_forward_train(const VitkDetectionHeadConfig* cfg, const VitkDetectionHe
       VITK_CHECK_CUDA(cudaMemcpyAsync(ws.xq, w->object_queries, static_cast<size_t>(Q) * D * 4,
                                       cudaMemcpyDeviceToDevice, stream));
       VITK_TRY(cast_f32_to_bf16(w->object_queries, sl.xb_in, static_cast<long long>(Q) * D, stream));
-      VITK_TRY(linear(sl.xb_in, D, lw.sa_in_w, Q, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, sl.qkv,
-                      3 * D, stream));
+      VITK_TRY(linear_fwd(sl.xb_in, D, lw.sa_in_w, Q, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, 0,
+                          sl.qkv, nullptr, 3 * D, stream));
       const AttnXSrc src{qkv, 0, 3 * D, qkv + D, qkv + 2 * D, 0, 3 * D};
       VITK_TRY(attn_train(d, 1, src, Q, sl.ctx_sa, sl.lse_sa, stream));
-      VITK_TRY(linear(sl.ctx_sa, D, lw.sa_out_w, Q, D, D, EPI_RESID_F32, lw.sa_out_b, ws.xq, nullptr,
-                      D, stream));
+      VITK_TRY(linear_fwd(sl.ctx_sa, D, lw.sa_out_w, Q, D, D, EPI_RESID_F32, lw.sa_out_b, ws.xq, D,
+                          ws.xq, nullptr, D, stream));
       VITK_TRY(ln_post(ws.xq, Q, lw.norm1_w, lw.norm1_b, ws.x, sl.xb1, M, D, cfg->ln_eps, stream,
                        sl.r1, sl.mean1, sl.rstd1));
     } else {
       // sl.xb_in was written by the previous layer's norm3
-      VITK_TRY(linear(sl.xb_in, D, lw.sa_in_w, M, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, sl.qkv,
-                      3 * D, stream));
+      VITK_TRY(linear_fwd(sl.xb_in, D, lw.sa_in_w, M, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, 0,
+                          sl.qkv, nullptr, 3 * D, stream));
       const long long img = static_cast<long long>(Q) * 3 * D;
       const AttnXSrc src{qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D};
       VITK_TRY(attn_train(d, d.B, src, Q, sl.ctx_sa, sl.lse_sa, stream,
                           drop.at(DROP_DEC_SA_ATTN, l)));
-      VITK_TRY(linear(sl.ctx_sa, D, lw.sa_out_w, M, D, D, EPI_RESID_F32, lw.sa_out_b, ws.x, nullptr,
-                      D, stream, drop.at(DROP_DEC_SA_OUT, l)));
+      VITK_TRY(linear_fwd(sl.ctx_sa, D, lw.sa_out_w, M, D, D, EPI_RESID_F32, lw.sa_out_b, ws.x, D,
+                          ws.x, nullptr, D, stream, drop.at(DROP_DEC_SA_OUT, l)));
       VITK_TRY(ln_post(ws.x, M, lw.norm1_w, lw.norm1_b, ws.x, sl.xb1, M, D, cfg->ln_eps, stream,
                        sl.r1, sl.mean1, sl.rstd1));
     }
-    VITK_TRY(linear(sl.xb1, D, lw.ca_q_w, M, D, D, EPI_BF16, lw.ca_q_b, nullptr, sl.qc, D, stream));
+    VITK_TRY(linear_fwd(sl.xb1, D, lw.ca_q_w, M, D, D, EPI_BF16, lw.ca_q_b, nullptr, 0, sl.qc,
+                        nullptr, D, stream));
     {
       const __nv_bfloat16* kl = kv + static_cast<size_t>(d.skip) * ldkv + static_cast<size_t>(l) * 2 * D;
       const AttnXSrc src{sl.qc, static_cast<long long>(Q) * D, D, kl, kl + D,
@@ -536,14 +495,14 @@ int head_forward_train(const VitkDetectionHeadConfig* cfg, const VitkDetectionHe
       VITK_TRY(attn_train(d, d.B, src, d.P, sl.ctx_ca, sl.lse_ca, stream,
                           drop.at(DROP_DEC_CA_ATTN, l)));
     }
-    VITK_TRY(linear(sl.ctx_ca, D, lw.ca_out_w, M, D, D, EPI_RESID_F32, lw.ca_out_b, ws.x, nullptr, D,
-                    stream, drop.at(DROP_DEC_CA_OUT, l)));
+    VITK_TRY(linear_fwd(sl.ctx_ca, D, lw.ca_out_w, M, D, D, EPI_RESID_F32, lw.ca_out_b, ws.x, D,
+                        ws.x, nullptr, D, stream, drop.at(DROP_DEC_CA_OUT, l)));
     VITK_TRY(ln_post(ws.x, M, lw.norm2_w, lw.norm2_b, ws.x, sl.xb2, M, D, cfg->ln_eps, stream, sl.r2,
                      sl.mean2, sl.rstd2));
-    VITK_TRY(linear(sl.xb2, D, lw.ff1_w, M, d.F, D, EPI_RELU_BF16, lw.ff1_b, nullptr, sl.h, d.F,
-                    stream, drop.at(DROP_DEC_FFN, l)));
-    VITK_TRY(linear(sl.h, d.F, lw.ff2_w, M, D, d.F, EPI_RESID_F32, lw.ff2_b, ws.x, nullptr, D, stream,
-                    drop.at(DROP_DEC_FF2, l)));
+    VITK_TRY(linear_fwd(sl.xb2, D, lw.ff1_w, M, d.F, D, EPI_RELU_BF16, lw.ff1_b, nullptr, 0, sl.h,
+                        nullptr, d.F, stream, drop.at(DROP_DEC_FFN, l)));
+    VITK_TRY(linear_fwd(sl.h, d.F, lw.ff2_w, M, D, d.F, EPI_RESID_F32, lw.ff2_b, ws.x, D, ws.x,
+                        nullptr, D, stream, drop.at(DROP_DEC_FF2, l)));
     const bool last = (l == d.L - 1);
     void* xb_next = last ? sv.xb_last
                          : carve_layer(d, l + 1, sv.layers + (l + 1) * sv.layer_bytes, nullptr).xb_in;
@@ -687,52 +646,6 @@ int attn_bwd_x(const AttnXSrc& s, const void* ctx, const void* dctx, long long c
                             lddkv, B, Nq, Nk, H, hd, stream, drop);
 }
 
-// dX[M, in] = dY[M, out] W[out, in] with W^T [in, out] as the K-major B operand; bf16 out, or
-// accumulated into an fp32 stream (TMA reduce-add) / written as fp32
-int dgrad(const void* dY, int out_f, const void* Wt, int M, int in_f, void* dX_bf16, float* dX_f32,
-          float beta, cudaStream_t stream) {
-  GemmProblem p;
-  p.A = dY;
-  p.lda = out_f;
-  p.B = Wt;
-  p.ldb = out_f;
-  p.M = M;
-  p.N = in_f;
-  p.K = out_f;
-  p.epi = dX_bf16 != nullptr ? EPI_BF16 : EPI_F32;
-  p.e.out = dX_bf16 != nullptr ? dX_bf16 : static_cast<void*>(dX_f32);
-  p.e.ldo = in_f;
-  p.e.beta = beta;
-  return gemm_bf16_tn(p, stream);
-}
-
-// dW[out, in] += dY[rows, out]^T X[rows, in]; db[out] += column sums of dY
-int wgrad(const void* dY, int out_f, const void* X, int in_f, int rows, float* dW, float* db,
-          cudaStream_t stream) {
-  GemmProblem p;
-  p.A = dY;
-  p.lda = out_f;
-  p.B = X;
-  p.ldb = in_f;
-  p.M = out_f;
-  p.N = in_f;
-  p.K = rows;
-  p.epi = EPI_F32;
-  p.mn_major = true;
-  p.e.out = dW;
-  p.e.ldo = in_f;
-  p.e.beta = 1.f;
-  const int tiles = ((out_f + 255) / 256) * ((in_f + 255) / 256);
-  int split = (sm_count() / 2 * 2) / (tiles > 0 ? tiles : 1);
-  if (split < 1) split = 1;
-  const int num_kb = (rows + 63) / 64;
-  if (split > num_kb / 4) split = num_kb / 4 > 0 ? num_kb / 4 : 1;
-  p.split_k = split;
-  VITK_TRY(gemm_bf16_tn(p, stream));
-  if (db != nullptr) VITK_TRY(colsum_bf16(dY, out_f, rows, out_f, db, stream));
-  return VITK_OK;
-}
-
 // norm backward in place on the fp32 gradient stream: dx <- LN'(dx), bf16 copy, dgamma / dbeta
 // accumulated, column sums of the result into `colsum` (the bias gradient of the Linear whose
 // output the normalised sum received)
@@ -779,7 +692,7 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
     // ---- x = norm3(x2 + linear2(relu(linear1(x2))))
     VITK_TRY(norm_bwd(ws.x, ws.dxb, sl.r3, sl.mean3, sl.rstd3, lw.norm3_w, lg.norm3_w, lg.norm3_b,
                       lg.ff2_b, M, D, stream, drop.at(DROP_DEC_FF2, l)));
-    VITK_TRY(dgrad(ws.dxb, D, lt.ff2_wt, M, F, ws.dh, nullptr, 0.f, stream));
+    VITK_TRY(linear_dgrad(ws.dxb, D, lt.ff2_wt, M, F, EPI_BF16, nullptr, ws.dh, 0.f, stream));
     {
       const long long n8 = static_cast<long long>(M) * F / 8;
       ProfileScope prof(PROF_OTHER, static_cast<double>(M) * F * 6.0, stream);
@@ -788,14 +701,14 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
           drop.at(DROP_DEC_FFN, l).scale);
       VITK_CHECK_LAUNCH("relu_bwd_kernel");
     }
-    VITK_TRY(wgrad(ws.dxb, D, sl.h, F, M, lg.ff2_w, nullptr, stream));
-    VITK_TRY(dgrad(ws.dh, F, lt.ff1_wt, M, D, nullptr, ws.x, 1.f, stream));
-    VITK_TRY(wgrad(ws.dh, F, sl.xb2, D, M, lg.ff1_w, lg.ff1_b, stream));
+    VITK_TRY(linear_wgrad(ws.dxb, D, sl.h, F, M, lg.ff2_w, nullptr, stream));
+    VITK_TRY(linear_dgrad(ws.dh, F, lt.ff1_wt, M, D, EPI_F32, nullptr, ws.x, 1.f, stream));
+    VITK_TRY(linear_wgrad(ws.dh, F, sl.xb2, D, M, lg.ff1_w, lg.ff1_b, stream));
     // ---- x2 = norm2(x1 + multihead_attn(x1, memory, memory))
     VITK_TRY(norm_bwd(ws.x, ws.dxb, sl.r2, sl.mean2, sl.rstd2, lw.norm2_w, lg.norm2_w, lg.norm2_b,
                       lg.ca_out_b, M, D, stream, drop.at(DROP_DEC_CA_OUT, l)));
-    VITK_TRY(dgrad(ws.dxb, D, lt.ca_out_wt, M, D, ws.dctx, nullptr, 0.f, stream));
-    VITK_TRY(wgrad(ws.dxb, D, sl.ctx_ca, D, M, lg.ca_out_w, nullptr, stream));
+    VITK_TRY(linear_dgrad(ws.dxb, D, lt.ca_out_wt, M, D, EPI_BF16, nullptr, ws.dctx, 0.f, stream));
+    VITK_TRY(linear_wgrad(ws.dxb, D, sl.ctx_ca, D, M, lg.ca_out_w, nullptr, stream));
     {
       const size_t koff = static_cast<size_t>(d.skip) * ldkv + static_cast<size_t>(l) * 2 * D;
       const AttnXSrc src{sl.qc, imgD, D, kv + koff, kv + koff + D,
@@ -805,14 +718,15 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
                                   dkv + koff, dkv + koff + D, static_cast<long long>(d.Ntok) * ldkv,
                                   ldkv, d.B, Q, d.P, d.H, d.hd, stream, &drop_ca));
     }
-    VITK_TRY(dgrad(dqkv, D, lt.ca_q_wt, M, D, nullptr, ws.x, 1.f, stream));
-    VITK_TRY(wgrad(dqkv, D, sl.xb1, D, M, lg.ca_q_w, lg.ca_q_b, stream));
+    VITK_TRY(linear_dgrad(dqkv, D, lt.ca_q_wt, M, D, EPI_F32, nullptr, ws.x, 1.f, stream));
+    VITK_TRY(linear_wgrad(dqkv, D, sl.xb1, D, M, lg.ca_q_w, lg.ca_q_b, stream));
     // ---- x1 = norm1(x0 + self_attn(x0, x0, x0))
     if (l > 0 || drop.on()) {
       VITK_TRY(norm_bwd(ws.x, ws.dxb, sl.r1, sl.mean1, sl.rstd1, lw.norm1_w, lg.norm1_w, lg.norm1_b,
                         lg.sa_out_b, M, D, stream, drop.at(DROP_DEC_SA_OUT, l)));
-      VITK_TRY(dgrad(ws.dxb, D, lt.sa_out_wt, M, D, ws.dctx, nullptr, 0.f, stream));
-      VITK_TRY(wgrad(ws.dxb, D, sl.ctx_sa, D, M, lg.sa_out_w, nullptr, stream));
+      VITK_TRY(linear_dgrad(ws.dxb, D, lt.sa_out_wt, M, D, EPI_BF16, nullptr, ws.dctx, 0.f,
+                            stream));
+      VITK_TRY(linear_wgrad(ws.dxb, D, sl.ctx_sa, D, M, lg.sa_out_w, nullptr, stream));
       const __nv_bfloat16* qkv = static_cast<const __nv_bfloat16*>(sl.qkv);
       const long long img = static_cast<long long>(Q) * 3 * D;
       const AttnXSrc src{qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D};
@@ -820,8 +734,8 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
       VITK_TRY(attn_bwd_x(src, sl.ctx_sa, ws.dctx, imgD, D, sl.lse_sa, dqkv, img, 3 * D,
                                   dqkv + D, dqkv + 2 * D, img, 3 * D, d.B, Q, Q, d.H, d.hd, stream,
                                   &drop_sa));
-      VITK_TRY(dgrad(dqkv, 3 * D, lt.sa_in_wt, M, D, nullptr, ws.x, 1.f, stream));
-      VITK_TRY(wgrad(dqkv, 3 * D, sl.xb_in, D, M, lg.sa_in_w, lg.sa_in_b, stream));
+      VITK_TRY(linear_dgrad(dqkv, 3 * D, lt.sa_in_wt, M, D, EPI_F32, nullptr, ws.x, 1.f, stream));
+      VITK_TRY(linear_wgrad(dqkv, 3 * D, sl.xb_in, D, M, lg.sa_in_w, lg.sa_in_b, stream));
       if (l == 0) {
         // (dropout: layer 0 ran on every image's own copy of the queries) d queries = sum over images
         batch_sum_kernel<<<static_cast<unsigned>((imgD / 4 + 255) / 256), 256, 0, stream>>>(
@@ -842,14 +756,15 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
       }
       VITK_TRY(norm_bwd(ws.xq, ws.dsumb, sl.r1, sl.mean1, sl.rstd1, lw.norm1_w, lg.norm1_w,
                         lg.norm1_b, lg.sa_out_b, Q, D, stream));
-      VITK_TRY(dgrad(ws.dsumb, D, lt.sa_out_wt, Q, D, ws.dctx, nullptr, 0.f, stream));
-      VITK_TRY(wgrad(ws.dsumb, D, sl.ctx_sa, D, Q, lg.sa_out_w, nullptr, stream));
+      VITK_TRY(linear_dgrad(ws.dsumb, D, lt.sa_out_wt, Q, D, EPI_BF16, nullptr, ws.dctx, 0.f,
+                            stream));
+      VITK_TRY(linear_wgrad(ws.dsumb, D, sl.ctx_sa, D, Q, lg.sa_out_w, nullptr, stream));
       const __nv_bfloat16* qkv = static_cast<const __nv_bfloat16*>(sl.qkv);
       const AttnXSrc src{qkv, 0, 3 * D, qkv + D, qkv + 2 * D, 0, 3 * D};
       VITK_TRY(attn_bwd_x(src, sl.ctx_sa, ws.dctx, 0, D, sl.lse_sa, dqkv, 0, 3 * D, dqkv + D,
                           dqkv + 2 * D, 0, 3 * D, 1, Q, Q, d.H, d.hd, stream, nullptr));
-      VITK_TRY(dgrad(dqkv, 3 * D, lt.sa_in_wt, Q, D, nullptr, ws.xq, 1.f, stream));
-      VITK_TRY(wgrad(dqkv, 3 * D, sl.xb_in, D, Q, lg.sa_in_w, lg.sa_in_b, stream));
+      VITK_TRY(linear_dgrad(dqkv, 3 * D, lt.sa_in_wt, Q, D, EPI_F32, nullptr, ws.xq, 1.f, stream));
+      VITK_TRY(linear_wgrad(dqkv, 3 * D, sl.xb_in, D, Q, lg.sa_in_w, lg.sa_in_b, stream));
       accumulate_kernel<<<static_cast<unsigned>((imgD + 255) / 256), 256, 0, stream>>>(
           g->object_queries, ws.xq, imgD);
       VITK_CHECK_LAUNCH("accumulate_kernel");
@@ -857,9 +772,10 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
   }
   // ---- K / V projections of the memory (all layers at once) and the encoder features
   if (d_tokens != nullptr)
-    VITK_TRY(dgrad(ws.dkv, ldkv, wt->ca_kv_wt, static_cast<int>(d.Mm), D, nullptr, d_tokens, 0.f,
-                   stream));
-  VITK_TRY(wgrad(ws.dkv, ldkv, sv.mem, D, static_cast<int>(d.Mm), g->ca_kv_w, g->ca_kv_b, stream));
+    VITK_TRY(linear_dgrad(ws.dkv, ldkv, wt->ca_kv_wt, static_cast<int>(d.Mm), D, EPI_F32, nullptr,
+                          d_tokens, 0.f, stream));
+  VITK_TRY(linear_wgrad(ws.dkv, ldkv, sv.mem, D, static_cast<int>(d.Mm), g->ca_kv_w, g->ca_kv_b,
+                        stream));
   return VITK_OK;
 }
 

@@ -13,12 +13,17 @@
 //                     by TMA (bulk tensor store; the fp32 residual update x += acc + bias is a
 //                     TMA reduce-add, so the residual stream is never read by the SM).  A direct
 //                     register->global path remains for the token-row remap of the patch embed.
+//
+// After gemm_bf16_tn, at the end of the file: the host-side GEMM calls that the encoder, training
+// and detection-head drivers share (linear_fwd, linear_dgrad, linear_wgrad, ...).
 #include "gemm_sm100.cuh"
 
 #include <mutex>
 
 #include "common.h"
 #include "ptx.cuh"
+#include "rowops.cuh"
+#include "train_ops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -1319,6 +1324,167 @@ int gemm_bf16_tn(const GemmProblem& p, cudaStream_t stream) {
       return dispatch<EPI_DGELU_BF16>(p, stream);
     default: return set_error(VITK_ERR_INVALID, "gemm: unknown epilogue %d", (int)p.epi);
   }
+}
+
+int linear_fwd(const void* A, int lda, const void* W, int M, int N, int K, GemmEpi epi,
+               const float* bias, const float* resid, int ldr, void* out, void* out2, int ldo,
+               cudaStream_t stream, const DropParams& drop) {
+  GemmProblem p;
+  p.A = A;
+  p.lda = lda;
+  p.B = W;
+  p.ldb = K;
+  p.M = M;
+  p.N = N;
+  p.K = K;
+  p.epi = epi;
+  p.e.bias = bias;
+  p.e.resid = resid;
+  p.e.ldr = ldr;
+  p.e.out = out;
+  p.e.out2 = out2;
+  p.e.ldo = ldo;
+  p.e.drop = drop;
+  return gemm_bf16_tn(p, stream);
+}
+
+int linear_dgrad(const void* dY, int out_f, const void* Wt, int M, int in_f, GemmEpi epi,
+                 const void* aux, void* dX, float beta, cudaStream_t stream,
+                 const DropParams& drop) {
+  GemmProblem p;
+  p.A = dY;
+  p.lda = out_f;
+  p.B = Wt;
+  p.ldb = out_f;
+  p.M = M;
+  p.N = in_f;
+  p.K = out_f;
+  p.epi = epi;
+  p.e.aux = aux;
+  p.e.out = dX;
+  p.e.ldo = in_f;
+  p.e.beta = beta;
+  p.e.drop = drop;
+  return gemm_bf16_tn(p, stream);
+}
+
+int gemm_wgrad(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* out,
+               int ldo, float alpha, float beta, int split_k, cudaStream_t stream) {
+  GemmProblem p;
+  p.A = A;
+  p.lda = lda;
+  p.B = B;
+  p.ldb = ldb;
+  p.M = M;
+  p.N = N;
+  p.K = K;
+  p.epi = EPI_F32;
+  p.mn_major = true;
+  p.split_k = split_k;
+  p.e.out = out;
+  p.e.ldo = ldo;
+  p.e.alpha = alpha;
+  p.e.beta = beta;
+  return gemm_bf16_tn(p, stream);
+}
+
+int linear_wgrad(const void* dY, int out_f, const void* X, int in_f, int rows, float* dW,
+                 float* db, cudaStream_t stream) {
+  // enough K splits to give every CTA pair about two work items
+  const int tiles = ((out_f + 255) / 256) * ((in_f + 255) / 256);
+  int split = (sm_count() / 2 * 2) / (tiles > 0 ? tiles : 1);
+  if (split < 1) split = 1;
+  const int num_kb = (rows + 63) / 64;
+  if (split > num_kb / 4) split = num_kb / 4 > 0 ? num_kb / 4 : 1;
+  VITK_TRY(gemm_wgrad(dY, out_f, X, in_f, out_f, in_f, rows, dW, in_f, 1.f, 1.f, split, stream));
+  if (db != nullptr) VITK_TRY(colsum_bf16(dY, out_f, rows, out_f, db, stream));
+  return VITK_OK;
+}
+
+int patch_embed(const void* patches, const void* W, int B, int P, int K, int D, int N, int prefix,
+                const float* bias, const float* pos_embed, float* x, cudaStream_t stream) {
+  GemmProblem p;
+  p.A = patches;
+  p.lda = K;
+  p.B = W;
+  p.ldb = K;
+  p.M = B * P;
+  p.N = D;
+  p.K = K;
+  p.epi = EPI_RESID_F32;
+  p.e.bias = bias;
+  p.e.resid = pos_embed;
+  p.e.ldr = D;
+  p.e.out = x;
+  p.e.ldo = D;
+  p.e.rows_per_group = P;
+  p.e.group_stride = N;
+  p.e.group_offset = prefix;
+  return gemm_bf16_tn(p, stream);
+}
+
+int linear_resid_ln(const void* A, int lda, const void* W, int ldb, int M, int N, int K,
+                    const float* bias, float* x, const float* gamma, const float* beta, float eps,
+                    void* ln_out, float* mean_out, float* rstd_out, cudaStream_t stream) {
+  GemmProblem p;
+  p.A = A;
+  p.lda = lda;
+  p.B = W;
+  p.ldb = ldb;
+  p.M = M;
+  p.N = N;
+  p.K = K;
+  p.epi = EPI_RESID_F32;
+  p.e.bias = bias;
+  p.e.resid = x;
+  p.e.ldr = N;
+  p.e.out = x;
+  p.e.ldo = N;
+  VITK_TRY(gemm_bf16_tn(p, stream));
+  return layernorm_fwd(x, N, gamma, beta, ln_out, 0, N, mean_out, rstd_out, M, N, eps, stream);
+}
+
+int linear_resid_stats(const void* A, int lda, const void* W, int ldb, int M, int N, int K,
+                       const float* bias, float* x, void* xb, float2* stats, cudaStream_t stream) {
+  GemmProblem p;
+  p.A = A;
+  p.lda = lda;
+  p.B = W;
+  p.ldb = ldb;
+  p.M = M;
+  p.N = N;
+  p.K = K;
+  p.epi = EPI_RESID_STATS_F32;
+  p.e.bias = bias;
+  p.e.resid = x;
+  p.e.ldr = N;
+  p.e.out = x;
+  p.e.out2 = xb;
+  p.e.ldo = N;
+  p.e.ln_part_out = stats;
+  return gemm_bf16_tn(p, stream);
+}
+
+int linear_ln(const void* xb, int lda, const void* w_ln, int ldb, int M, int N, int K, GemmEpi epi,
+              const float* b_ln, const float2* stats, int nparts, float eps, void* out, int ldo,
+              cudaStream_t stream) {
+  GemmProblem p;
+  p.A = xb;
+  p.lda = lda;
+  p.B = w_ln;
+  p.ldb = ldb;
+  p.M = M;
+  p.N = N;
+  p.K = K;
+  p.epi = epi;
+  p.e.bias = b_ln;
+  p.e.out = out;
+  p.e.ldo = ldo;
+  p.e.ln_part = stats;
+  p.e.ln_nparts = nparts;
+  p.e.ln_dim = K;
+  p.e.ln_eps = eps;
+  return gemm_bf16_tn(p, stream);
 }
 
 }  // namespace vitk

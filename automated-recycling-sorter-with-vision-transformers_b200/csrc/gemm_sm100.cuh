@@ -88,4 +88,45 @@ void gemm_force_direct_epilogue(int on);
 int gemm_debug_trace(long long* out, int n);
 // Column groups per row of EPI_RESID_STATS_F32's partial sums for an N-column output.
 int gemm_stats_parts(int N);
+
+// ---- The GEMM calls of the encoder, training and detection-head drivers (gemm_sm100.cu).  W is
+// bf16 [N, K] with K contiguous; leading dimensions are in elements.
+
+// out = epilogue(A W^T + bias): EPI_RESID_F32 adds resid (rows of ldr elements; out == resid
+// updates in place), the GELU epilogues keep the pre-activation in out2.
+int linear_fwd(const void* A, int lda, const void* W, int M, int N, int K, GemmEpi epi,
+               const float* bias, const float* resid, int ldr, void* out, void* out2, int ldo,
+               cudaStream_t stream, const DropParams& drop = DropParams());
+// dX[M, in_f] = dY[M, out_f] W[out_f, in_f] with Wt = W^T [in_f, out_f] as the K-major operand:
+// a bf16 epilogue (aux: EPI_DGELU_BF16's pre-activation), or EPI_F32 with dX = acc + beta * dX.
+int linear_dgrad(const void* dY, int out_f, const void* Wt, int M, int in_f, GemmEpi epi,
+                 const void* aux, void* dX, float beta, cudaStream_t stream,
+                 const DropParams& drop = DropParams());
+// dW[out_f, in_f] += dY[rows, out_f]^T X[rows, in_f], split over the rows so that every CTA pair
+// gets about two work items; db[out_f] += column sums of dY unless db is null.
+int linear_wgrad(const void* dY, int out_f, const void* X, int in_f, int rows, float* dW,
+                 float* db, cudaStream_t stream);
+// out[M, N] = alpha * A^T B + beta * out with A [K, lda] (M contiguous) and B [K, ldb] (N
+// contiguous): the MN-major form linear_wgrad runs, with the caller's split_k.
+int gemm_wgrad(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* out,
+               int ldo, float alpha, float beta, int split_k, cudaStream_t stream);
+// Patch embedding: x[token row] = patches W^T + bias + pos_embed[token], patches [B * P, K], for
+// the P patch rows of every image; they land after the `prefix` learned tokens of its N-row block
+// of the residual stream x [B * N, D].
+int patch_embed(const void* patches, const void* W, int B, int P, int K, int D, int N, int prefix,
+                const float* bias, const float* pos_embed, float* x, cudaStream_t stream);
+// x[M, N] += A W^T + bias in place, then ln_out bf16 = LN(x) * gamma + beta with optional mean /
+// rstd: the residual GEMM and a layernorm_fwd launch.
+int linear_resid_ln(const void* A, int lda, const void* W, int ldb, int M, int N, int K,
+                    const float* bias, float* x, const float* gamma, const float* beta, float eps,
+                    void* ln_out, float* mean_out, float* rstd_out, cudaStream_t stream);
+// x[M, N] += A W^T + bias in place; xb = bf16(x); partial row statistics of the updated x
+// (EPI_RESID_STATS_F32).
+int linear_resid_stats(const void* A, int lda, const void* W, int ldb, int M, int N, int K,
+                       const float* bias, float* x, void* xb, float2* stats, cudaStream_t stream);
+// out = epilogue(Linear(LayerNorm(x))) from xb = bf16(x) [M, K], the folded weights w_ln / b_ln
+// and nparts partial row statistics (the consumer side of GemmEpilogue::ln_part).
+int linear_ln(const void* xb, int lda, const void* w_ln, int ldb, int M, int N, int K, GemmEpi epi,
+              const float* b_ln, const float2* stats, int nparts, float eps, void* out, int ldo,
+              cudaStream_t stream);
 }  // namespace vitk
