@@ -193,11 +193,21 @@ __device__ __forceinline__ float gelu_erf_grad(float x) {
   return cdf + x * pdf;
 }
 
+__device__ __forceinline__ bool aligned16(const void* p) {
+  return (reinterpret_cast<uintptr_t>(p) & 15u) == 0;
+}
+
 // Processes one 32-column chunk of one accumulator row held in v[] (raw fp32 bits).
 template <int EPI>
 __device__ __forceinline__ void epilogue_chunk(const uint32_t (&v)[32], int m, int n0, int N,
                                                const GemmEpilogue& e) {
-  const bool full = (n0 + 32 <= N);
+  // The 16-byte accesses below need 16-byte aligned rows.  ldo is a multiple of 8 elements and n0
+  // of 32, so that comes down to the base pointers: this path is also the fallback for an output
+  // (and out2 / aux, which share its pitch) at a 2- or 4-byte aligned column offset.
+  bool vec_ok = aligned16(e.out);
+  if constexpr (is_gelu_epi<EPI>()) vec_ok = vec_ok && aligned16(e.out2);
+  if constexpr (EPI == EPI_DGELU_BF16) vec_ok = vec_ok && aligned16(e.aux);
+  const bool full = (n0 + 32 <= N) && vec_ok;
   float x[32];
   // ---- alpha * accumulator (+ bias); alpha is only honoured by EPI_F32
   float acc_scale = 1.f;
@@ -427,6 +437,8 @@ __device__ __forceinline__ void resid_chunk_staged(const uint32_t (&v)[32], int 
   __syncwarp();
   const int piece = lane & 7;
   const bool col_ok = n0 + 4 * piece < N;   // N is a multiple of 8
+  // ldo and ldr are multiples of 4: 16-byte accesses unless a base pointer sits at a column offset
+  const bool vec_ok = aligned16(e.out) && aligned16(e.resid);
 #pragma unroll
   for (int it = 0; it < 8; ++it) {
     const int r = it * 4 + (lane >> 3);
@@ -445,11 +457,18 @@ __device__ __forceinline__ void resid_chunk_staged(const uint32_t (&v)[32], int 
                    : "r"(slab + static_cast<uint32_t>(r) * 128u +
                          (static_cast<uint32_t>(piece ^ (r & 7)) << 4))
                    : "memory");
-      const float4 rs = *reinterpret_cast<const float4*>(
-          e.resid + static_cast<size_t>(res_row) * e.ldr + n0 + 4 * piece);
-      *reinterpret_cast<float4*>(reinterpret_cast<float*>(e.out) +
-                                 static_cast<size_t>(out_row) * e.ldo + n0 + 4 * piece) =
-          make_float4(a0 + rs.x, a1 + rs.y, a2 + rs.z, a3 + rs.w);
+      const float* rs = e.resid + static_cast<size_t>(res_row) * e.ldr + n0 + 4 * piece;
+      float* o = reinterpret_cast<float*>(e.out) + static_cast<size_t>(out_row) * e.ldo + n0 +
+                 4 * piece;
+      if (vec_ok) {
+        const float4 r4 = *reinterpret_cast<const float4*>(rs);
+        *reinterpret_cast<float4*>(o) = make_float4(a0 + r4.x, a1 + r4.y, a2 + r4.z, a3 + r4.w);
+      } else {
+        o[0] = a0 + rs[0];
+        o[1] = a1 + rs[1];
+        o[2] = a2 + rs[2];
+        o[3] = a3 + rs[3];
+      }
     }
   }
   __syncwarp();   // the slab is rewritten by the next chunk

@@ -9,12 +9,21 @@ namespace vitk {
 
 // Epilogue selector (compile-time variants of one kernel).
 enum GemmEpi : int {
+  // Per-element bounds of the approximations against the exact erf forms, x = acc + bias (enforced
+  // by tests/test_gemm_epilogues_gpu.py):
   EPI_BF16 = 0,        // out_bf16 = acc + bias
-  EPI_GELU_BF16 = 1,   // out_bf16 = gelu_erf(acc + bias); optional out2_bf16 = acc + bias
+  // out_bf16 = x Phi(x) with an erf-fitted logistic Phi (gelu_fast): |error| <= 9e-5;
+  // optional out2_bf16 = x
+  EPI_GELU_BF16 = 1,
   EPI_RESID_F32 = 2,   // out_f32 = acc + bias + resid_f32   (optional row remap: patch embed)
   EPI_F32 = 3,         // out_f32 = alpha * acc + bias (+ beta * out_f32)
-  EPI_DGELU_BF16 = 4,  // out_bf16 = (acc + bias) * gelu'(aux_bf16)            (fc2 dgrad)
-  EPI_GELU_TANH_BF16 = 6,  // as EPI_GELU_BF16 with the tanh.approx form of the normal CDF (A/B)
+  // out_bf16 = g * gelu'(aux_bf16), g = acc + bias (fc2 dgrad): the exact erf derivative on the
+  // direct path (|error| <= 1e-5 |g|), dgelu_tanh_pair on the TMA path (|error| <= |g| (1.3e-4 +
+  // 2^-11 (0.5 + 2 |x|)))
+  EPI_DGELU_BF16 = 4,
+  // the fc1 epilogue of the encoder forward and training: as EPI_GELU_BF16 with the tanh.approx
+  // form of the normal CDF, |error| <= 3.3e-5 + 2.5e-4 |x|
+  EPI_GELU_TANH_BF16 = 6,
   EPI_RELU_BF16 = 7,   // out_bf16 = max(acc + bias, 0)   (decoder feed-forward, evaluation.py:170-176)
   // x = x + acc + bias in place (out == resid; the tile of x is TMA-loaded into the staging slab,
   // updated there and TMA-stored back), out2_bf16 = bf16(x) and per-row partial sums (sum x,
