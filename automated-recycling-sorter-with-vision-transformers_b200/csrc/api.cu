@@ -6,6 +6,7 @@
 
 #include <cstdlib>
 
+#include "attention.cuh"
 #include "common.h"
 #include "encoder.cuh"
 #include "fp32_mode.cuh"
@@ -72,12 +73,8 @@ int cls_tail(const VitkConfig* cfg, const VitkWeights* w, const Dims& d, const W
   const VitkBlockWeights& bw = w->blocks[d.L - 1];
   const __nv_bfloat16* qkv = static_cast<const __nv_bfloat16*>(ws.qkv);
   const long long img = static_cast<long long>(d.N) * 3 * D;
-  if (attention_xtc_applicable(img, img, d.B, 1, d.N, d.hd))
-    VITK_TRY(attention_xtc(qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D, ws.c_b, D, D, d.B, 1,
-                           d.N, d.H, d.hd, stream));
-  else
-    VITK_TRY(attention_x(qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D, ws.c_b, D, D, d.B, 1,
-                         d.N, d.H, d.hd, stream));
+  const AttnXSrc src{qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D};
+  VITK_TRY(attention_src_fwd(src, ws.c_b, D, D, nullptr, d.B, 1, d.N, d.H, d.hd, stream));
   VITK_TRY(linear_fwd(ws.c_b, D, bw.proj_w, d.B, D, D, EPI_RESID_F32, bw.proj_b, ws.x, d.N * D,
                       ws.c_x, nullptr, D, stream));
   VITK_TRY(layernorm_fwd(ws.c_x, D, bw.ln2_w, bw.ln2_b, ws.c_b, 0, D, nullptr, nullptr, d.B, D,

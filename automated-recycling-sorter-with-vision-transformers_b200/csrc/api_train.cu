@@ -4,6 +4,7 @@
 //     outputs = model(images) ; loss.backward() ; optimizer.step()
 #include "../../include/vitk.h"
 
+#include "attention.cuh"
 #include "common.h"
 #include "encoder.cuh"
 #include "gemm_sm100.cuh"
@@ -18,10 +19,7 @@ int check_train_config(const VitkConfig* cfg, int batch, Dims* d) {
   VITK_TRY(check_config(cfg, batch, d));
   VITK_REQUIRE(cfg->precision == 0, "training runs in the bf16 mode only");
   VITK_REQUIRE(cfg->dropout_p >= 0.f && cfg->dropout_p < 1.f, "dropout_p must be in [0, 1)");
-  // head_dim 64 up to 256 tokens: tcgen05 attention kernels; every other shape (train.py's own
-  // Config has head_dim 16; a 384 px fine-tune 577 tokens): the CUDA-core kernels of
-  // attention_gen.cu, as far as one head's operands fit in shared memory
-  VITK_REQUIRE((d->hd == 64 && d->N <= 256) || attention_gen_fits(d->N, d->hd),
+  VITK_REQUIRE(attention_trainable(d->N, d->hd),
                "training: head_dim %d with %d tokens is not covered (head_dim 8..128 in steps of 8, "
                "and tokens * head_dim within shared memory)", d->hd, d->N);
   VITK_REQUIRE(cfg->dropout_p == 0.f || d->M * d->Mlp < (1ll << 32),

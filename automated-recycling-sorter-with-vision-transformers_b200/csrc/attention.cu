@@ -1,315 +1,145 @@
-// Fused attention core: ctx = softmax(q k^T / sqrt(hd)) v per (image, head) without materialising
-// the [B,H,N,N] score tensor (reference train.py:543-549 materialises it; evaluation.py:66-72).
+// Kernel selection for every attention entry point (attention.cuh).  The rule lives here and
+// nowhere else; the kernels and their launchers are in the other attention_*.cu files.
 //
-// Flash-style: one CTA per (image, head). K and V of that head (N <= ~800 keys, hd = 64) are
-// staged once in shared memory (cp.async, XOR-swizzled 128-byte rows); each warp owns 16-query
-// tiles and sweeps the keys in blocks of 64 with a warp-level online softmax (running max / sum in
-// registers, quad shuffles), bf16 tensor-core MMAs (m16n8k16, fp32 accumulate) for q k^T and p v.
-// Reads the packed qkv activation in place (no permute copies) and writes ctx already in
-// [B, N, H*hd] order (the reference's transpose(1,2).reshape is free).
-#include <cuda_bf16.h>
-
-#include <mutex>
-
+// "dropping": drop != nullptr && drop->thresh != 0.  "impl": vitk_attention_set_impl.
+//
+// packed fwd   hd != 64, with lse or dropping or hd not in {32, 96, 128}:
+//                impl != 1 and xmma fits -> attn_xmma_fwd_kernel, else attn_gen_fwd_kernel
+//              hd in {32, 96, 128}, no lse, not dropping -> attn_x_kernel
+//              hd 64, dropping: N <= 208 on sm_100 -> attn_fwd_tc2_kernel<true>, else attn_gen_fwd
+//              hd 64, impl 0: on sm_100 with N <= 640, tc2 up to 208 tokens, attn_fwd_tc_kernel up
+//                to 256, attn_fwd_tc3_kernel above; otherwise attn_fwd_hd64_kernel
+//              hd 64, impl 1: hd64.  2: tc2 / tc / tc3 by N as for impl 0, without the device
+//                check.  3: tc up to 256 tokens, tc3 above.  4: tc3
+// packed bwd   hd 64, N <= 256, sm_100, and impl != 1 or dropping: attn_bwd_tc2_kernel where its
+//                shared memory fits, else attn_bwd_tc_kernel
+//              else hd != 64 or N > 256 or dropping: impl != 1 and xmma fits ->
+//                attn_xmma_bwd_kernel + colsum_bf16 (dbias), else attn_gen_bwd_kernel
+//              else attn_bwd_hd64_kernel + colsum_bf16 (dbias)
+// src fwd      no lse: impl != 1 and xtc applies -> attn_xtc_kernel, else attn_x_kernel
+//              lse: impl != 1, not dropping and xtc applies -> xtc; else impl != 1 and xmma fits
+//                -> attn_xmma_fwd_kernel; else attn_xgen_fwd_kernel
+// src bwd      impl != 1 and xmma fits -> attn_xmma_bwd_kernel, else attn_xgen_bwd_kernel
+#include "attention_kernels.cuh"
 #include "common.h"
-#include "ptx.cuh"
-#include "rowops.cuh"
+#include "train_ops.cuh"
 
 namespace vitk {
-using namespace ptx;
 
 namespace {
 
-constexpr int kAttnWarps = 7;
-constexpr int kAttnThreads = kAttnWarps * 32;
+// Values of vitk_attention_set_impl (tests and A/B timing).
+enum AttnImpl : int {
+  kImplAuto = 0,
+  kImplNoTcgen05 = 1,      // the mma.sync / CUDA-core kernels wherever a choice exists
+  kImplTcgen05 = 2,        // head_dim 64 forward: the tcgen05 kernels, chosen by N
+  kImplTcUnpipelined = 3,  // ... without the item-pipelined one (attention_tc2.cu)
+  kImplTcKeyBlock = 4,     // ... the key-block one (attention_tc3.cu) for every N
+};
+AttnImpl g_attn_impl = kImplAuto;
 
-__device__ __forceinline__ void mma_m16n8k16(float (&c)[4], const uint32_t (&a)[4], uint32_t b0,
-                                             uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
-      "{%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void ldmatrix_x4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2,
-                                            uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void ldmatrix_x4_trans(uint32_t addr, uint32_t& r0, uint32_t& r1,
-                                                  uint32_t& r2, uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void cp_async_16(uint32_t dst, const void* src, bool valid) {
-  const int sz = valid ? 16 : 0;  // src-size 0 -> zero fill
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(sz)
-               : "memory");
-}
-__device__ __forceinline__ float quad_max(float v) {
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1));
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
-  return v;
-}
-__device__ __forceinline__ float quad_sum(float v) {
-  v += __shfl_xor_sync(0xffffffffu, v, 1);
-  v += __shfl_xor_sync(0xffffffffu, v, 2);
-  return v;
-}
-
-// hd == 64 only: one K/V row is exactly one 128-byte swizzle row.
-__global__ void __launch_bounds__(kAttnThreads, 2)
-attn_fwd_hd64_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ ctx,
-                     float* __restrict__ lse, int N, int H, float scale) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  constexpr int HD = 64;
-  const int Nkv = (N + 15) & ~15;
-  const uint32_t sK = smem_u32(smem);
-  const uint32_t sV = sK + Nkv * 128;
-  const uint32_t sO = sV + Nkv * 128;  // kAttnWarps * 2048 bytes of output staging
-
-  const int b = blockIdx.x / H;
-  const int h = blockIdx.x - b * H;
-  const int D = H * HD;
-  const int D3 = 3 * D;
-  const __nv_bfloat16* base = qkv + static_cast<size_t>(b) * N * D3 + h * HD;
-
-  const int tid = threadIdx.x;
-  const int warp = tid >> 5;
-  const int lane = tid & 31;
-  const int g = lane >> 2;  // fragment row
-  const int t = lane & 3;   // fragment column pair
-
-  // ---- stage K and V (all keys of this head) into swizzled shared memory
-  for (int idx = tid; idx < Nkv * 8; idx += kAttnThreads) {
-    const int row = idx >> 3;
-    const int ch = idx & 7;
-    const bool valid = row < N;
-    const __nv_bfloat16* src = base + static_cast<size_t>(valid ? row : 0) * D3 + ch * 8;
-    const uint32_t off = row * 128 + ((ch ^ (row & 7)) << 4);
-    cp_async_16(sK + off, src + D, valid);
-    cp_async_16(sV + off, src + 2 * D, valid);
-  }
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
-  __syncthreads();
-
-  const float c = scale * 1.44269504088896340736f;  // softmax in base 2
-  const uint32_t sOw = sO + warp * 2048;
-
-  for (int qt = warp; qt * 16 < N; qt += kAttnWarps) {
-    const int q0 = qt * 16;
-    const int r0 = q0 + g, r1 = r0 + 8;
-    // ---- Q fragments straight from global (each 128-byte query row is consumed whole)
-    uint32_t qa[4][4];
-    {
-      const uint32_t* p0 = reinterpret_cast<const uint32_t*>(base + static_cast<size_t>(r0) * D3);
-      const uint32_t* p1 = reinterpret_cast<const uint32_t*>(base + static_cast<size_t>(r1) * D3);
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) {
-        const int w = kk * 8 + t;  // 32-bit word index of d = kk*16 + 2t
-        qa[kk][0] = (r0 < N) ? __ldg(p0 + w) : 0u;
-        qa[kk][1] = (r1 < N) ? __ldg(p1 + w) : 0u;
-        qa[kk][2] = (r0 < N) ? __ldg(p0 + w + 4) : 0u;
-        qa[kk][3] = (r1 < N) ? __ldg(p1 + w + 4) : 0u;
-      }
-    }
-    float o[8][4];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) o[j][0] = o[j][1] = o[j][2] = o[j][3] = 0.f;
-    float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-
-    for (int kb = 0; kb * 64 < N; ++kb) {
-      const int rem = N - kb * 64;  // valid keys from the start of this block
-      float s[8][4];
-      // ---- S = Q K^T for 64 keys
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        if (j * 8 < rem) {
-          s[j][0] = s[j][1] = s[j][2] = s[j][3] = 0.f;
-          const int key = kb * 64 + j * 8 + (lane & 7);
-#pragma unroll
-          for (int half = 0; half < 2; ++half) {
-            const int ch = (lane >> 3) + 4 * half;
-            uint32_t k0, k1, k2, k3;
-            ldmatrix_x4(sK + key * 128 + ((ch ^ (key & 7)) << 4), k0, k1, k2, k3);
-            mma_m16n8k16(s[j], qa[2 * half], k0, k1);
-            mma_m16n8k16(s[j], qa[2 * half + 1], k2, k3);
-          }
-        } else {
-          s[j][0] = s[j][1] = s[j][2] = s[j][3] = -INFINITY;
-        }
-      }
-      if (rem < 64) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int k0 = j * 8 + t * 2;
-          if (k0 >= rem) s[j][0] = s[j][2] = -INFINITY;
-          if (k0 + 1 >= rem) s[j][1] = s[j][3] = -INFINITY;
-        }
-      }
-      // ---- online softmax update
-      float mx0 = -INFINITY, mx1 = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        mx0 = fmaxf(mx0, fmaxf(s[j][0], s[j][1]));
-        mx1 = fmaxf(mx1, fmaxf(s[j][2], s[j][3]));
-      }
-      mx0 = quad_max(mx0);
-      mx1 = quad_max(mx1);
-      const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);
-      const float a0 = exp2f((m0 - mn0) * c), a1 = exp2f((m1 - mn1) * c);
-      m0 = mn0;
-      m1 = mn1;
-      const float mc0 = mn0 * c, mc1 = mn1 * c;
-      float ps0 = 0.f, ps1 = 0.f;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        s[j][0] = exp2f(fmaf(s[j][0], c, -mc0));
-        s[j][1] = exp2f(fmaf(s[j][1], c, -mc0));
-        s[j][2] = exp2f(fmaf(s[j][2], c, -mc1));
-        s[j][3] = exp2f(fmaf(s[j][3], c, -mc1));
-        ps0 += s[j][0] + s[j][1];
-        ps1 += s[j][2] + s[j][3];
-      }
-      l0 = l0 * a0 + ps0;
-      l1 = l1 * a1 + ps1;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        o[j][0] *= a0;
-        o[j][1] *= a0;
-        o[j][2] *= a1;
-        o[j][3] *= a1;
-      }
-      // ---- O += P V
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) {
-        if (kk * 16 < rem) {
-          uint32_t pa[4];
-          pa[0] = pack_bf16x2(s[2 * kk][0], s[2 * kk][1]);
-          pa[1] = pack_bf16x2(s[2 * kk][2], s[2 * kk][3]);
-          pa[2] = pack_bf16x2(s[2 * kk + 1][0], s[2 * kk + 1][1]);
-          pa[3] = pack_bf16x2(s[2 * kk + 1][2], s[2 * kk + 1][3]);
-          const int mi = lane >> 3;
-          const int key = kb * 64 + kk * 16 + (mi & 1) * 8 + (lane & 7);
-#pragma unroll
-          for (int jj = 0; jj < 4; ++jj) {
-            const int ch = 2 * jj + (mi >> 1);
-            uint32_t v0, v1, v2, v3;
-            ldmatrix_x4_trans(sV + key * 128 + ((ch ^ (key & 7)) << 4), v0, v1, v2, v3);
-            mma_m16n8k16(o[2 * jj], pa, v0, v1);
-            mma_m16n8k16(o[2 * jj + 1], pa, v2, v3);
-          }
-        }
-      }
-    }
-
-    // ---- finalise: divide by the row sum, stage through smem, 16-byte coalesced stores
-    l0 = quad_sum(l0);
-    l1 = quad_sum(l1);
-    const float inv0 = 1.f / l0, inv1 = 1.f / l1;
-    __syncwarp();
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const uint32_t w0 = pack_bf16x2(o[j][0] * inv0, o[j][1] * inv0);
-      const uint32_t w1 = pack_bf16x2(o[j][2] * inv1, o[j][3] * inv1);
-      const uint32_t a_lo = sOw + g * 128 + ((j ^ (g & 7)) << 4) + t * 4;
-      const uint32_t a_hi = sOw + (g + 8) * 128 + ((j ^ ((g + 8) & 7)) << 4) + t * 4;
-      asm volatile("st.shared.b32 [%0], %1;" ::"r"(a_lo), "r"(w0) : "memory");
-      asm volatile("st.shared.b32 [%0], %1;" ::"r"(a_hi), "r"(w1) : "memory");
-    }
-    __syncwarp();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int idx = lane + 32 * i;
-      const int row = idx >> 3, ch = idx & 7;
-      if (q0 + row < N) {
-        uint4 val;
-        const uint32_t a = sOw + row * 128 + ((ch ^ (row & 7)) << 4);
-        asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];"
-                     : "=r"(val.x), "=r"(val.y), "=r"(val.z), "=r"(val.w)
-                     : "r"(a)
-                     : "memory");
-        *reinterpret_cast<uint4*>(ctx + (static_cast<size_t>(b) * N + q0 + row) * D + h * HD +
-                                  ch * 8) = val;
-      }
-    }
-    if (lse != nullptr && t == 0) {
-      float* lrow = lse + (static_cast<size_t>(b) * H + h) * N;
-      if (r0 < N) lrow[r0] = m0 * scale + logf(l0);
-      if (r1 < N) lrow[r1] = m1 * scale + logf(l1);
-    }
-  }
-}
+bool dropping(const DropParams* drop) { return drop != nullptr && drop->thresh != 0u; }
 
 }  // namespace
 
-// 0 auto, 1 = mma.sync flash kernel, 2 = tcgen05 kernels, 3 = the unpipelined tcgen05 forward
-// (attention_tc.cu) also where the pipelined one (attention_tc2.cu) applies, 4 = the key-block
-// long-sequence kernel (attention_tc3.cu) for every N <= 640
-static int g_attn_impl = 0;
-void attention_force_impl(int impl) { g_attn_impl = impl; }
-int attention_impl() { return g_attn_impl; }
+void attention_force_impl(int impl) { g_attn_impl = static_cast<AttnImpl>(impl); }
+
+// head_dim 64 up to 256 tokens: the tcgen05 backward kernels; every other shape (train.py's own
+// Config has head_dim 16; a 384 px fine-tune 577 tokens): the CUDA-core kernels, as far as one
+// head's operands fit in shared memory.
+bool attention_trainable(int N, int hd) {
+  return (hd == 64 && N <= 256) || attention_gen_fits(N, hd);
+}
 
 int attention_fwd(const void* qkv, void* ctx, float* lse, int B, int N, int H, int hd,
                   cudaStream_t stream, const DropParams* drop) {
   VITK_REQUIRE(qkv && ctx, "attention: null operand");
-  const bool dropping = drop != nullptr && drop->thresh != 0u;
   if (hd != 64) {
-    // training (log-sum-exp / dropout) and head sizes the mma.sync kernel has no form for (e.g.
-    // the 16 of train.py's Config): the CUDA-core kernel; inference at 32 / 96 / 128: the
-    // generic-source mma.sync kernel on the packed activation
     const __nv_bfloat16* p = static_cast<const __nv_bfloat16*>(qkv);
     const int D = H * hd;
     const long long img = static_cast<long long>(N) * 3 * D;
-    if (lse != nullptr || dropping || !(hd == 32 || hd == 96 || hd == 128)) {
-      // tensor cores (mma.sync, whole head in shared memory) when the shape allows, else CUDA cores
-      if (g_attn_impl != 1 && attention_xmma_bwd_applicable(N, N, hd)) {
-        const AttnXSrc src{p, img, 3 * D, p + D, p + 2 * D, img, 3 * D};
-        return attention_xmma_fwd(src, ctx, static_cast<long long>(N) * D, D, lse, B, N, N, H, hd,
-                                  stream, drop);
-      }
-      return attention_gen_fwd(qkv, ctx, lse, B, N, H, hd, stream, drop);
+    if (lse == nullptr && !dropping(drop) && (hd == 32 || hd == 96 || hd == 128))
+      return attention_x(p, img, 3 * D, p + D, p + 2 * D, img, 3 * D, ctx,
+                         static_cast<long long>(N) * D, D, B, N, N, H, hd, stream);
+    if (g_attn_impl != kImplNoTcgen05 && attention_xmma_fits(N, N, hd)) {
+      const AttnXSrc src{p, img, 3 * D, p + D, p + 2 * D, img, 3 * D};
+      return attention_xmma_fwd(src, ctx, static_cast<long long>(N) * D, D, lse, B, N, N, H, hd,
+                                stream, drop);
     }
-    return attention_x(p, img, 3 * D, p + D, p + 2 * D, img, 3 * D, ctx,
-                       static_cast<long long>(N) * D, D, B, N, N, H, hd, stream);
+    return attention_gen_fwd(qkv, ctx, lse, B, N, H, hd, stream, drop);
   }
-  if (dropping) {
+  if (dropping(drop)) {
     // the pipelined tcgen05 kernel regenerates the masks in its softmax warps up to 208 tokens
     if (N <= 208 && device_cc() >= 100)
       return attention_fwd_tc2(qkv, ctx, lse, B, N, H, hd, stream, drop);
     return attention_gen_fwd(qkv, ctx, lse, B, N, H, hd, stream, drop);
   }
-  if (g_attn_impl == 2 || g_attn_impl == 3 ||
-      (g_attn_impl == 0 && hd == 64 && N <= 640 && device_cc() >= 100)) {
-    if (g_attn_impl != 3 && hd == 64 && N <= 208)
-      return attention_fwd_tc2(qkv, ctx, lse, B, N, H, hd, stream);
-    if (N > 256 || g_attn_impl == 4) return attention_fwd_tc3(qkv, ctx, lse, B, N, H, hd, stream);
-    return attention_fwd_tc(qkv, ctx, lse, B, N, H, hd, stream);
+  const AttnImpl impl = g_attn_impl;
+  if (impl == kImplNoTcgen05 || (impl == kImplAuto && (N > 640 || device_cc() < 100)))
+    return attention_fwd_hd64(qkv, ctx, lse, B, N, H, hd, stream);
+  if (impl == kImplTcKeyBlock) return attention_fwd_tc3(qkv, ctx, lse, B, N, H, hd, stream);
+  if (impl != kImplTcUnpipelined && N <= 208)
+    return attention_fwd_tc2(qkv, ctx, lse, B, N, H, hd, stream);
+  if (N <= 256) return attention_fwd_tc(qkv, ctx, lse, B, N, H, hd, stream);
+  return attention_fwd_tc3(qkv, ctx, lse, B, N, H, hd, stream);
+}
+
+int attention_bwd(const void* qkv, const void* ctx, const void* dctx, const float* lse, void* dqkv,
+                  int B, int N, int H, int hd, cudaStream_t stream, const DropParams* drop,
+                  float* dbias) {
+  VITK_REQUIRE(qkv && ctx && dctx && lse && dqkv, "attention_bwd: null operand");
+  const bool tcgen05 = g_attn_impl != kImplNoTcgen05;
+  if ((tcgen05 || dropping(drop)) && hd == 64 && N <= 256 && device_cc() >= 100) {
+    if (attention_bwd_tc2_fits(N, H, dbias != nullptr))
+      return attention_bwd_tc2(qkv, ctx, dctx, lse, dqkv, B, N, H, hd, stream, drop, dbias);
+    return attention_bwd_tc(qkv, ctx, dctx, lse, dqkv, B, N, H, hd, stream, drop, dbias);
   }
-  if (g_attn_impl == 4) return attention_fwd_tc3(qkv, ctx, lse, B, N, H, hd, stream);
-  VITK_REQUIRE(B > 0 && N > 0 && H > 0, "attention: bad shape B=%d N=%d H=%d", B, N, H);
-  VITK_REQUIRE(hd == 64, "attention: head_dim %d unsupported by the bf16 kernel (needs 64)", hd);
-  const int Nkv = (N + 15) & ~15;
-  const size_t smem = static_cast<size_t>(Nkv) * 256 + kAttnWarps * 2048;
-  VITK_REQUIRE(smem <= 232448, "attention: N=%d keys do not fit in shared memory", N);
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_fwd_hd64_kernel,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention) failed: %s",
-                     cudaGetErrorString(attr_err));
-  const float scale = 1.0f / sqrtf(static_cast<float>(hd));
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(N) * N * hd, stream);
-  attn_fwd_hd64_kernel<<<B * H, kAttnThreads, smem, stream>>>(
-      static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(ctx), lse, N, H, scale);
-  VITK_CHECK_LAUNCH("attn_fwd_hd64_kernel");
+  const int D = H * hd;
+  if (hd != 64 || N > 256 || dropping(drop)) {
+    if (!tcgen05 || !attention_xmma_fits(N, N, hd))
+      return attention_gen_bwd(qkv, ctx, dctx, lse, dqkv, B, N, H, hd, stream, drop, dbias);
+    // q, k, v are column blocks of the packed activation
+    const __nv_bfloat16* p = static_cast<const __nv_bfloat16*>(qkv);
+    __nv_bfloat16* dp = static_cast<__nv_bfloat16*>(dqkv);
+    const long long img = static_cast<long long>(N) * 3 * D, cimg = static_cast<long long>(N) * D;
+    const AttnXSrc src{p, img, 3 * D, p + D, p + 2 * D, img, 3 * D};
+    VITK_TRY(attention_xmma_bwd(src, ctx, dctx, cimg, D, lse, dp, img, 3 * D, dp + D, dp + 2 * D,
+                                img, 3 * D, B, N, N, H, hd, stream, drop));
+  } else {
+    VITK_TRY(attention_bwd_hd64(qkv, ctx, dctx, lse, dqkv, B, N, H, hd, stream));
+  }
+  // neither kernel accumulates the bias gradient itself
+  if (dbias != nullptr) return colsum_bf16(dqkv, 3ll * D, B * N, 3 * D, dbias, stream);
   return VITK_OK;
+}
+
+int attention_src_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc, float* lse, int B,
+                      int Nq, int Nk, int H, int hd, cudaStream_t stream, const DropParams* drop) {
+  const bool tcgen05 = g_attn_impl != kImplNoTcgen05;
+  if (lse == nullptr) {
+    if (tcgen05 && attention_xtc_applicable(s.q_img, s.kv_img, B, Nq, Nk, hd))
+      return attention_xtc(s.q, s.q_img, s.ldq, s.k, s.v, s.kv_img, s.ldkv, ctx, ctx_img, ldc, B,
+                           Nq, Nk, H, hd, stream);
+    return attention_x(s.q, s.q_img, s.ldq, s.k, s.v, s.kv_img, s.ldkv, ctx, ctx_img, ldc, B, Nq,
+                       Nk, H, hd, stream);
+  }
+  if (tcgen05 && !dropping(drop) && attention_xtc_applicable(s.q_img, s.kv_img, B, Nq, Nk, hd))
+    return attention_xtc(s.q, s.q_img, s.ldq, s.k, s.v, s.kv_img, s.ldkv, ctx, ctx_img, ldc, B, Nq,
+                         Nk, H, hd, stream, lse);
+  if (tcgen05 && attention_xmma_fits(Nq, Nk, hd))
+    return attention_xmma_fwd(s, ctx, ctx_img, ldc, lse, B, Nq, Nk, H, hd, stream, drop);
+  return attention_xgen_fwd(s, ctx, ctx_img, ldc, lse, B, Nq, Nk, H, hd, stream, drop);
+}
+
+int attention_src_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, long long ctx_img,
+                      int ldc, const float* lse, void* dq, long long dq_img, int lddq, void* dk,
+                      void* dv, long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
+                      cudaStream_t stream, const DropParams* drop) {
+  if (g_attn_impl != kImplNoTcgen05 && attention_xmma_fits(Nq, Nk, hd))
+    return attention_xmma_bwd(s, ctx, dctx, ctx_img, ldc, lse, dq, dq_img, lddq, dk, dv, dkv_img,
+                              lddkv, B, Nq, Nk, H, hd, stream, drop);
+  return attention_xgen_bwd(s, ctx, dctx, ctx_img, ldc, lse, dq, dq_img, lddq, dk, dv, dkv_img,
+                            lddkv, B, Nq, Nk, H, hd, stream, drop);
 }
 
 }  // namespace vitk

@@ -17,12 +17,10 @@
 // (rows >= N zero-filled); d_qkv leaves through TMA stores whose 3-D map clips rows >= N.
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "dropout.cuh"
 #include "ptx.cuh"
-#include "train_ops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -32,18 +30,7 @@ namespace {
 // warp 0 TMA, 1 MMA, 2 TMEM alloc, 2-3 per-row vectors of the next item, 4-11 softmax-backward /
 // epilogue (warps 4-7 own the first half of a block's query chunks, warps 8-11 the second half)
 constexpr int kThreads = 12 * 32;
-constexpr float kLog2e = 1.44269504088896340736f;
 constexpr uint32_t kColS = 0, kColDP = 128, kColDV = 256, kColDK = 320, kColDQ = 384;
-
-struct BwdParams {
-  int B, N, H, Nk;
-  float scale;
-  const __nv_bfloat16* ctx;
-  const __nv_bfloat16* dctx;
-  const float* lse;
-  DropParams drop;  // attention-probability dropout of the forward (same index space / key)
-  float* dbias;     // optional [3 D]: += column sums of d_qkv (the qkv bias gradient)
-};
 
 // DROP: attention-probability dropout compiled in (a separate instantiation, so that the p = 0
 // kernel carries neither the extra registers nor the per-element branch).
@@ -456,24 +443,12 @@ int attention_bwd_tc(const void* qkv, const void* ctx, const void* dctx, const f
   const size_t smem = 4 * static_cast<size_t>(Nk) * 128 + 32768 + 32768 + 4096 + 256 + 1024 +
                       (dbias != nullptr ? static_cast<size_t>(3) * D * 4 : 0);
   VITK_REQUIRE(smem <= 232448, "attention_bwd(tc): shared memory budget exceeded");
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_bwd_tc_kernel<false>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (attr_err == cudaSuccess)
-      attr_err = cudaFuncSetAttribute(attn_bwd_tc_kernel<true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention_bwd tc) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_bwd_tc_kernel<false>>(232448, "attn_bwd_tc_kernel<false>"));
+  VITK_TRY(opt_in_smem<attn_bwd_tc_kernel<true>>(232448, "attn_bwd_tc_kernel<true>"));
   CUtensorMap tq, tdo, tout;
-  const uint64_t qkv_pitch = static_cast<uint64_t>(3) * D * 2;
-  const uint64_t ctx_pitch = static_cast<uint64_t>(D) * 2;
-  VITK_TRY(make_tmap_3d(&tq, qkv, 2, 3 * D, N, B, qkv_pitch, qkv_pitch * N, 64, Nk));
-  VITK_TRY(make_tmap_3d(&tdo, dctx, 2, D, N, B, ctx_pitch, ctx_pitch * N, 64, Nk));
-  VITK_TRY(make_tmap_3d(&tout, dqkv, 2, 3 * D, N, B, qkv_pitch, qkv_pitch * N, 64, 32));
+  VITK_TRY(make_row_map(&tq, qkv, B, N, 3 * D, 3 * D, Nk));
+  VITK_TRY(make_row_map(&tdo, dctx, B, N, D, D, Nk));
+  VITK_TRY(make_row_map(&tout, dqkv, B, N, 3 * D, 3 * D, 32));
   BwdParams prm;
   prm.B = B;
   prm.N = N;
@@ -485,9 +460,8 @@ int attention_bwd_tc(const void* qkv, const void* ctx, const void* dctx, const f
   prm.lse = lse;
   if (drop != nullptr) prm.drop = *drop;
   prm.dbias = dbias;
-  int grid = sm_count();
-  if (B * H < grid) grid = B * H;
-  ProfileScope prof(PROF_ATTN, 10.0 * B * H * static_cast<double>(N) * N * hd, stream);
+  const int grid = persistent_grid(B * H);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, N, N, hd, true), stream);
   if (prm.drop.thresh != 0u)
     attn_bwd_tc_kernel<true><<<grid, kThreads, smem, stream>>>(tq, tdo, tout, prm);
   else

@@ -26,12 +26,10 @@
 // staging - which is what limits this kernel to Nk <= 224; attention_bwd_tc.cu covers 225..256.
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "dropout.cuh"
 #include "ptx.cuh"
-#include "train_ops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -52,18 +50,7 @@ namespace {
 // warp 0 TMA, 1 MMA, 2 TMEM alloc, 2-3 per-row vectors of the next item, 4-11 softmax-backward /
 // epilogue (warps 4-7 own the first half of a block's query chunks, warps 8-11 the second half)
 constexpr int kThreads = 12 * 32;
-constexpr float kLog2e = 1.44269504088896340736f;
 constexpr uint32_t kColDPofs = 64, kColDV = 256, kColDK = 320, kColDQ = 384;  // S at buffer * 128
-
-struct BwdParams {
-  int B, N, H, Nk;
-  float scale;
-  const __nv_bfloat16* ctx;
-  const __nv_bfloat16* dctx;
-  const float* lse;
-  DropParams drop;  // attention-probability dropout of the forward (same index space / key)
-  float* dbias;     // optional [3 D]: += column sums of d_qkv (the qkv bias gradient)
-};
 
 // Per-row vectors of one (image, head): vLse[r] = lse_r * log2(e) (+inf for rows >= N, so that
 // P = 2^(-inf) = 0) and vD[r] = -scale * rowsum(d_ctx_r * ctx_r), r < 256.  Called by a group of nw
@@ -675,27 +662,15 @@ int attention_bwd_tc2(const void* qkv, const void* ctx, const void* dctx, const 
   const int Nk = (N + 15) & ~15;
   const int D = H * 64;
   const size_t smem = tc2_smem_bytes(N, H, dbias != nullptr);
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_bwd_tc2_kernel<false>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (attr_err == cudaSuccess)
-      attr_err = cudaFuncSetAttribute(attn_bwd_tc2_kernel<true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention_bwd tc2) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_bwd_tc2_kernel<false>>(232448, "attn_bwd_tc2_kernel<false>"));
+  VITK_TRY(opt_in_smem<attn_bwd_tc2_kernel<true>>(232448, "attn_bwd_tc2_kernel<true>"));
   CUtensorMap tq, tdo, tq1, tdo1, tout;
-  const uint64_t qkv_pitch = static_cast<uint64_t>(3) * D * 2;
-  const uint64_t ctx_pitch = static_cast<uint64_t>(D) * 2;
   const int rows0 = Nk < 128 ? Nk : 128, rows1 = Nk > 128 ? Nk - 128 : rows0;
-  VITK_TRY(make_tmap_3d(&tq, qkv, 2, 3 * D, N, B, qkv_pitch, qkv_pitch * N, 64, rows0));
-  VITK_TRY(make_tmap_3d(&tdo, dctx, 2, D, N, B, ctx_pitch, ctx_pitch * N, 64, rows0));
-  VITK_TRY(make_tmap_3d(&tq1, qkv, 2, 3 * D, N, B, qkv_pitch, qkv_pitch * N, 64, rows1));
-  VITK_TRY(make_tmap_3d(&tdo1, dctx, 2, D, N, B, ctx_pitch, ctx_pitch * N, 64, rows1));
-  VITK_TRY(make_tmap_3d(&tout, dqkv, 2, 3 * D, N, B, qkv_pitch, qkv_pitch * N, 64, 32));
+  VITK_TRY(make_row_map(&tq, qkv, B, N, 3 * D, 3 * D, rows0));
+  VITK_TRY(make_row_map(&tdo, dctx, B, N, D, D, rows0));
+  VITK_TRY(make_row_map(&tq1, qkv, B, N, 3 * D, 3 * D, rows1));
+  VITK_TRY(make_row_map(&tdo1, dctx, B, N, D, D, rows1));
+  VITK_TRY(make_row_map(&tout, dqkv, B, N, 3 * D, 3 * D, 32));
   BwdParams prm;
   prm.B = B;
   prm.N = N;
@@ -707,9 +682,8 @@ int attention_bwd_tc2(const void* qkv, const void* ctx, const void* dctx, const 
   prm.lse = lse;
   if (drop != nullptr) prm.drop = *drop;
   prm.dbias = dbias;
-  int grid = sm_count();
-  if (B * H < grid) grid = B * H;
-  ProfileScope prof(PROF_ATTN, 10.0 * B * H * static_cast<double>(N) * N * hd, stream);
+  const int grid = persistent_grid(B * H);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, N, N, hd, true), stream);
   if (prm.drop.thresh != 0u)
     attn_bwd_tc2_kernel<true><<<grid, kThreads, smem, stream>>>(tq, tdo, tq1, tdo1, tout, prm);
   else

@@ -16,13 +16,11 @@
 //   backward pass 2: per key row    P / dS column, dK, dV row (Q, dO resident in shared memory)
 // Both backward passes recompute the probabilities from the saved log-sum-exp with the same
 // accumulation order as the forward.
-#include <mutex>
-
 #include <cuda_bf16.h>
 
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "ptx.cuh"
-#include "rowops.cuh"
 #include "train_ops.cuh"
 
 namespace vitk {
@@ -476,18 +474,6 @@ int check_shape(int B, int N, int H, int hd, const DropParams* drop) {
   return VITK_OK;
 }
 
-template <typename K>
-int raise_smem(K kernel, size_t smem, const char* what) {
-  if (smem > 48 * 1024) {
-    const cudaError_t e =
-        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e != cudaSuccess)
-      return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(%s) failed: %s", what,
-                       cudaGetErrorString(e));
-  }
-  return VITK_OK;
-}
-
 }  // namespace
 
 bool attention_gen_fits(int N, int hd) {
@@ -515,8 +501,8 @@ int attention_gen_fwd(const void* qkv, void* ctx, float* lse, int B, int N, int 
   const size_t smem = 2 * static_cast<size_t>(N) * p.hdp * 2 + kGenWarps * (static_cast<size_t>(hd) + N) * 4;
   VITK_REQUIRE(smem <= 232448, "attention (generic): %d tokens x head_dim %d do not fit in shared "
                "memory", N, hd);
-  VITK_TRY(raise_smem(attn_gen_fwd_kernel, smem, "attn_gen_fwd_kernel"));
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(N) * N * hd, stream);
+  if (smem > 48 * 1024) VITK_TRY(opt_in_smem<attn_gen_fwd_kernel>(232448, "attn_gen_fwd_kernel"));
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, N, N, hd), stream);
   const dim3 grid((N + kGenRowsPerBlock - 1) / kGenRowsPerBlock, B * H);
   attn_gen_fwd_kernel<<<grid, kGenThreads, smem, stream>>>(p);
   VITK_CHECK_LAUNCH("attn_gen_fwd_kernel");
@@ -545,8 +531,8 @@ int attention_gen_bwd(const void* qkv, const void* ctx, const void* dctx, const 
   if (drop != nullptr) p.drop = *drop;
   const size_t smem = 2 * static_cast<size_t>(N) * p.hdp * 2 + 2 * static_cast<size_t>(N) * 4 +
                       kGenWarps * (2 * static_cast<size_t>(hd) + 2 * N) * 4;
-  VITK_TRY(raise_smem(attn_gen_bwd_kernel, smem, "attn_gen_bwd_kernel"));
-  ProfileScope prof(PROF_ATTN, 10.0 * B * H * static_cast<double>(N) * N * hd, stream);
+  if (smem > 48 * 1024) VITK_TRY(opt_in_smem<attn_gen_bwd_kernel>(232448, "attn_gen_bwd_kernel"));
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, N, N, hd, true), stream);
   const dim3 grid((N + kGenRowsPerBlock - 1) / kGenRowsPerBlock, B * H, 2);
   attn_gen_bwd_kernel<<<grid, kGenThreads, smem, stream>>>(p);
   VITK_CHECK_LAUNCH("attn_gen_bwd_kernel");
@@ -591,8 +577,8 @@ int attention_xgen_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc,
   const size_t smem = 2 * static_cast<size_t>(Nk) * p.hdp * 2 + kGenWarps * (static_cast<size_t>(hd) + Nk) * 4;
   VITK_REQUIRE(smem <= 232448, "attention (generic sources): %d keys x head_dim %d do not fit in "
                "shared memory", Nk, hd);
-  VITK_TRY(raise_smem(attn_xgen_fwd_kernel, smem, "attn_xgen_fwd_kernel"));
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * hd, stream);
+  if (smem > 48 * 1024) VITK_TRY(opt_in_smem<attn_xgen_fwd_kernel>(232448, "attn_xgen_fwd_kernel"));
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, Nq, Nk, hd), stream);
   const dim3 grid((Nq + kGenRowsPerBlock - 1) / kGenRowsPerBlock, B * H);
   attn_xgen_fwd_kernel<<<grid, kGenThreads, smem, stream>>>(p);
   VITK_CHECK_LAUNCH("attn_xgen_fwd_kernel");
@@ -625,8 +611,8 @@ int attention_xgen_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, lon
   const size_t smem = 2 * nmax * p.hdp * 2 + 2 * nmax * 4 + kGenWarps * (2 * static_cast<size_t>(hd) + 2 * nmax) * 4;
   VITK_REQUIRE(smem <= 232448, "attention_bwd (generic sources): %d x head_dim %d do not fit in "
                "shared memory", static_cast<int>(nmax), hd);
-  VITK_TRY(raise_smem(attn_xgen_bwd_kernel, smem, "attn_xgen_bwd_kernel"));
-  ProfileScope prof(PROF_ATTN, 10.0 * B * H * static_cast<double>(Nq) * Nk * hd, stream);
+  if (smem > 48 * 1024) VITK_TRY(opt_in_smem<attn_xgen_bwd_kernel>(232448, "attn_xgen_bwd_kernel"));
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, Nq, Nk, hd, true), stream);
   const int rows = Nq > Nk ? Nq : Nk;
   const dim3 grid((rows + kGenRowsPerBlock - 1) / kGenRowsPerBlock, B * H, 2);
   attn_xgen_bwd_kernel<<<grid, kGenThreads, smem, stream>>>(p);

@@ -14,11 +14,9 @@
 // buffer (no permute copies) and ctx is written directly in [B, N, H*hd] order.
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "ptx.cuh"
-#include "rowops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -151,7 +149,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     // ======================= softmax + output (thread == query row) =======================
     const int t = (warp - 4) >> 2;  // q-tile of this warpgroup
     const int q = warp & 3;         // TMEM lane quarter
-    const float c = p.scale * 1.44269504088896340736f;
+    const float c = p.scale * kLog2e;
     const int N = p.N;
     const int row_in_img0 = t * 128 + q * 32;  // first row of this warp
     const bool warp_active = (t < p.q_tiles);
@@ -301,21 +299,11 @@ int attention_fwd_tc(const void* qkv, void* ctx, float* lse, int B, int N, int H
   const int D = H * 64;
   const size_t smem = 2 * (2 * kQTileBytes + 2 * static_cast<size_t>(Nk) * 128) + 8 * 4096 + 256 + 1024;
   VITK_REQUIRE(smem <= 232448, "attention(tc): shared memory budget exceeded");
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention tc) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_fwd_tc_kernel>(232448, "attn_fwd_tc_kernel"));
   CUtensorMap tq, tkv, to;
-  const uint64_t row_pitch = static_cast<uint64_t>(3) * D * 2;
-  VITK_TRY(make_tmap_3d(&tq, qkv, 2, 3 * D, N, B, row_pitch, row_pitch * N, 64, 128));
-  VITK_TRY(make_tmap_3d(&tkv, qkv, 2, 3 * D, N, B, row_pitch, row_pitch * N, 64, Nk));
-  VITK_TRY(make_tmap_3d(&to, ctx, 2, D, N, B, static_cast<uint64_t>(D) * 2,
-                        static_cast<uint64_t>(D) * 2 * N, 64, 32));
+  VITK_TRY(make_row_map(&tq, qkv, B, N, 3 * D, 3 * D, 128));
+  VITK_TRY(make_row_map(&tkv, qkv, B, N, 3 * D, 3 * D, Nk));
+  VITK_TRY(make_row_map(&to, ctx, B, N, D, D, 32));
   TcParams prm;
   prm.B = B;
   prm.N = N;
@@ -324,9 +312,8 @@ int attention_fwd_tc(const void* qkv, void* ctx, float* lse, int B, int N, int H
   prm.q_tiles = (N + 127) / 128;
   prm.scale = 1.0f / sqrtf(static_cast<float>(hd));
   prm.lse = lse;
-  int grid = sm_count();
-  if (B * H < grid) grid = B * H;
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(N) * N * hd, stream);
+  const int grid = persistent_grid(B * H);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, N, N, hd), stream);
   attn_fwd_tc_kernel<<<grid, kTcThreads, smem, stream>>>(tq, tkv, to, prm);
   VITK_CHECK_LAUNCH("attn_fwd_tc_kernel");
   return VITK_OK;

@@ -24,12 +24,10 @@
 // Registers: 768 threads x 80 at launch, re-balanced with setmaxnreg to 40 / 88 (softmax) / 72.
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "dropout.cuh"
 #include "ptx.cuh"
-#include "rowops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -48,10 +46,6 @@ struct Tc2Params {
   float scale;
   float* lse;
 };
-
-__device__ __forceinline__ void named_bar_sync(int id, int threads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
-}
 
 // Row maximum over COLS score columns starting at key k0 (4 independent chains of 3-input max).
 template <int COLS>
@@ -307,7 +301,7 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tm_q,
     // ================= softmax (thread == one column quarter of one query row) ================
     const int cq = (warp - 4) >> 2;  // column quarter
     const int q = warp & 3;          // TMEM lane quarter
-    const float c = p.scale * 1.44269504088896340736f;
+    const float c = p.scale * kLog2e;
     const int N = p.N;
     const int kbeg = quarter_begin(cq);
     const int cols = quarter_begin(cq + 1) - kbeg;  // multiple of 16, <= 64
@@ -481,24 +475,12 @@ int attention_fwd_tc2(const void* qkv, void* ctx, float* lse, int B, int N, int 
       2 * (2 * static_cast<size_t>(kQTile) + 2 * static_cast<size_t>(Nk) * 128) + 8 * 4096 + 16384 +
       256 + 1024;
   VITK_REQUIRE(smem <= 232448, "attention(tc2): shared memory budget exceeded");
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_fwd_tc2_kernel<false>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (attr_err == cudaSuccess)
-      attr_err = cudaFuncSetAttribute(attn_fwd_tc2_kernel<true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention tc2) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_fwd_tc2_kernel<false>>(232448, "attn_fwd_tc2_kernel<false>"));
+  VITK_TRY(opt_in_smem<attn_fwd_tc2_kernel<true>>(232448, "attn_fwd_tc2_kernel<true>"));
   CUtensorMap tq, tkv, to;
-  const uint64_t row_pitch = static_cast<uint64_t>(3) * D * 2;
-  VITK_TRY(make_tmap_3d(&tq, qkv, 2, 3 * D, N, B, row_pitch, row_pitch * N, 64, 128));
-  VITK_TRY(make_tmap_3d(&tkv, qkv, 2, 3 * D, N, B, row_pitch, row_pitch * N, 64, Nk));
-  VITK_TRY(make_tmap_3d(&to, ctx, 2, D, N, B, static_cast<uint64_t>(D) * 2,
-                        static_cast<uint64_t>(D) * 2 * N, 64, 32));
+  VITK_TRY(make_row_map(&tq, qkv, B, N, 3 * D, 3 * D, 128));
+  VITK_TRY(make_row_map(&tkv, qkv, B, N, 3 * D, 3 * D, Nk));
+  VITK_TRY(make_row_map(&to, ctx, B, N, D, D, 32));
   Tc2Params prm;
   prm.B = B;
   prm.N = N;
@@ -511,9 +493,8 @@ int attention_fwd_tc2(const void* qkv, void* ctx, float* lse, int B, int N, int 
   if (drop != nullptr) prm.drop = *drop;
   VITK_REQUIRE(prm.drop.thresh == 0u || static_cast<long long>(B) * H * N * Nk < (1ll << 32),
                "attention: dropout index space exceeds 32 bits");
-  int grid = sm_count();
-  if (B * H < grid) grid = B * H;
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(N) * N * hd, stream);
+  const int grid = persistent_grid(B * H);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, N, N, hd), stream);
   if (prm.drop.thresh != 0u)
     attn_fwd_tc2_kernel<true><<<grid, kThreads2, smem, stream>>>(tq, tkv, to, prm);
   else

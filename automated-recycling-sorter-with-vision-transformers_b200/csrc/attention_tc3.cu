@@ -29,11 +29,9 @@
 // TMEM (512 columns): score regions [0,128) [128,256) [256,384) | O [384,448).
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "ptx.cuh"
-#include "rowops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -67,10 +65,6 @@ enum : int {
   kFinal = 32,   // [4 lane quarters] reference maximum of the finished q-tile published
   kNumBars3 = 36
 };
-
-__device__ __forceinline__ void named_bar_sync3(int id, int threads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
-}
 
 #ifdef VITK_ATTN_TRACE
 #define TR3(role, idx, k)                                                                  \
@@ -283,7 +277,7 @@ attn_fwd_tc3_kernel(const __grid_constant__ CUtensorMap tm_q,    // box {64, 128
     // ============ softmax: set = score region, thread == query row over the whole key block =====
     const int set = (warp - 4) >> 2;  // owns region `set` and the units u with u % 3 == set
     const int q = warp & 3;           // TMEM lane quarter
-    const float c = p.scale * 1.44269504088896340736f;
+    const float c = p.scale * kLog2e;
     const uint64_t cc = pack2(__float_as_uint(c), __float_as_uint(c));
     const int r_in_tile = q * 32 + lane;
     const uint32_t lane_off = static_cast<uint32_t>(q * 32) << 16;
@@ -558,24 +552,14 @@ int attention_fwd_tc3(const void* qkv, void* ctx, float* lse, int B, int N, int 
   const size_t smem = 2 * static_cast<size_t>(Nk) * 128 + 2 * kQTile3 + 4 * 4096 +
                       (2 * 4 * 128 * 2 + 2 * 128) * 4 + 8 * kNumBars3 + 64 + 1024;
   VITK_REQUIRE(smem <= 232448, "attention(tc3): shared memory budget exceeded");
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_fwd_tc3_kernel,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention tc3) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_fwd_tc3_kernel>(232448, "attn_fwd_tc3_kernel"));
   CUtensorMap tq, tkv, tkv_tail, to;
-  const uint64_t row_pitch = static_cast<uint64_t>(3) * D * 2;
   const int kv_box = Nk < 256 ? Nk : 256;
   const int kv_tail = (Nk >= 256 && Nk % 256 != 0) ? Nk % 256 : kv_box;
-  VITK_TRY(make_tmap_3d(&tq, qkv, 2, 3 * D, N, B, row_pitch, row_pitch * N, 64, 128));
-  VITK_TRY(make_tmap_3d(&tkv, qkv, 2, 3 * D, N, B, row_pitch, row_pitch * N, 64, kv_box));
-  VITK_TRY(make_tmap_3d(&tkv_tail, qkv, 2, 3 * D, N, B, row_pitch, row_pitch * N, 64, kv_tail));
-  VITK_TRY(make_tmap_3d(&to, ctx, 2, D, N, B, static_cast<uint64_t>(D) * 2,
-                        static_cast<uint64_t>(D) * 2 * N, 64, 32));
+  VITK_TRY(make_row_map(&tq, qkv, B, N, 3 * D, 3 * D, 128));
+  VITK_TRY(make_row_map(&tkv, qkv, B, N, 3 * D, 3 * D, kv_box));
+  VITK_TRY(make_row_map(&tkv_tail, qkv, B, N, 3 * D, 3 * D, kv_tail));
+  VITK_TRY(make_row_map(&to, ctx, B, N, D, D, 32));
   Tc3Params prm;
   prm.B = B;
   prm.N = N;
@@ -599,8 +583,8 @@ int attention_fwd_tc3(const void* qkv, void* ctx, float* lse, int B, int N, int 
       prm.parts = static_cast<int>(want);
     }
   }
-  if (static_cast<long long>(B) * H * prm.parts < grid) grid = B * H * prm.parts;
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(N) * N * hd, stream);
+  grid = persistent_grid(static_cast<long long>(B) * H * prm.parts);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, N, N, hd), stream);
   attn_fwd_tc3_kernel<<<grid, kThreads3, smem, stream>>>(tq, tkv, tkv_tail, to, prm);
   VITK_CHECK_LAUNCH("attn_fwd_tc3_kernel");
   return VITK_OK;

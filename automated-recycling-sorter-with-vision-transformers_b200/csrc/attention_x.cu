@@ -5,11 +5,9 @@
 // head_dim is not 64.  Scores are never materialised.
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "ptx.cuh"
-#include "rowops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -27,42 +25,6 @@ namespace {
 constexpr int kXWarps = 7;
 constexpr int kXThreads = kXWarps * 32;
 constexpr int kSegKeys = 208;
-
-__device__ __forceinline__ void mma_m16n8k16(float (&c)[4], const uint32_t (&a)[4], uint32_t b0,
-                                             uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
-      "{%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2,
-                                        uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_trans(uint32_t addr, uint32_t& r0, uint32_t& r1,
-                                              uint32_t& r2, uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void cp_async_16z(uint32_t dst, const void* src, bool valid) {
-  const int sz = valid ? 16 : 0;  // src-size 0 -> zero fill
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(sz)
-               : "memory");
-}
-__device__ __forceinline__ float quad_max(float v) {
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1));
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
-  return v;
-}
-__device__ __forceinline__ float quad_sum(float v) {
-  v += __shfl_xor_sync(0xffffffffu, v, 1);
-  v += __shfl_xor_sync(0xffffffffu, v, 2);
-  return v;
-}
 
 struct AttnXArgs {
   const __nv_bfloat16* q;  // row r of image b, head h: q + b*q_img + r*ldq + h*HD
@@ -100,7 +62,7 @@ __device__ __forceinline__ void attn_x_block(uint32_t sK, uint32_t sV, int key0,
         const int key = key0 + j * 8 + (lane & 7);
         const int ch = (lane >> 3) + 4 * half;
         uint32_t k0, k1, k2, k3;
-        ldsm_x4(sK + key * PITCH + ch * 16, k0, k1, k2, k3);
+        ldmatrix_x4(sK + key * PITCH + ch * 16, k0, k1, k2, k3);
         mma_m16n8k16(s[j], qa[2 * half], k0, k1);
         mma_m16n8k16(s[j], qa[2 * half + 1], k2, k3);
       }
@@ -160,7 +122,7 @@ __device__ __forceinline__ void attn_x_block(uint32_t sK, uint32_t sV, int key0,
       for (int jj = 0; jj < HD / 16; ++jj) {
         const int ch = 2 * jj + (mi >> 1);
         uint32_t v0, v1, v2, v3;
-        ldsm_x4_trans(sV + key * PITCH + ch * 16, v0, v1, v2, v3);
+        ldmatrix_x4_trans(sV + key * PITCH + ch * 16, v0, v1, v2, v3);
         mma_m16n8k16(o[2 * jj], pa, v0, v1);
         mma_m16n8k16(o[2 * jj + 1], pa, v2, v3);
       }
@@ -207,7 +169,7 @@ __global__ void __launch_bounds__(kXThreads, HD > 96 ? 1 : 2) attn_x_kernel(cons
 #pragma unroll
   for (int j = 0; j < NT; ++j) o[j][0] = o[j][1] = o[j][2] = o[j][3] = 0.f;
   float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-  const float c = a.scale * 1.44269504088896340736f;  // softmax in base 2
+  const float c = a.scale * kLog2e;  // softmax in base 2
 
   for (int seg0 = 0; seg0 < a.Nk; seg0 += kSegKeys) {
     const int nseg = min(kSegKeys, a.Nk - seg0);
@@ -217,14 +179,14 @@ __global__ void __launch_bounds__(kXThreads, HD > 96 ? 1 : 2) attn_x_kernel(cons
       const int row = idx / CH, ch = idx - row * CH;
       const bool valid = row < nseg;
       const size_t off = static_cast<size_t>(seg0 + (valid ? row : 0)) * a.ldkv + ch * 8;
-      cp_async_16z(sK + row * PITCH + ch * 16, kbase + off, valid);
+      cp_async_16(sK + row * PITCH + ch * 16, kbase + off, valid);
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
     for (int idx = tid; idx < nrows * CH; idx += kXThreads) {
       const int row = idx / CH, ch = idx - row * CH;
       const bool valid = row < nseg;
       const size_t off = static_cast<size_t>(seg0 + (valid ? row : 0)) * a.ldkv + ch * 8;
-      cp_async_16z(sV + row * PITCH + ch * 16, vbase + off, valid);
+      cp_async_16(sV + row * PITCH + ch * 16, vbase + off, valid);
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
     // K first: the score MMAs of the first key block start while V is still in flight
@@ -287,21 +249,12 @@ template <int HD>
 int launch_attn_x(const AttnXArgs& a, int B, cudaStream_t stream) {
   constexpr int PITCH = HD * 2 + 16;
   constexpr size_t smem = static_cast<size_t>(2 * kSegKeys + kXWarps * 16) * PITCH;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_x_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    static_cast<int>(smem));
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attn_x) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_x_kernel<HD>>(static_cast<int>(smem), "attn_x_kernel"));
   const dim3 grid(B * a.H, (a.Nq + kXWarps * 16 - 1) / (kXWarps * 16));
   attn_x_kernel<HD><<<grid, kXThreads, smem, stream>>>(a);
   VITK_CHECK_LAUNCH("attn_x_kernel");
   return VITK_OK;
 }
-
 
 }  // namespace
 
@@ -334,7 +287,7 @@ int attention_x(const void* q, long long q_img, int ldq, const void* k, const vo
   a.Nk = Nk;
   a.H = H;
   a.scale = 1.0f / sqrtf(static_cast<float>(hd));
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * hd, stream);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, Nq, Nk, hd), stream);
   switch (hd) {
     case 32: return launch_attn_x<32>(a, B, stream);
     case 64: return launch_attn_x<64>(a, B, stream);

@@ -12,19 +12,17 @@
 //
 // One CTA per (image, head): q, d_ctx, k, v of the head are staged once by cp.async into rows
 // padded by 16 bytes (conflict-free ldmatrix for every head size).  Two passes, as in
-// attention_bwd.cu, so that no sum ever crosses a warp: a warp owns 16 query rows (dq) or 16 key
+// attention_flash.cu, so that no sum ever crosses a warp: a warp owns 16 query rows (dq) or 16 key
 // rows (dk, dv) and walks the other side in chunks of 32, recomputing its score blocks with bf16
 // m16n8k16 MMAs (fp32 accumulate) from the saved log-sum-exp; the probabilities and dS go straight
 // from the accumulator registers into the A fragments of the second product.
 // (Replaces the CUDA-core attn_xgen_bwd_kernel for these shapes: 1.2 ms -> see DESIGN.md 3.7.)
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "dropout.cuh"
 #include "ptx.cuh"
-#include "rowops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -33,7 +31,6 @@ namespace {
 
 constexpr int kWarps = 8;
 constexpr int kThreads = kWarps * 32;
-constexpr float kLog2e = 1.44269504088896340736f;
 constexpr int kCW = 32;  // columns of a score block
 
 struct XmParams {
@@ -46,37 +43,6 @@ struct XmParams {
   float scale;
   DropParams drop;
 };
-
-__device__ __forceinline__ void mma16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0,
-                                         uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
-      "{%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void ldsm4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2,
-                                      uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void ldsm2(uint32_t addr, uint32_t& r0, uint32_t& r1) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x2.shared.b16 {%0,%1}, [%2];"
-               : "=r"(r0), "=r"(r1)
-               : "r"(addr));
-}
-__device__ __forceinline__ void ldsm4t(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2,
-                                       uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-               : "r"(addr));
-}
-__device__ __forceinline__ void cp16(uint32_t dst, const void* src, bool valid) {
-  const int sz = valid ? 16 : 0;  // size 0: the 16 bytes are zero-filled
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(sz)
-               : "memory");
-}
 
 template <int HD>
 struct Tile {
@@ -91,7 +57,7 @@ struct Tile {
     for (int idx = threadIdx.x; idx < rows16 * (HD / 8); idx += kThreads) {
       const int row = idx / (HD / 8), ch = idx - row * (HD / 8);
       const bool valid = row < rows;
-      cp16(at(dst, row, ch), src + static_cast<long long>(valid ? row : 0) * ld + ch * 8, valid);
+      cp_async_16(at(dst, row, ch), src + static_cast<long long>(valid ? row : 0) * ld + ch * 8, valid);
     }
   }
   // A fragments (m16 x HD) of rows [row0, row0 + 16)
@@ -100,7 +66,7 @@ struct Tile {
     const int r = row0 + (lane & 7) + ((lane >> 3) & 1) * 8;
 #pragma unroll
     for (int kk = 0; kk < kKS; ++kk)
-      ldsm4(at(base, r, kk * 2 + (lane >> 4)), a[kk][0], a[kk][1], a[kk][2], a[kk][3]);
+      ldmatrix_x4(at(base, r, kk * 2 + (lane >> 4)), a[kk][0], a[kk][1], a[kk][2], a[kk][3]);
   }
   // acc[16 x 32] = A[16 x HD] * Brows[row0 .. row0 + 32)[HD]^T; 8-row groups at or beyond `rem`
   // are skipped (acc = 0)
@@ -114,14 +80,14 @@ struct Tile {
 #pragma unroll
         for (int q4 = 0; q4 < HD / 32; ++q4) {
           uint32_t b0, b1, b2, b3;
-          ldsm4(at(sB, row, (lane >> 3) + 4 * q4), b0, b1, b2, b3);
-          mma16816(acc[j], a[2 * q4], b0, b1);
-          mma16816(acc[j], a[2 * q4 + 1], b2, b3);
+          ldmatrix_x4(at(sB, row, (lane >> 3) + 4 * q4), b0, b1, b2, b3);
+          mma_m16n8k16(acc[j], a[2 * q4], b0, b1);
+          mma_m16n8k16(acc[j], a[2 * q4 + 1], b2, b3);
         }
         if constexpr (HD % 32 != 0) {   // odd number of k-steps: the last one alone
           uint32_t b0, b1;
-          ldsm2(at(sB, row, ((lane >> 3) & 1) + 4 * (HD / 32)), b0, b1);
-          mma16816(acc[j], a[kKS - 1], b0, b1);
+          ldmatrix_x2(at(sB, row, ((lane >> 3) & 1) + 4 * (HD / 32)), b0, b1);
+          mma_m16n8k16(acc[j], a[kKS - 1], b0, b1);
         }
       }
     }
@@ -142,9 +108,9 @@ struct Tile {
 #pragma unroll
         for (int jj = 0; jj < kKS; ++jj) {
           uint32_t v0, v1, v2, v3;
-          ldsm4t(at(sB, row, 2 * jj + (mi >> 1)), v0, v1, v2, v3);
-          mma16816(out[2 * jj], wa, v0, v1);
-          mma16816(out[2 * jj + 1], wa, v2, v3);
+          ldmatrix_x4_trans(at(sB, row, 2 * jj + (mi >> 1)), v0, v1, v2, v3);
+          mma_m16n8k16(out[2 * jj], wa, v0, v1);
+          mma_m16n8k16(out[2 * jj + 1], wa, v2, v3);
         }
       }
     }
@@ -431,15 +397,7 @@ attn_xmma_fwd_kernel(const XmParams p, __nv_bfloat16* __restrict__ out, float* _
 template <int HD>
 int launch_xmma_fwd(const XmParams& p, int B, void* out, float* lse, cudaStream_t stream) {
   const size_t smem = static_cast<size_t>(p.Nq16 + 2 * p.Nk16) * Tile<HD>::kPitch;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_xmma_fwd_kernel<HD>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention xmma fwd) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_xmma_fwd_kernel<HD>>(232448, "attn_xmma_fwd_kernel"));
   attn_xmma_fwd_kernel<HD><<<B * p.H, kThreads, smem, stream>>>(p, static_cast<__nv_bfloat16*>(out), lse);
   VITK_CHECK_LAUNCH("attn_xmma_fwd_kernel");
   return VITK_OK;
@@ -453,15 +411,7 @@ size_t xmma_smem(int Nq16, int Nk16) {
 template <int HD>
 int launch_xmma(const XmParams& p, int B, cudaStream_t stream) {
   const size_t smem = xmma_smem<HD>(p.Nq16, p.Nk16);
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_xmma_bwd_kernel<HD>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention xmma) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_xmma_bwd_kernel<HD>>(232448, "attn_xmma_bwd_kernel"));
   attn_xmma_bwd_kernel<HD><<<B * p.H, kThreads, smem, stream>>>(p);
   VITK_CHECK_LAUNCH("attn_xmma_bwd_kernel");
   return VITK_OK;
@@ -469,7 +419,7 @@ int launch_xmma(const XmParams& p, int B, cudaStream_t stream) {
 
 }  // namespace
 
-bool attention_xmma_bwd_applicable(int Nq, int Nk, int hd) {
+bool attention_xmma_fits(int Nq, int Nk, int hd) {
   if (hd < 16 || hd > 128 || hd % 16 != 0) return false;
   if (Nq <= 0 || Nk <= 0) return false;
   const int Nq16 = (Nq + 15) & ~15, Nk16 = (Nk + 15) & ~15;
@@ -484,7 +434,7 @@ int attention_xmma_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, lon
                        cudaStream_t stream, const DropParams* drop) {
   VITK_REQUIRE(s.q && s.k && s.v && ctx && dctx && lse && dq && dk && dv,
                "attention_bwd (tensor-core, generic sources): null operand");
-  VITK_REQUIRE(B > 0 && H > 0 && attention_xmma_bwd_applicable(Nq, Nk, hd),
+  VITK_REQUIRE(B > 0 && H > 0 && attention_xmma_fits(Nq, Nk, hd),
                "attention_bwd (tensor-core, generic sources): head_dim a multiple of 16 up to 128 and queries + "
                "keys within shared memory (got %d x %d, head_dim %d)", Nq, Nk, hd);
   // 16-byte cp.async / uint4 reads and 4-byte paired stores
@@ -511,7 +461,7 @@ int attention_xmma_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, lon
   p.Nkp = (Nk + 15) & ~15;
   p.scale = 1.0f / sqrtf(static_cast<float>(hd));
   if (drop != nullptr) p.drop = *drop;
-  ProfileScope prof(PROF_ATTN, 10.0 * B * H * static_cast<double>(Nq) * Nk * hd, stream);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, Nq, Nk, hd, true), stream);
   switch (hd) {
     case 16: return launch_xmma<16>(p, B, stream);
     case 32: return launch_xmma<32>(p, B, stream);
@@ -527,7 +477,7 @@ int attention_xmma_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, lon
 int attention_xmma_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc, float* lse, int B,
                        int Nq, int Nk, int H, int hd, cudaStream_t stream, const DropParams* drop) {
   VITK_REQUIRE(s.q && s.k && s.v && ctx, "attention (tensor-core, generic sources): null operand");
-  VITK_REQUIRE(B > 0 && H > 0 && attention_xmma_bwd_applicable(Nq, Nk, hd),
+  VITK_REQUIRE(B > 0 && H > 0 && attention_xmma_fits(Nq, Nk, hd),
                "attention (tensor-core, generic sources): head_dim a multiple of 16 up to 128 and queries + keys "
                "within shared memory (got %d x %d, head_dim %d)", Nq, Nk, hd);
   VITK_REQUIRE(s.ldq % 8 == 0 && s.ldkv % 8 == 0 && ldc % 2 == 0 && s.q_img % 8 == 0 &&
@@ -546,7 +496,7 @@ int attention_xmma_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc,
   p.Nkp = (Nk + 15) & ~15;
   p.scale = 1.0f / sqrtf(static_cast<float>(hd));
   if (drop != nullptr) p.drop = *drop;
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * hd, stream);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, Nq, Nk, hd), stream);
   switch (hd) {
     case 16: return launch_xmma_fwd<16>(p, B, ctx, lse, stream);
     case 32: return launch_xmma_fwd<32>(p, B, ctx, lse, stream);

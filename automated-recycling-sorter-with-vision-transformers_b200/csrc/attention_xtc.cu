@@ -21,11 +21,9 @@
 // item's softmax runs.
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention_kernels.cuh"
 #include "common.h"
 #include "ptx.cuh"
-#include "rowops.cuh"
 
 namespace vitk {
 using namespace ptx;
@@ -181,7 +179,7 @@ attn_xtc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
     // ======================= softmax + output (thread == query row) =======================
     const int r = (warp - 4) >> 2;  // region / item parity of this warpgroup
     const int q = warp & 3;         // TMEM lane quarter
-    const float c = p.scale * 1.44269504088896340736f;
+    const float c = p.scale * kLog2e;
     const int N = p.Nkeys;
     const int row = q * 32 + lane;
     const bool warp_rows = q * 32 < p.Nq;
@@ -314,25 +312,13 @@ int launch_xtc(const void* q, long long q_img, int ldq, const void* k, const voi
   const size_t smem = static_cast<size_t>(NB) * (128 * 128 + 3 * static_cast<size_t>(prm.Nk) * 128) +
                       256 + 1024;
   VITK_REQUIRE(smem <= 232448, "attention(xtc): shared memory budget exceeded");
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(attn_xtc_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    232448);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(attention xtc) failed: %s",
-                     cudaGetErrorString(attr_err));
+  VITK_TRY(opt_in_smem<attn_xtc_kernel<HD>>(232448, "attn_xtc_kernel"));
   const int D = prm.H * HD;
   CUtensorMap tq, tk, tv;
-  VITK_TRY(make_tmap_3d(&tq, q, 2, D, prm.Nq, prm.B, static_cast<uint64_t>(ldq) * 2,
-                        static_cast<uint64_t>(q_img) * 2, 64, 128));
-  VITK_TRY(make_tmap_3d(&tk, k, 2, D, prm.Nkeys, prm.B, static_cast<uint64_t>(ldkv) * 2,
-                        static_cast<uint64_t>(kv_img) * 2, 64, prm.Nk));
-  VITK_TRY(make_tmap_3d(&tv, v, 2, D, prm.Nkeys, prm.B, static_cast<uint64_t>(ldkv) * 2,
-                        static_cast<uint64_t>(kv_img) * 2, 64, prm.Nk));
-  int grid = sm_count();
-  if (prm.B * prm.H < grid) grid = prm.B * prm.H;
+  VITK_TRY(make_row_map(&tq, q, prm.B, prm.Nq, D, ldq, 128, q_img));
+  VITK_TRY(make_row_map(&tk, k, prm.B, prm.Nkeys, D, ldkv, prm.Nk, kv_img));
+  VITK_TRY(make_row_map(&tv, v, prm.B, prm.Nkeys, D, ldkv, prm.Nk, kv_img));
+  const int grid = persistent_grid(prm.B * prm.H);
   attn_xtc_kernel<HD><<<grid, kThreads, smem, stream>>>(tq, tk, tv, prm);
   VITK_CHECK_LAUNCH("attn_xtc_kernel");
   return VITK_OK;
@@ -373,7 +359,7 @@ int attention_xtc(const void* q, long long q_img, int ldq, const void* k, const 
     if (q_img <= 0) q_img = static_cast<long long>(Nq) * ldq;
     if (kv_img <= 0) kv_img = static_cast<long long>(Nk) * ldkv;
   }
-  ProfileScope prof(PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * hd, stream);
+  ProfileScope prof(PROF_ATTN, attention_flops(B, H, Nq, Nk, hd), stream);
   switch (hd) {
     case 32: return launch_xtc<32>(q, q_img, ldq, k, v, kv_img, ldkv, prm, stream);
     case 64: return launch_xtc<64>(q, q_img, ldq, k, v, kv_img, ldkv, prm, stream);

@@ -122,6 +122,14 @@ int device_cc() {
   return g_cc[dev];
 }
 
+cudaError_t set_max_dynamic_smem(const void* kernel, int bytes) {
+  return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+}
+int smem_opt_in_failed(cudaError_t e, const char* kernel_name) {
+  return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(%s) failed: %s", kernel_name,
+                   cudaGetErrorString(e));
+}
+
 // cuTensorMapEncodeTiled is a driver entry point; resolve it through the runtime so libvitk does
 // not link against libcuda (only stubs exist on the build box).
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,
@@ -205,6 +213,13 @@ int make_tmap_3d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t in
   if (r != CUDA_SUCCESS)
     return set_error(VITK_ERR_CUDA, "cuTensorMapEncodeTiled(3d) failed (%d)", (int)r);
   return VITK_OK;
+}
+
+int make_row_map(CUtensorMap* out, const void* base, int B, int rows, int row_elems, long long pitch,
+                 int box_rows, long long img_stride) {
+  if (img_stride < 0) img_stride = static_cast<long long>(rows) * pitch;
+  return make_tmap_3d(out, base, 2, row_elems, rows, B, static_cast<uint64_t>(pitch) * 2,
+                      static_cast<uint64_t>(img_stride) * 2, 64, box_rows);
 }
 
 }  // namespace vitk

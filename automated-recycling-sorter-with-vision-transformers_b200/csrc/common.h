@@ -97,6 +97,27 @@ int sweep_next();  // direction for the kernel being launched: 0 ascending, 1 de
 int sm_count();
 void reserve_sms(int n);
 int device_cc();  // e.g. 100
+// Grid of a persistent kernel over `items` work items: one CTA per SM, fewer when items run out.
+inline int persistent_grid(long long items) {
+  const int sms = sm_count();
+  return items < sms ? static_cast<int>(items) : sms;
+}
+
+// Lets `Kernel` launch with up to `bytes` of dynamic shared memory.  cudaFuncSetAttribute runs on
+// the first call for each kernel in the process; later calls report its result.
+cudaError_t set_max_dynamic_smem(const void* kernel, int bytes);
+int smem_opt_in_failed(cudaError_t e, const char* kernel_name);
+template <auto Kernel>
+int opt_in_smem(int bytes, const char* kernel_name) {
+  static const cudaError_t e = set_max_dynamic_smem(reinterpret_cast<const void*>(Kernel), bytes);
+  return e == cudaSuccess ? VITK_OK : smem_opt_in_failed(e, kernel_name);
+}
+
+// FLOPs of softmax(q k^T) v over B * H heads (two products of 2 * Nq * Nk * hd each); the
+// backward recomputes the scores and forms four more products: 10 instead of 4.
+inline double attention_flops(int B, int H, int Nq, int Nk, int hd, bool backward = false) {
+  return (backward ? 10.0 : 4.0) * B * H * static_cast<double>(Nq) * Nk * hd;
+}
 
 // 2-D bf16 (or any 2-byte / 4-byte element) row-major tensor map: dims {inner, outer},
 // row pitch in bytes, box {box_inner, box_outer}, 128-byte swizzle. Cached by value.
@@ -110,5 +131,11 @@ int make_tmap_2d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t in
 int make_tmap_3d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t inner, uint64_t rows,
                  uint64_t batch, uint64_t row_pitch_bytes, uint64_t batch_pitch_bytes,
                  uint32_t box_inner, uint32_t box_rows);
+
+// Per-image row map: bf16 [B][rows][row_elems], rows `pitch` elements apart and images
+// `img_stride` elements apart (rows * pitch when negative); box of 64 elements (128 bytes,
+// swizzled) by `box_rows` rows.
+int make_row_map(CUtensorMap* out, const void* base, int B, int rows, int row_elems, long long pitch,
+                 int box_rows, long long img_stride = -1);
 
 }  // namespace vitk

@@ -19,8 +19,7 @@
 //   * attention (head_dim = D / 8 = 96 for ViT-B) never materialises [B, 8, Q, keys] scores.
 #include <cuda_bf16.h>
 
-#include <mutex>
-
+#include "attention.cuh"
 #include "common.h"
 #include "gemm_sm100.cuh"
 #include "ptx.cuh"
@@ -230,22 +229,11 @@ int check(const VitkDetectionHeadConfig* cfg, int batch, int n_tokens, int skip,
   return VITK_OK;
 }
 
-int attn_x(const HeadDims& d, int B, const void* q, long long q_img, int ldq, const void* k,
-           const void* v, long long kv_img, int ldkv, int Nk, void* ctx, cudaStream_t stream) {
-  const long long ctx_img = static_cast<long long>(d.Q) * d.D;
-  // tcgen05 kernel when the queries are one MMA tile and the keys one block (the reference's 100
-  // queries against 100 / 196 keys); attention impl 1 forces the mma.sync kernel (tests, A/B)
-  if (attention_impl() != 1 && attention_xtc_applicable(q_img, kv_img, B, d.Q, Nk, d.hd))
-    return attention_xtc(q, q_img, ldq, k, v, kv_img, ldkv, ctx, ctx_img, d.D, B, d.Q, Nk, d.H, d.hd,
-                         stream);
-  return attention_x(q, q_img, ldq, k, v, kv_img, ldkv, ctx, ctx_img, d.D, B, d.Q, Nk, d.H, d.hd,
-                     stream);
-}
-
 int head_forward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWeights* w,
                  const float* tokens, const HeadDims& d, float* class_logits, float* bbox,
                  const HeadWorkspace& ws, cudaStream_t stream) {
   const int D = d.D, M = static_cast<int>(d.M), Q = d.Q;
+  const long long imgD = static_cast<long long>(Q) * D;
   const __nv_bfloat16* qkv = static_cast<const __nv_bfloat16*>(ws.qkv);
   const __nv_bfloat16* kv = static_cast<const __nv_bfloat16*>(ws.kv);
   const int ldkv = d.L * 2 * D;
@@ -266,7 +254,8 @@ int head_forward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWeig
       VITK_TRY(cast_f32_to_bf16(w->object_queries, ws.xqb, static_cast<long long>(Q) * D, stream));
       VITK_TRY(linear_fwd(ws.xqb, D, lw.sa_in_w, Q, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, 0,
                           ws.qkv, nullptr, 3 * D, stream));
-      VITK_TRY(attn_x(d, 1, qkv, 0, 3 * D, qkv + D, qkv + 2 * D, 0, 3 * D, Q, ws.ctx, stream));
+      const AttnXSrc src{qkv, 0, 3 * D, qkv + D, qkv + 2 * D, 0, 3 * D};
+      VITK_TRY(attention_src_fwd(src, ws.ctx, imgD, D, nullptr, 1, Q, Q, d.H, d.hd, stream));
       VITK_TRY(linear_fwd(ws.ctx, D, lw.sa_out_w, Q, D, D, EPI_RESID_F32, lw.sa_out_b, ws.xq, D,
                           ws.xq, nullptr, D, stream));
       VITK_TRY(ln_post(ws.xq, Q, lw.norm1_w, lw.norm1_b, ws.x, ws.xb, M, D, cfg->ln_eps, stream));
@@ -274,7 +263,8 @@ int head_forward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWeig
       VITK_TRY(linear_fwd(ws.xb, D, lw.sa_in_w, M, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, 0,
                           ws.qkv, nullptr, 3 * D, stream));
       const long long img = static_cast<long long>(Q) * 3 * D;
-      VITK_TRY(attn_x(d, d.B, qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D, Q, ws.ctx, stream));
+      const AttnXSrc src{qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D};
+      VITK_TRY(attention_src_fwd(src, ws.ctx, imgD, D, nullptr, d.B, Q, Q, d.H, d.hd, stream));
       VITK_TRY(linear_fwd(ws.ctx, D, lw.sa_out_w, M, D, D, EPI_RESID_F32, lw.sa_out_b, ws.x, D,
                           ws.x, nullptr, D, stream));
       VITK_TRY(ln_post(ws.x, M, lw.norm1_w, lw.norm1_b, ws.x, ws.xb, M, D, cfg->ln_eps, stream));
@@ -284,8 +274,8 @@ int head_forward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWeig
                         nullptr, D, stream));
     {
       const __nv_bfloat16* kl = kv + static_cast<size_t>(d.skip) * ldkv + static_cast<size_t>(l) * 2 * D;
-      VITK_TRY(attn_x(d, d.B, qkv, static_cast<long long>(Q) * D, D, kl, kl + D,
-                      static_cast<long long>(d.Ntok) * ldkv, ldkv, d.P, ws.ctx, stream));
+      const AttnXSrc src{qkv, imgD, D, kl, kl + D, static_cast<long long>(d.Ntok) * ldkv, ldkv};
+      VITK_TRY(attention_src_fwd(src, ws.ctx, imgD, D, nullptr, d.B, Q, d.P, d.H, d.hd, stream));
     }
     VITK_TRY(linear_fwd(ws.ctx, D, lw.ca_out_w, M, D, D, EPI_RESID_F32, lw.ca_out_b, ws.x, D, ws.x,
                         nullptr, D, stream));
@@ -427,25 +417,11 @@ broadcast_rows_kernel(const float* __restrict__ in, int in_rows, float* __restri
   *reinterpret_cast<uint2*>(out_bf16 + i) = pk;
 }
 
-// attention with the log-sum-exp output: tcgen05 when the shape fits one query tile / key block
-// (no dropout on the probabilities), else the CUDA-core kernel
-int attn_train(const HeadDims& d, int B, const AttnXSrc& s, int Nk, void* ctx, float* lse,
-               cudaStream_t stream, const DropParams& drop = DropParams()) {
-  const long long ctx_img = static_cast<long long>(d.Q) * d.D;
-  if (attention_impl() != 1) {
-    if (drop.thresh == 0u && attention_xtc_applicable(s.q_img, s.kv_img, B, d.Q, Nk, d.hd))
-      return attention_xtc(s.q, s.q_img, s.ldq, s.k, s.v, s.kv_img, s.ldkv, ctx, ctx_img, d.D, B,
-                           d.Q, Nk, d.H, d.hd, stream, lse);
-    if (attention_xmma_bwd_applicable(d.Q, Nk, d.hd))   // dropout, or beyond one tcgen05 tile
-      return attention_xmma_fwd(s, ctx, ctx_img, d.D, lse, B, d.Q, Nk, d.H, d.hd, stream, &drop);
-  }
-  return attention_xgen_fwd(s, ctx, ctx_img, d.D, lse, B, d.Q, Nk, d.H, d.hd, stream, &drop);
-}
-
 int head_forward_train(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWeights* w,
                        const float* tokens, const HeadDims& d, float* class_logits, float* bbox,
                        const SavedHead& sv, const HeadTrainWs& ws, cudaStream_t stream) {
   const int D = d.D, M = static_cast<int>(d.M), Q = d.Q;
+  const long long imgD = static_cast<long long>(Q) * D;
   const HeadDrop drop{cfg->dropout_p, static_cast<uint32_t>(cfg->seed)};
   const __nv_bfloat16* kv = static_cast<const __nv_bfloat16*>(sv.kv);
   const int ldkv = d.L * 2 * D;
@@ -468,7 +444,7 @@ int head_forward_train(const VitkDetectionHeadConfig* cfg, const VitkDetectionHe
       VITK_TRY(linear_fwd(sl.xb_in, D, lw.sa_in_w, Q, 3 * D, D, EPI_BF16, lw.sa_in_b, nullptr, 0,
                           sl.qkv, nullptr, 3 * D, stream));
       const AttnXSrc src{qkv, 0, 3 * D, qkv + D, qkv + 2 * D, 0, 3 * D};
-      VITK_TRY(attn_train(d, 1, src, Q, sl.ctx_sa, sl.lse_sa, stream));
+      VITK_TRY(attention_src_fwd(src, sl.ctx_sa, imgD, D, sl.lse_sa, 1, Q, Q, d.H, d.hd, stream));
       VITK_TRY(linear_fwd(sl.ctx_sa, D, lw.sa_out_w, Q, D, D, EPI_RESID_F32, lw.sa_out_b, ws.xq, D,
                           ws.xq, nullptr, D, stream));
       VITK_TRY(ln_post(ws.xq, Q, lw.norm1_w, lw.norm1_b, ws.x, sl.xb1, M, D, cfg->ln_eps, stream,
@@ -479,8 +455,9 @@ int head_forward_train(const VitkDetectionHeadConfig* cfg, const VitkDetectionHe
                           sl.qkv, nullptr, 3 * D, stream));
       const long long img = static_cast<long long>(Q) * 3 * D;
       const AttnXSrc src{qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D};
-      VITK_TRY(attn_train(d, d.B, src, Q, sl.ctx_sa, sl.lse_sa, stream,
-                          drop.at(DROP_DEC_SA_ATTN, l)));
+      const DropParams drop_sa = drop.at(DROP_DEC_SA_ATTN, l);
+      VITK_TRY(attention_src_fwd(src, sl.ctx_sa, imgD, D, sl.lse_sa, d.B, Q, Q, d.H, d.hd, stream,
+                                 &drop_sa));
       VITK_TRY(linear_fwd(sl.ctx_sa, D, lw.sa_out_w, M, D, D, EPI_RESID_F32, lw.sa_out_b, ws.x, D,
                           ws.x, nullptr, D, stream, drop.at(DROP_DEC_SA_OUT, l)));
       VITK_TRY(ln_post(ws.x, M, lw.norm1_w, lw.norm1_b, ws.x, sl.xb1, M, D, cfg->ln_eps, stream,
@@ -490,10 +467,10 @@ int head_forward_train(const VitkDetectionHeadConfig* cfg, const VitkDetectionHe
                         nullptr, D, stream));
     {
       const __nv_bfloat16* kl = kv + static_cast<size_t>(d.skip) * ldkv + static_cast<size_t>(l) * 2 * D;
-      const AttnXSrc src{sl.qc, static_cast<long long>(Q) * D, D, kl, kl + D,
-                         static_cast<long long>(d.Ntok) * ldkv, ldkv};
-      VITK_TRY(attn_train(d, d.B, src, d.P, sl.ctx_ca, sl.lse_ca, stream,
-                          drop.at(DROP_DEC_CA_ATTN, l)));
+      const AttnXSrc src{sl.qc, imgD, D, kl, kl + D, static_cast<long long>(d.Ntok) * ldkv, ldkv};
+      const DropParams drop_ca = drop.at(DROP_DEC_CA_ATTN, l);
+      VITK_TRY(attention_src_fwd(src, sl.ctx_ca, imgD, D, sl.lse_ca, d.B, Q, d.P, d.H, d.hd, stream,
+                                 &drop_ca));
     }
     VITK_TRY(linear_fwd(sl.ctx_ca, D, lw.ca_out_w, M, D, D, EPI_RESID_F32, lw.ca_out_b, ws.x, D,
                         ws.x, nullptr, D, stream, drop.at(DROP_DEC_CA_OUT, l)));
@@ -633,19 +610,6 @@ accumulate_kernel(float* __restrict__ dst, const float* __restrict__ src, long l
   if (i < n) dst[i] += src[i];
 }
 
-// attention backward with separate sources: tensor cores (mma.sync) for head_dim 32 / 64 / 96,
-// the CUDA-core kernel otherwise (attention impl 1 forces the latter: tests, A/B)
-int attn_bwd_x(const AttnXSrc& s, const void* ctx, const void* dctx, long long ctx_img, int ldc,
-               const float* lse, void* dq, long long dq_img, int lddq, void* dk, void* dv,
-               long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
-               cudaStream_t stream, const DropParams* drop) {
-  if (attention_impl() != 1 && attention_xmma_bwd_applicable(Nq, Nk, hd))
-    return attention_xmma_bwd(s, ctx, dctx, ctx_img, ldc, lse, dq, dq_img, lddq, dk, dv, dkv_img,
-                              lddkv, B, Nq, Nk, H, hd, stream, drop);
-  return attention_xgen_bwd(s, ctx, dctx, ctx_img, ldc, lse, dq, dq_img, lddq, dk, dv, dkv_img,
-                            lddkv, B, Nq, Nk, H, hd, stream, drop);
-}
-
 // norm backward in place on the fp32 gradient stream: dx <- LN'(dx), bf16 copy, dgamma / dbeta
 // accumulated, column sums of the result into `colsum` (the bias gradient of the Linear whose
 // output the normalised sum received)
@@ -714,7 +678,7 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
       const AttnXSrc src{sl.qc, imgD, D, kv + koff, kv + koff + D,
                          static_cast<long long>(d.Ntok) * ldkv, ldkv};
       const DropParams drop_ca = drop.at(DROP_DEC_CA_ATTN, l);
-      VITK_TRY(attn_bwd_x(src, sl.ctx_ca, ws.dctx, imgD, D, sl.lse_ca, dqkv, imgD, D,
+      VITK_TRY(attention_src_bwd(src, sl.ctx_ca, ws.dctx, imgD, D, sl.lse_ca, dqkv, imgD, D,
                                   dkv + koff, dkv + koff + D, static_cast<long long>(d.Ntok) * ldkv,
                                   ldkv, d.B, Q, d.P, d.H, d.hd, stream, &drop_ca));
     }
@@ -731,7 +695,7 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
       const long long img = static_cast<long long>(Q) * 3 * D;
       const AttnXSrc src{qkv, img, 3 * D, qkv + D, qkv + 2 * D, img, 3 * D};
       const DropParams drop_sa = drop.at(DROP_DEC_SA_ATTN, l);
-      VITK_TRY(attn_bwd_x(src, sl.ctx_sa, ws.dctx, imgD, D, sl.lse_sa, dqkv, img, 3 * D,
+      VITK_TRY(attention_src_bwd(src, sl.ctx_sa, ws.dctx, imgD, D, sl.lse_sa, dqkv, img, 3 * D,
                                   dqkv + D, dqkv + 2 * D, img, 3 * D, d.B, Q, Q, d.H, d.hd, stream,
                                   &drop_sa));
       VITK_TRY(linear_dgrad(dqkv, 3 * D, lt.sa_in_wt, M, D, EPI_F32, nullptr, ws.x, 1.f, stream));
@@ -761,7 +725,7 @@ int head_backward(const VitkDetectionHeadConfig* cfg, const VitkDetectionHeadWei
       VITK_TRY(linear_wgrad(ws.dsumb, D, sl.ctx_sa, D, Q, lg.sa_out_w, nullptr, stream));
       const __nv_bfloat16* qkv = static_cast<const __nv_bfloat16*>(sl.qkv);
       const AttnXSrc src{qkv, 0, 3 * D, qkv + D, qkv + 2 * D, 0, 3 * D};
-      VITK_TRY(attn_bwd_x(src, sl.ctx_sa, ws.dctx, 0, D, sl.lse_sa, dqkv, 0, 3 * D, dqkv + D,
+      VITK_TRY(attention_src_bwd(src, sl.ctx_sa, ws.dctx, 0, D, sl.lse_sa, dqkv, 0, 3 * D, dqkv + D,
                           dqkv + 2 * D, 0, 3 * D, 1, Q, Q, d.H, d.hd, stream, nullptr));
       VITK_TRY(linear_dgrad(dqkv, 3 * D, lt.sa_in_wt, Q, D, EPI_F32, nullptr, ws.xq, 1.f, stream));
       VITK_TRY(linear_wgrad(dqkv, 3 * D, sl.xb_in, D, Q, lg.sa_in_w, lg.sa_in_b, stream));

@@ -18,8 +18,6 @@
 // and detection-head drivers share (linear_fwd, linear_dgrad, linear_wgrad, ...).
 #include "gemm_sm100.cuh"
 
-#include <mutex>
-
 #include "common.h"
 #include "ptx.cuh"
 #include "rowops.cuh"
@@ -1133,15 +1131,8 @@ template <int BLOCK_N, int EPI, int CTAS, bool TMA_EPI, bool MN>
 int launch(const GemmProblem& p, cudaStream_t stream) {
   using C = Cfg<BLOCK_N, CTAS, (TMA_EPI && EPI == EPI_DGELU_BF16) ? 3 : 2>;
   auto kernel = gemm_tn_kernel<BLOCK_N, EPI, CTAS, TMA_EPI, MN>;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [&] {
-    attr_err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    C::kSmemBytes);
-  });
-  if (attr_err != cudaSuccess)
-    return set_error(VITK_ERR_CUDA, "cudaFuncSetAttribute(gemm smem %d) failed: %s", C::kSmemBytes,
-                     cudaGetErrorString(attr_err));
+  VITK_TRY((opt_in_smem<gemm_tn_kernel<BLOCK_N, EPI, CTAS, TMA_EPI, MN>>(C::kSmemBytes,
+                                                                       "gemm_tn_kernel")));
   CUtensorMap ta, tb, tc, tc2;
   if constexpr (MN) {
     VITK_TRY(make_tmap_2d(&ta, p.A, 2, (uint64_t)p.M, (uint64_t)p.K, (uint64_t)p.lda * 2, 64, 64));

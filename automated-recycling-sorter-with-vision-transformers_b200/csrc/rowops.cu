@@ -648,8 +648,7 @@ int linear_rows_bwd(const float* x, long long row_stride, const float* w, const 
                "linear_rows_bwd: rows * n_out = %d * %d exceeds the staged 48 K values", rows, n_out);
   const size_t smem = static_cast<size_t>(rows) * n_out * sizeof(float);
   if (smem > 48 * 1024)
-    VITK_CHECK_CUDA(cudaFuncSetAttribute(linear_rows_bwd_kernel,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, 192 * 1024));
+    VITK_TRY(opt_in_smem<linear_rows_bwd_kernel>(192 * 1024, "linear_rows_bwd_kernel"));
   linear_rows_bwd_kernel<<<(D + 127) / 128, 128, smem, stream>>>(x, row_stride, w, dy, dx, dw, db,
                                                                  rows, D, n_out);
   VITK_CHECK_LAUNCH("linear_rows_bwd_kernel");

@@ -1,8 +1,6 @@
-// HBM-bound row kernels (rowops.cu) and the attention core (attention.cu): host launchers.
+// HBM-bound row kernels (rowops.cu): host launchers.
 #pragma once
 #include <cuda_runtime.h>
-
-#include "dropout.cuh"
 
 namespace vitk {
 
@@ -63,72 +61,5 @@ int postprocess_detections(const float* logits, const float* boxes, int batch, i
                            float* scores_out, cudaStream_t stream);
 
 int cast_f32_to_bf16(const float* in, void* out, long long n, cudaStream_t stream);
-
-// softmax(q k^T / sqrt(hd)) v for every (image, head); qkv bf16 [B*N, 3*D] packed as the reference
-// packs it (column = which*D + h*hd + d); ctx bf16 [B*N, D]; optional lse fp32 [B, H, N].
-// `drop` (training only): dropout on the attention probabilities (train.py:545), N <= 208.
-int attention_fwd(const void* qkv, void* ctx, float* lse, int B, int N, int H, int hd,
-                  cudaStream_t stream, const DropParams* drop = nullptr);
-
-// tcgen05 variant for N <= 256 (attention_tc.cu); attention_fwd dispatches to it automatically.
-int attention_fwd_tc(const void* qkv, void* ctx, float* lse, int B, int N, int H, int hd,
-                     cudaStream_t stream);
-// Item-pipelined tcgen05 variant for N <= 208 (attention_tc2.cu); the default for the 224 px models.
-int attention_fwd_tc2(const void* qkv, void* ctx, float* lse, int B, int N, int H, int hd,
-                      cudaStream_t stream, const DropParams* drop = nullptr);
-// Key-block tcgen05 variant (online softmax with a lazily moved reference) for long sequences, N <= 640 (attention_tc3.cu): 384 px -> 577 tokens.
-int attention_fwd_tc3(const void* qkv, void* ctx, float* lse, int B, int N, int H, int hd,
-                      cudaStream_t stream);
-// Generic-source attention (attention_x.cu): query rows at q + b*q_img + r*ldq + h*hd, keys / values
-// at k|v + b*kv_img + r*ldkv + h*hd, output at ctx + b*ctx_img + r*ldc + h*hd (all bf16, strides
-// in elements); head_dim 32 / 64 / 96 / 128.  Decoder self-/cross-attention and the encoder's
-// attention when head_dim != 64 (inference: no log-sum-exp output).
-int attention_x(const void* q, long long q_img, int ldq, const void* k, const void* v,
-                long long kv_img, int ldkv, void* ctx, long long ctx_img, int ldc, int B, int Nq,
-                int Nk, int H, int hd, cudaStream_t stream);
-// tcgen05 form of attention_x for one query tile and one key block (<= 128 queries, <= 256 keys):
-// the decoder layers of the detection head (attention_xtc.cu).
-bool attention_xtc_applicable(long long q_img, long long kv_img, int B, int Nq, int Nk, int hd);
-int attention_xtc(const void* q, long long q_img, int ldq, const void* k, const void* v,
-                  long long kv_img, int ldkv, void* ctx, long long ctx_img, int ldc, int B, int Nq,
-                  int Nk, int H, int hd, cudaStream_t stream, float* lse = nullptr);
-// Generic-source attention on CUDA cores with the log-sum-exp output, and its backward
-// (attention_gen.cu): the decoder layers of the detection head under training (any head_dim
-// 8 .. 128 in steps of 8, up to 1024 queries / keys).  Strides in elements; lse f32 [B, H, Nq].
-// Backward: dq rows at dq + b*dq_img + r*lddq + h*hd, dk / dv rows at dk|dv + b*dkv_img + r*lddkv +
-// h*hd (overwritten).
-struct AttnXSrc {
-  const void* q; long long q_img; int ldq;
-  const void* k; const void* v; long long kv_img; int ldkv;
-};
-int attention_xgen_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc, float* lse, int B,
-                       int Nq, int Nk, int H, int hd, cudaStream_t stream,
-                       const DropParams* drop = nullptr);
-// Tensor-core (mma.sync) forms of attention_xgen_fwd / _bwd for head_dim 16 .. 128 in steps of 16
-// (attention_xmma.cu): the detection head under training, and the encoder's own attention under
-// training when head_dim != 64; same contracts.
-bool attention_xmma_bwd_applicable(int Nq, int Nk, int hd);
-int attention_xmma_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc, float* lse, int B,
-                       int Nq, int Nk, int H, int hd, cudaStream_t stream,
-                       const DropParams* drop = nullptr);
-int attention_xmma_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, long long ctx_img,
-                       int ldc, const float* lse, void* dq, long long dq_img, int lddq, void* dk,
-                       void* dv, long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
-                       cudaStream_t stream, const DropParams* drop = nullptr);
-int attention_xgen_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, long long ctx_img,
-                       int ldc, const float* lse, void* dq, long long dq_img, int lddq, void* dk,
-                       void* dv, long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
-                       cudaStream_t stream, const DropParams* drop = nullptr);
-// CUDA-core attention for the shapes the tensor-core kernels do not cover (attention_gen.cu):
-// head_dim 8 .. 128 in steps of 8, up to 1024 tokens, optional log-sum-exp output and
-// attention-probability dropout - forward and (train_ops.cuh: attention_bwd) backward.
-bool attention_gen_fits(int N, int hd);
-int attention_gen_fwd(const void* qkv, void* ctx, float* lse, int B, int N, int H, int hd,
-                      cudaStream_t stream, const DropParams* drop = nullptr);
-int attention_gen_bwd(const void* qkv, const void* ctx, const void* dctx, const float* lse,
-                      void* dqkv, int B, int N, int H, int hd, cudaStream_t stream,
-                      const DropParams* drop, float* dbias);
-void attention_force_impl(int impl);
-int attention_impl();
 
 }  // namespace vitk

@@ -1,4 +1,4 @@
-// Host launchers of the training-step kernels (train_ops.cu, attention_bwd.cu).
+// Host launchers of the training-step kernels (train_ops.cu).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -64,22 +64,5 @@ int adamw_flat(float* p, const float* g, float* m, float* v, void* shadow_bf16, 
 // finish: folds the flag into the skipped count once the step's AdamW launches are queued.
 int grad_guard_scan(const float* g, long long n, int* guard, int reset, cudaStream_t stream);
 int grad_guard_finish(int* guard, cudaStream_t stream);
-
-// dqkv = backward of softmax(q k^T / sqrt(hd)) v given d_ctx, using the saved log-sum-exp.
-// dbias (optional, [3 H hd]) += column sums of dqkv: the bias gradient of the qkv Linear.
-int attention_bwd(const void* qkv, const void* ctx, const void* dctx, const float* lse, void* dqkv,
-                  int B, int N, int H, int hd, cudaStream_t stream,
-                  const DropParams* drop = nullptr, float* dbias = nullptr);
-
-// tcgen05 variant (attention_bwd_tc.cu); attention_bwd dispatches to it for N <= 256.
-int attention_bwd_tc(const void* qkv, const void* ctx, const void* dctx, const float* lse,
-                     void* dqkv, int B, int N, int H, int hd, cudaStream_t stream,
-                     const DropParams* drop = nullptr, float* dbias = nullptr);
-// Software-pipelined form of the same kernel (attention_bwd_tc2.cu: 64-query sub-blocks, score
-// tiles double-buffered in TMEM); preferred whenever its larger shared-memory footprint fits.
-bool attention_bwd_tc2_fits(int N, int H, bool with_dbias);
-int attention_bwd_tc2(const void* qkv, const void* ctx, const void* dctx, const float* lse,
-                      void* dqkv, int B, int N, int H, int hd, cudaStream_t stream,
-                      const DropParams* drop = nullptr, float* dbias = nullptr);
 
 }  // namespace vitk

@@ -167,8 +167,17 @@ int vitk_linear_rows_backward(const float* x, long long row_stride, const float*
  * for the NCCL kernels of a gradient all-reduce that overlaps the backward pass. 0 restores all. */
 int vitk_reserve_sms(int n);
 
-/* Attention kernel choice: 0 = automatic (tcgen05 single-key-block kernel when N <= 256, else the
- * flash kernel), 1 = flash (mma.sync, any N), 2 = tcgen05.  Tests and A/B timing. */
+/* Attention kernel choice, for tests and A/B timing (the table in csrc/attention.cu):
+ *   0 = automatic: by shape and device.
+ *   1 = no tcgen05 kernel where another one covers the call: the head_dim-64 mma.sync flash
+ *       kernels, the mma.sync generic-source inference kernel, and the CUDA-core training kernels
+ *       of the separate-source (detection head) and head_dim != 64 paths.  Dropout in the
+ *       head_dim-64 encoder still uses the tcgen05 kernels.
+ *   2-4 change the head_dim-64 inference / log-sum-exp forward only (elsewhere they act as 0):
+ *   2 = tcgen05 forwards chosen by N as 0 does (item-pipelined up to 208 tokens, single key block
+ *       up to 256, key blocks up to 640), also off sm_100;
+ *   3 = the single-key-block kernel up to 256 tokens, key blocks above (never the pipelined one);
+ *   4 = the key-block kernel for every N (up to 640). */
 int vitk_attention_set_impl(int impl);
 
 /* Scratch bytes vitk_forward needs for `batch` images. */
