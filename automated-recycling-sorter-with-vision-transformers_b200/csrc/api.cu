@@ -407,8 +407,10 @@ int vitk_forward_cls(const VitkConfig* cfg, const VitkWeights* w, const float* i
   VITK_TRY(check_config(cfg, batch, &d));
   VITK_REQUIRE(images != nullptr && logits_out != nullptr, "null argument");
   VITK_REQUIRE(cfg->precision == 0, "the CLS-only tail is implemented for the bf16 path");
-  VITK_REQUIRE(d.hd == 32 || d.hd == 64 || d.hd == 96 || d.hd == 128,
-               "head_dim %d unsupported (32, 64, 96 or 128)", d.hd);
+  VITK_REQUIRE(d.hd == 32 || d.hd == 64 || d.hd == 96 || d.hd == 128 ||
+                   attention_src_supported(1, d.N, d.hd),
+               "head_dim %d unsupported (32, 64, 96 or 128; any other head_dim from 16 to 128 up to "
+               "256 tokens)", d.hd);
   VITK_TRY(check_forward_args(cfg, w, d, nullptr, logits_out, workspace, workspace_bytes));
   return forward_bf16(cfg, w, images, d, nullptr, logits_out, carve(d, workspace),
                       static_cast<cudaStream_t>(stream), nullptr, true);
@@ -488,6 +490,34 @@ int vitk_attention(const void* qkv_bf16, void* ctx_bf16, float* lse_or_null, int
                    int num_heads, int head_dim, vitk_stream_t stream) {
   return attention_fwd(qkv_bf16, ctx_bf16, lse_or_null, batch, n_tokens, num_heads, head_dim,
                        static_cast<cudaStream_t>(stream));
+}
+
+int vitk_attention_src(const void* q, long long q_img, int ldq, const void* k, const void* v,
+                       long long kv_img, int ldkv, void* ctx, long long ctx_img, int ldc,
+                       float* lse_or_null, int batch, int n_q, int n_k, int num_heads,
+                       int head_dim, float dropout_p, unsigned int seed, int site, int layer,
+                       vitk_stream_t stream) {
+  VITK_REQUIRE(((site >= 0 && site <= 4) || (site >= 8 && site <= 13)) && layer >= 0,
+               "bad dropout site / layer (encoder sites 0..4, decoder-layer sites 8..13)");
+  const AttnXSrc src{q, q_img, ldq, k, v, kv_img, ldkv};
+  const DropParams drop = make_drop_params(dropout_p, seed, site, layer);
+  return attention_src_fwd(src, ctx, ctx_img, ldc, lse_or_null, batch, n_q, n_k, num_heads,
+                           head_dim, static_cast<cudaStream_t>(stream), &drop);
+}
+
+int vitk_attention_src_bwd(const void* q, long long q_img, int ldq, const void* k, const void* v,
+                           long long kv_img, int ldkv, const void* ctx, const void* dctx,
+                           long long ctx_img, int ldc, const float* lse, void* dq, long long dq_img,
+                           int lddq, void* dk, void* dv, long long dkv_img, int lddkv, int batch,
+                           int n_q, int n_k, int num_heads, int head_dim, float dropout_p,
+                           unsigned int seed, int site, int layer, vitk_stream_t stream) {
+  VITK_REQUIRE(((site >= 0 && site <= 4) || (site >= 8 && site <= 13)) && layer >= 0,
+               "bad dropout site / layer (encoder sites 0..4, decoder-layer sites 8..13)");
+  const AttnXSrc src{q, q_img, ldq, k, v, kv_img, ldkv};
+  const DropParams drop = make_drop_params(dropout_p, seed, site, layer);
+  return attention_src_bwd(src, ctx, dctx, ctx_img, ldc, lse, dq, dq_img, lddq, dk, dv, dkv_img,
+                           lddkv, batch, n_q, n_k, num_heads, head_dim,
+                           static_cast<cudaStream_t>(stream), &drop);
 }
 
 int vitk_patchify(const float* images, void* patches_bf16, int batch, int channels, int image_size,

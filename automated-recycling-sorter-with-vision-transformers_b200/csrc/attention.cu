@@ -16,10 +16,15 @@
 //              else hd != 64 or N > 256 or dropping: impl != 1 and xmma fits ->
 //                attn_xmma_bwd_kernel + colsum_bf16 (dbias), else attn_gen_bwd_kernel
 //              else attn_bwd_hd64_kernel + colsum_bf16 (dbias)
-// src fwd      no lse: impl != 1 and xtc applies -> attn_xtc_kernel, else attn_x_kernel
-//              lse: impl != 1, not dropping and xtc applies -> xtc; else impl != 1 and xmma fits
-//                -> attn_xmma_fwd_kernel; else attn_xgen_fwd_kernel
-// src bwd      impl != 1 and xmma fits -> attn_xmma_bwd_kernel, else attn_xgen_bwd_kernel
+// "ragged": hd not in {32, 64, 96, 128} and attention_src_supported(Nq, Nk, hd) (16 <= hd <= 128,
+// Nq <= 128, Nk <= 256): the shapes only the xr kernels (attention_xr.cu, attention_xr_bwd.cu) take.
+// src fwd      no lse: impl != 1 and xtc applies -> attn_xtc_kernel; ragged -> attn_xr_fwd_kernel
+//                (any impl); else attn_x_kernel
+//              lse: impl != 1, not dropping and xtc applies -> xtc; ragged, unless impl 1 and hd
+//                is a multiple of 8 -> xr; else impl != 1 and xmma fits -> attn_xmma_fwd_kernel;
+//                else attn_xgen_fwd_kernel
+// src bwd      ragged, unless impl 1 and hd is a multiple of 8 -> attn_xr_bwd_kernel; else
+//                impl != 1 and xmma fits -> attn_xmma_bwd_kernel, else attn_xgen_bwd_kernel
 #include "attention_kernels.cuh"
 #include "common.h"
 #include "train_ops.cuh"
@@ -39,6 +44,15 @@ enum AttnImpl : int {
 AttnImpl g_attn_impl = kImplAuto;
 
 bool dropping(const DropParams* drop) { return drop != nullptr && drop->thresh != 0u; }
+
+bool ragged(int Nq, int Nk, int hd) {
+  return !(hd == 32 || hd == 64 || hd == 96 || hd == 128) && attention_src_supported(Nq, Nk, hd);
+}
+
+// impl 1 keeps the CUDA-core training kernels wherever they take the head_dim
+bool xr_for_training(int Nq, int Nk, int hd) {
+  return ragged(Nq, Nk, hd) && !(g_attn_impl == kImplNoTcgen05 && hd % 8 == 0);
+}
 
 }  // namespace
 
@@ -120,12 +134,16 @@ int attention_src_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc, 
     if (tcgen05 && attention_xtc_applicable(s.q_img, s.kv_img, B, Nq, Nk, hd))
       return attention_xtc(s.q, s.q_img, s.ldq, s.k, s.v, s.kv_img, s.ldkv, ctx, ctx_img, ldc, B,
                            Nq, Nk, H, hd, stream);
+    if (ragged(Nq, Nk, hd))
+      return attention_xr_fwd(s, ctx, ctx_img, ldc, nullptr, B, Nq, Nk, H, hd, stream);
     return attention_x(s.q, s.q_img, s.ldq, s.k, s.v, s.kv_img, s.ldkv, ctx, ctx_img, ldc, B, Nq,
                        Nk, H, hd, stream);
   }
   if (tcgen05 && !dropping(drop) && attention_xtc_applicable(s.q_img, s.kv_img, B, Nq, Nk, hd))
     return attention_xtc(s.q, s.q_img, s.ldq, s.k, s.v, s.kv_img, s.ldkv, ctx, ctx_img, ldc, B, Nq,
                          Nk, H, hd, stream, lse);
+  if (xr_for_training(Nq, Nk, hd))
+    return attention_xr_fwd(s, ctx, ctx_img, ldc, lse, B, Nq, Nk, H, hd, stream, drop);
   if (tcgen05 && attention_xmma_fits(Nq, Nk, hd))
     return attention_xmma_fwd(s, ctx, ctx_img, ldc, lse, B, Nq, Nk, H, hd, stream, drop);
   return attention_xgen_fwd(s, ctx, ctx_img, ldc, lse, B, Nq, Nk, H, hd, stream, drop);
@@ -135,6 +153,9 @@ int attention_src_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, long
                       int ldc, const float* lse, void* dq, long long dq_img, int lddq, void* dk,
                       void* dv, long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
                       cudaStream_t stream, const DropParams* drop) {
+  if (xr_for_training(Nq, Nk, hd))
+    return attention_xr_bwd(s, ctx, dctx, ctx_img, ldc, lse, dq, dq_img, lddq, dk, dv, dkv_img,
+                            lddkv, B, Nq, Nk, H, hd, stream, drop);
   if (g_attn_impl != kImplNoTcgen05 && attention_xmma_fits(Nq, Nk, hd))
     return attention_xmma_bwd(s, ctx, dctx, ctx_img, ldc, lse, dq, dq_img, lddq, dk, dv, dkv_img,
                               lddkv, B, Nq, Nk, H, hd, stream, drop);

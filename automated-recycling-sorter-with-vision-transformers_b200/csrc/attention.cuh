@@ -41,6 +41,11 @@ int attention_src_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, long
                       void* dv, long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
                       cudaStream_t stream, const DropParams* drop = nullptr);
 
+// Whether the separate-source entry points take (Nq, Nk) at any head_dim hd, not only 32 / 64 /
+// 96 / 128, in every mode (inference, log-sum-exp, dropout, backward): 16 <= hd <= 128, at most
+// 128 queries and at most 256 keys.  A shape-only check, usable before anything is launched.
+bool attention_src_supported(int Nq, int Nk, int hd);
+
 // Whether attention_bwd covers N tokens of head_dim hd.
 bool attention_trainable(int N, int hd);
 

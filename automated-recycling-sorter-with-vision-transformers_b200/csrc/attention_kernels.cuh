@@ -72,6 +72,15 @@ int attention_xmma_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, lon
                        int ldc, const float* lse, void* dq, long long dq_img, int lddq, void* dk,
                        void* dv, long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
                        cudaStream_t stream, const DropParams* drop = nullptr);
+// tcgen05 forward (inference, log-sum-exp, dropout) and backward for any head_dim 16 .. 128 within
+// attention_src_supported: <= 128 queries, <= 256 keys (attention_xr.cu, attention_xr_bwd.cu).
+int attention_xr_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc, float* lse, int B,
+                     int Nq, int Nk, int H, int hd, cudaStream_t stream,
+                     const DropParams* drop = nullptr);
+int attention_xr_bwd(const AttnXSrc& s, const void* ctx, const void* dctx, long long ctx_img,
+                     int ldc, const float* lse, void* dq, long long dq_img, int lddq, void* dk,
+                     void* dv, long long dkv_img, int lddkv, int B, int Nq, int Nk, int H, int hd,
+                     cudaStream_t stream, const DropParams* drop = nullptr);
 // CUDA-core training forward and backward, head_dim 8 .. 128 in steps of 8, up to 1024 queries /
 // keys (attention_gen.cu).
 int attention_xgen_fwd(const AttnXSrc& s, void* ctx, long long ctx_img, int ldc, float* lse, int B,

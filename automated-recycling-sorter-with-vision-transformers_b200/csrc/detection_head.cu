@@ -201,8 +201,14 @@ int check(const VitkDetectionHeadConfig* cfg, int batch, int n_tokens, int skip,
                "detection head: embed_dim %d must be divisible by num_heads %d", cfg->embed_dim,
                cfg->num_heads);
   d->hd = cfg->embed_dim / cfg->num_heads;
-  VITK_REQUIRE(d->hd == 32 || d->hd == 64 || d->hd == 96 || d->hd == 128,
-               "detection head: head_dim %d unsupported (32, 64, 96 or 128)", d->hd);
+  // 32 / 64 / 96 / 128 at any token count; any other head_dim from 16 to 128 within the envelope
+  // of the ragged-head_dim attention kernels, for both the self- and the cross-attention
+  const bool regular_hd = d->hd == 32 || d->hd == 64 || d->hd == 96 || d->hd == 128;
+  VITK_REQUIRE(regular_hd || (attention_src_supported(cfg->num_queries, cfg->num_queries, d->hd) &&
+                              attention_src_supported(cfg->num_queries, n_tokens - skip, d->hd)),
+               "detection head: head_dim %d unsupported (32, 64, 96 or 128 at any size; any other "
+               "head_dim from 16 to 128 needs <= 128 queries and <= 256 memory tokens, got %d "
+               "queries and %d memory tokens)", d->hd, cfg->num_queries, n_tokens - skip);
   VITK_REQUIRE(cfg->embed_dim % 8 == 0 && cfg->embed_dim <= 128 * kLnVec && cfg->ffn_dim > 0 &&
                    cfg->ffn_dim % 8 == 0,
                "detection head: embed_dim (<= %d) and ffn_dim must be multiples of 8", 128 * kLnVec);

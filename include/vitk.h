@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define VITK_ABI_VERSION 6
+#define VITK_ABI_VERSION 7
 
 #define VITK_OK 0
 #define VITK_ERR_INVALID 1
@@ -194,7 +194,8 @@ int vitk_forward(const VitkConfig* cfg, const VitkWeights* w, const float* image
  * vitk_forward(tokens_out = NULL) returns, but since head(LN(x)[:, 0]) reads a single row per
  * image, the last block's attention is run for that one query (against the keys / values of all
  * tokens) and its projection, LayerNorm and MLP on `batch` rows instead of batch * N - 71 % of the
- * last block's contraction work feeds nothing the classifier returns.  bf16 mode. */
+ * last block's contraction work feeds nothing the classifier returns.  bf16 mode; head_dim 32,
+ * 64, 96 or 128, or any other head_dim from 16 to 128 up to 256 tokens (train.py's Config: 16). */
 int vitk_forward_cls(const VitkConfig* cfg, const VitkWeights* w, const float* images, int batch,
                      float* logits_out, void* workspace, size_t workspace_bytes,
                      vitk_stream_t stream);
@@ -300,6 +301,21 @@ int vitk_layernorm(const float* x, long long in_stride, const float* gamma, cons
 /* MultiHeadSelfAttention core (train.py:537-549) on the packed qkv activation. */
 int vitk_attention(const void* qkv_bf16, void* ctx_bf16, float* lse_or_null, int batch, int n_tokens,
                    int num_heads, int head_dim, vitk_stream_t stream);
+
+/* Attention with separate query and key / value sources (the detection head's decoder attentions,
+ * unit tests): per (image, head) ctx = softmax(q k^T / sqrt(head_dim)) v, bf16.  Query row r of
+ * image b at q + b*q_img + r*ldq + h*head_dim, key / value rows at k|v + b*kv_img + r*ldkv +
+ * h*head_dim, output rows at ctx + b*ctx_img + r*ldc + h*head_dim (strides in elements; q, k, v
+ * 16-byte aligned with pitches that are multiples of 8).  head_dim 32 / 64 / 96 / 128, or any
+ * other head_dim from 16 to 128 with n_q <= 128 and n_k <= 256.  lse_or_null (fp32
+ * [batch, num_heads, n_q]) selects the training forward; only then is dropout_p applied to the
+ * probabilities, with the masks of vitk_dropout_keep_mask(dropout_p, seed, site, layer) at index
+ * ((b*num_heads + h)*n_q + i)*Nk + j, Nk = n_k rounded up to 16. */
+int vitk_attention_src(const void* q, long long q_img, int ldq, const void* k, const void* v,
+                       long long kv_img, int ldkv, void* ctx, long long ctx_img, int ldc,
+                       float* lse_or_null, int batch, int n_q, int n_k, int num_heads,
+                       int head_dim, float dropout_p, unsigned int seed, int site, int layer,
+                       vitk_stream_t stream);
 
 /* Conv2d(k=p, s=p) input gather: f32 NCHW -> bf16 [B*P, C*p*p] (train.py:505-515). */
 int vitk_patchify(const float* images, void* patches_bf16, int batch, int channels, int image_size,
@@ -460,6 +476,15 @@ int vitk_layernorm_bwd(const void* dy, int dy_is_f32, const float* x, const floa
 int vitk_attention_bwd(const void* qkv_bf16, const void* ctx_bf16, const void* dctx_bf16,
                        const float* lse, void* dqkv_bf16, int batch, int n_tokens, int num_heads,
                        int head_dim, vitk_stream_t stream);
+/* Backward of vitk_attention_src with its saved log-sum-exp and the same dropout arguments: dq
+ * rows at dq + b*dq_img + r*lddq + h*head_dim, dk / dv rows at dk|dv + b*dkv_img + r*lddkv +
+ * h*head_dim (exactly head_dim columns of each row are written). */
+int vitk_attention_src_bwd(const void* q, long long q_img, int ldq, const void* k, const void* v,
+                           long long kv_img, int ldkv, const void* ctx, const void* dctx,
+                           long long ctx_img, int ldc, const float* lse, void* dq, long long dq_img,
+                           int lddq, void* dk, void* dv, long long dkv_img, int lddkv, int batch,
+                           int n_q, int n_k, int num_heads, int head_dim, float dropout_p,
+                           unsigned int seed, int site, int layer, vitk_stream_t stream);
 int vitk_colsum_bf16(const void* y, long long ld, int M, int N, float* out, vitk_stream_t stream);
 
 /* ============ detection head (ObjectDetectionHead, evaluation.py:160-200 == train.py:691-731) ====
@@ -475,7 +500,8 @@ int vitk_colsum_bf16(const void* y, long long ld, int M, int N, float* out, vitk
  * linear1, linear2, norm1, norm2, norm3}. */
 typedef struct VitkDetectionHeadConfig {
   int embed_dim;   /* D (768) */
-  int num_heads;   /* 8: head_dim = D / 8 must be 32, 64, 96 or 128 */
+  int num_heads;   /* 8: head_dim = D / 8 of 32, 64, 96 or 128, or any other head_dim from 16 to
+                    * 128 with num_queries <= 128 and at most 256 memory tokens (D = 400: 50) */
   int ffn_dim;     /* 2048 */
   int num_layers;  /* 6 */
   int num_queries; /* 100 */
