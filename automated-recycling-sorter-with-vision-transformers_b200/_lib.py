@@ -15,7 +15,7 @@ PKG_DIR = Path(__file__).resolve().parent
 # VITK_LIB: another build of the same library (same ABI), for A/B timing of kernel variants on one box
 LIB_PATH = Path(os.environ["VITK_LIB"]) if os.environ.get("VITK_LIB") else PKG_DIR / "libvitk.so"
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 EPI_BF16 = 0
 EPI_GELU_BF16 = 1
@@ -217,7 +217,15 @@ _SIGNATURES = {
                                               C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p]),
     "vitk_layernorm_bwd": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
-                                     C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+                                     C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_float, C.c_uint,
+                                     C.c_int, C.c_int, C.c_void_p]),
+    "vitk_classifier_head_loss_backward": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p,
+                                                     C.c_void_p, C.c_void_p, C.c_void_p,
+                                                     C.c_void_p, C.c_float, C.c_float, C.c_int,
+                                                     C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                                     C.c_void_p, C.c_void_p, C.c_void_p,
+                                                     C.c_void_p, C.c_void_p, C.c_void_p,
+                                                     C.c_void_p, C.c_void_p, C.c_void_p]),
     "vitk_attention_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vitk_attention_src": (C.c_int, [C.c_void_p, C.c_longlong, C.c_int, C.c_void_p, C.c_void_p,

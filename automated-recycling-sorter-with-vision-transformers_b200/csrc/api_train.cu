@@ -234,9 +234,13 @@ using namespace vitk;
 
 extern "C" {
 
+static bool valid_drop_site(int site, int layer) {
+  return ((site >= 0 && site <= 4) || (site >= 8 && site <= 13)) && layer >= 0;
+}
+
 int vitk_dropout_keep_mask(float p, unsigned int seed, int site, int layer, long long n,
                            unsigned char* out, vitk_stream_t stream) {
-  VITK_REQUIRE(((site >= 0 && site <= 4) || (site >= 8 && site <= 13)) && layer >= 0,
+  VITK_REQUIRE(valid_drop_site(site, layer),
                "bad dropout site / layer (encoder sites 0..4, decoder-layer sites 8..13)");
   return dropout_keep_mask(out, n, make_drop_params(p, seed, site, layer),
                            static_cast<cudaStream_t>(stream));
@@ -369,9 +373,25 @@ int vitk_transpose_bf16_batched(int n, const void* const* src, void* const* dst,
 int vitk_layernorm_bwd(const void* dy, int dy_is_f32, const float* x, const float* mean,
                        const float* rstd, const float* gamma, float* dx_io, int add_resid,
                        void* dx_bf16, float* dgamma, float* dbeta, int rows, int D,
+                       float* dx_colsum, float dropout_p, unsigned int seed, int site, int layer,
                        vitk_stream_t stream) {
+  VITK_REQUIRE(dropout_p <= 0.f || valid_drop_site(site, layer),
+               "bad dropout site / layer (encoder sites 0..4, decoder-layer sites 8..13)");
+  const DropParams drop = make_drop_params(dropout_p, seed, site, layer);
   return layernorm_bwd(dy, dy_is_f32, D, x, D, mean, rstd, gamma, dx_io, D, add_resid, dx_bf16, D,
-                       dgamma, dbeta, rows, D, static_cast<cudaStream_t>(stream));
+                       dgamma, dbeta, rows, D, static_cast<cudaStream_t>(stream), dx_colsum, &drop);
+}
+
+int vitk_classifier_head_loss_backward(const float* x, long long row_stride, const float* gamma,
+                                       const float* beta, const float* head_w, const float* head_b,
+                                       const long long* labels, float scale, float eps, int batch,
+                                       int D, int n_classes, float* logits_out, float* loss_out,
+                                       float* feat_ws, float* dlogits_ws, float* dx,
+                                       void* dx_bf16, float* dgamma, float* dbeta, float* dhead_w,
+                                       float* dhead_b, vitk_stream_t stream) {
+  return cls_loss_bwd(x, row_stride, gamma, beta, head_w, head_b, labels, scale, eps, batch, D,
+                      n_classes, logits_out, loss_out, feat_ws, dlogits_ws, dx, dx_bf16, dgamma,
+                      dbeta, dhead_w, dhead_b, static_cast<cudaStream_t>(stream));
 }
 
 int vitk_attention_bwd(const void* qkv_bf16, const void* ctx_bf16, const void* dctx_bf16,

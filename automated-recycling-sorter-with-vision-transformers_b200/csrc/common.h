@@ -51,6 +51,12 @@ long long launch_count();
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// True when p (null counts as aligned) is a multiple of `bytes`: the host-side check in front of
+// kernels that move 8- or 16-byte vectors.
+inline bool is_aligned(const void* p, uintptr_t bytes) {
+  return (reinterpret_cast<uintptr_t>(p) & (bytes - 1)) == 0;
+}
+
 // Lays buffers out in a caller-provided workspace, one after the other in the order they are
 // taken, each at a 1024-byte aligned offset.  A null base hands out null pointers and only counts
 // the bytes (the workspace-size queries).

@@ -345,6 +345,11 @@ int layernorm_fwd(const float* x, long long in_stride, const float* gamma, const
   VITK_REQUIRE(D % 4 == 0 && D <= 128 * kLnMaxVec, "layernorm: D=%d unsupported (need D%%4==0, D<=%d)",
                D, 128 * kLnMaxVec);
   VITK_REQUIRE(in_stride % 4 == 0 && out_stride % 4 == 0, "layernorm: strides must be multiples of 4");
+  // 16-byte row loads / stores (8-byte for bf16 rows)
+  VITK_REQUIRE(is_aligned(x, 16) && is_aligned(gamma, 16) && is_aligned(beta, 16) &&
+                   is_aligned(x_copy, 16) && is_aligned(y, y_is_f32 ? 16 : 8),
+               "layernorm: x, gamma, beta and x_copy must be 16-byte aligned, y %d-byte aligned",
+               y_is_f32 ? 16 : 8);
   const int block = 256;
   const int grid = (rows + 7) / 8;
   ProfileScope prof(PROF_LN, static_cast<double>(rows) * D * (4.0 + (y_is_f32 ? 4.0 : 2.0)), stream);

@@ -37,6 +37,11 @@ int grid_for(long long work_items, int block, int max_blocks_per_sm = 8) {
   return static_cast<int>(g);
 }
 
+// colsum_bf16_kernel reads 16-byte vectors of 8 columns
+bool colsum_args_ok(const void* y, long long ld, int N) {
+  return N % 8 == 0 && ld % 8 == 0 && is_aligned(y, 16);
+}
+
 // ------------------------------------------------------------------------------------------------
 // LayerNorm backward.  y = (x - mean) * rstd * gamma + beta  (reference nn.LayerNorm, train.py:581).
 //   dx = rstd * (g - mean_D(g) - xhat * mean_D(g * xhat)),  g = dy * gamma
@@ -799,22 +804,38 @@ int layernorm_bwd(const void* dy, int dy_is_f32, long long dy_stride, const floa
                   float* dx_io, long long dx_stride, int add_resid, void* dx_bf16,
                   long long dxb_stride, float* dgamma, float* dbeta, int rows, int D,
                   cudaStream_t stream, float* dx_colsum, const DropParams* drop) {
+  // every argument is checked here, before the first launch: a rejected call leaves dx_io,
+  // dgamma, dbeta and dx_colsum as they were
   VITK_REQUIRE(dy && x && mean && rstd && gamma && dx_io, "layernorm_bwd: null operand");
   const DropParams dp = drop != nullptr ? *drop : DropParams();
   const bool dropping = dp.thresh != 0u;
   VITK_REQUIRE(rows > 0 && D % 4 == 0 && D <= 128 * kLnMaxVec, "layernorm_bwd: bad shape");
+  VITK_REQUIRE(dy_stride % 4 == 0 && x_stride % 4 == 0 && dx_stride % 4 == 0 && dxb_stride % 4 == 0,
+               "layernorm_bwd: strides must be multiples of 4");
+  // 16-byte row accesses (8-byte for bf16 rows)
+  VITK_REQUIRE(is_aligned(dy, dy_is_f32 ? 16 : 8) && is_aligned(x, 16) && is_aligned(gamma, 16) &&
+                   is_aligned(dx_io, 16) && is_aligned(dx_bf16, 8),
+               "layernorm_bwd: x, gamma, dx_io (and an f32 dy) must be 16-byte aligned, a bf16 dy "
+               "and dx_bf16 8-byte aligned");
   VITK_REQUIRE((dgamma == nullptr) == (dbeta == nullptr), "layernorm_bwd: dgamma/dbeta together");
   const int block = 256;
   const int grid = (rows + 7) / 8;
   const __nv_bfloat16* dyb = static_cast<const __nv_bfloat16*>(dy);
   const float* dyf = static_cast<const float*>(dy);
   const int nv = (D / 4 + 31) / 32;
+  const bool fused = dgamma != nullptr && nv <= 6;
   VITK_REQUIRE(dx_colsum == nullptr || dx_bf16 != nullptr,
                "layernorm_bwd: dx_colsum needs the bf16 output");
+  // without the fused kernel the column sums are a colsum_bf16 pass over dx_bf16
+  VITK_REQUIRE(dx_colsum == nullptr || fused || colsum_args_ok(dx_bf16, dxb_stride, D),
+               "layernorm_bwd: dx_colsum outside the fused kernel (dgamma given, D <= 768) needs "
+               "D and the bf16 row pitch to be multiples of 8 and dx_bf16 16-byte aligned");
   VITK_REQUIRE(!dropping || (dx_bf16 != nullptr && dxb_stride == D &&
                              static_cast<long long>(rows) * D < (1ll << 32)),
                "layernorm_bwd: the dropout mask applies to a dense bf16 output");
-  if (dgamma != nullptr && nv <= 6) {
+  VITK_REQUIRE(!dropping || fused,
+               "layernorm_bwd: dropout needs the fused kernel (parameter gradients, D <= 768)");
+  if (fused) {
     // one pass: dx and the parameter gradients together
     ProfileScope prof(PROF_LN, static_cast<double>(rows) * D * (dy_is_f32 ? 14.0 : 12.0), stream);
     int fgrid = sm_count() * 2;
@@ -837,7 +858,6 @@ int layernorm_bwd(const void* dy, int dy_is_f32, long long dy_stride, const floa
     VITK_CHECK_LAUNCH("layernorm_bwd_fused_kernel");
     return VITK_OK;
   }
-  VITK_REQUIRE(!dropping, "layernorm_bwd: dropout needs the fused kernel (parameter gradients, D <= 768)");
   if (dgamma != nullptr) {
     // parameter gradients first: they read dy / x only, before dx_io is updated in place
     const int strips = (D + 255) / 256;
@@ -874,15 +894,13 @@ int layernorm_bwd(const void* dy, int dy_is_f32, long long dy_stride, const floa
   }
 #undef VITK_LN_BWD
   VITK_CHECK_LAUNCH("layernorm_bwd_dx_kernel");
-  if (dx_colsum != nullptr) {
-    VITK_REQUIRE(dx_bf16 != nullptr, "layernorm_bwd: dx_colsum needs the bf16 output");
-    return colsum_bf16(dx_bf16, dxb_stride, rows, D, dx_colsum, stream);
-  }
+  if (dx_colsum != nullptr) return colsum_bf16(dx_bf16, dxb_stride, rows, D, dx_colsum, stream);
   return VITK_OK;
 }
 
 int colsum_bf16(const void* y, long long ld, int M, int N, float* out, cudaStream_t stream) {
   VITK_REQUIRE(y && out && M > 0 && N > 0 && N % 8 == 0 && ld % 8 == 0, "colsum: bad argument");
+  VITK_REQUIRE(colsum_args_ok(y, ld, N), "colsum: y must be 16-byte aligned");
   const int strips = (N + 511) / 512;
   int chunks = (sm_count() * 12 + strips - 1) / strips;
   if (chunks > (M + 31) / 32) chunks = (M + 31) / 32;
@@ -903,7 +921,9 @@ int cls_loss_bwd(const float* x, long long row_stride, const float* gamma, const
                  float* dhead_w, float* dhead_b, cudaStream_t stream) {
   VITK_REQUIRE(x && gamma && beta && head_w && head_b && labels && dx && feat_ws && dlogits_ws,
                "cls_loss_bwd: null operand");
-  VITK_REQUIRE(B > 0 && D > 0 && C > 0 && C <= 1024, "cls_loss_bwd: bad shape");
+  VITK_REQUIRE(B > 0 && D > 0 && C > 0 && C <= 1024 && row_stride >= D, "cls_loss_bwd: bad shape");
+  VITK_REQUIRE((dgamma == nullptr) == (dbeta == nullptr), "cls_loss_bwd: dgamma/dbeta together");
+  VITK_REQUIRE((dhead_w == nullptr) == (dhead_b == nullptr), "cls_loss_bwd: dhead_w/dhead_b together");
   const size_t smem = (2 * static_cast<size_t>(D) + 8 + 2 * C) * sizeof(float);
   cls_loss_bwd_kernel<<<B, 128, smem, stream>>>(x, row_stride, gamma, beta, head_w, head_b, labels,
                                                 scale, eps, D, C, logits_out, loss_out, feat_ws,
@@ -911,7 +931,6 @@ int cls_loss_bwd(const float* x, long long row_stride, const float* gamma, const
                                                 static_cast<__nv_bfloat16*>(dx_bf16), dgamma, dbeta);
   VITK_CHECK_LAUNCH("cls_loss_bwd_kernel");
   if (dhead_w != nullptr) {
-    VITK_REQUIRE(dhead_b != nullptr, "cls_loss_bwd: dhead_b missing");
     head_wgrad_kernel<<<dim3(C, (D + 63) / 64), 256, 0, stream>>>(dlogits_ws, feat_ws, B, D, C,
                                                                   dhead_w, dhead_b);
     VITK_CHECK_LAUNCH("head_wgrad_kernel");

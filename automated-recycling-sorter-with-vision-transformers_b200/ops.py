@@ -218,7 +218,8 @@ def layernorm_bwd(dy: torch.Tensor, x: torch.Tensor, mean: torch.Tensor, rstd: t
     check(lib().vitk_layernorm_bwd(dy.data_ptr(), 1 if dy.dtype == torch.float32 else 0,
                                    x.data_ptr(), mean.data_ptr(), rstd.data_ptr(),
                                    weight.data_ptr(), dx.data_ptr(), 1 if dx_resid is not None else 0,
-                                   dxb.data_ptr(), dg.data_ptr(), db.data_ptr(), rows, D, _stream()))
+                                   dxb.data_ptr(), dg.data_ptr(), db.data_ptr(), rows, D, None,
+                                   0.0, 0, 0, 0, _stream()))
     return dx, dxb, dg, db
 
 

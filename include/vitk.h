@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define VITK_ABI_VERSION 7
+#define VITK_ABI_VERSION 8
 
 #define VITK_OK 0
 #define VITK_ERR_INVALID 1
@@ -293,7 +293,9 @@ int vitk_gemm_layernorm_folded(const void* x_bf16, int lda, const void* w_ln, in
 int vitk_gemm_wgrad(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* out,
                     int ldo, float alpha, float beta, int split_k, vitk_stream_t stream);
 
-/* nn.LayerNorm(D) over `rows` rows (train.py:581-582). y is bf16 (y_is_f32 = 0) or f32. */
+/* nn.LayerNorm(D) over `rows` rows (train.py:581-582). y is bf16 (y_is_f32 = 0) or f32.  D % 4 == 0,
+ * D <= 1024; strides multiples of 4; x, gamma, beta 16-byte aligned, y 16-byte (f32) or 8-byte
+ * (bf16) aligned. */
 int vitk_layernorm(const float* x, long long in_stride, const float* gamma, const float* beta,
                    void* y, int y_is_f32, long long out_stride, float* mean_out, float* rstd_out,
                    int rows, int D, float eps, vitk_stream_t stream);
@@ -469,10 +471,34 @@ int vitk_transpose_bf16_batched(int n, const void* const* src, void* const* dst,
                                 const int* cols, vitk_stream_t stream);
 
 /* Per-operator backward entry points (unit tests; the same kernels the step uses). */
+/* LayerNorm backward over dense [rows, D] rows (D % 4 == 0, D <= 1024): dx_io = dLN (+ dx_io when
+ * add_resid); dx_bf16 (optional) its bf16 copy; dgamma / dbeta (optional, together) accumulate.
+ * dx_colsum (optional, needs dx_bf16) accumulates the column sums of the bf16 copy; outside the
+ * fused kernel (dgamma given and D <= 768) it needs D % 8 == 0.  dropout_p > 0 (fused kernel and
+ * dx_bf16 only) applies the keep mask of vitk_dropout_keep_mask(dropout_p, seed, site, layer) at
+ * index row * D + column to the bf16 copy, which is then scaled by 1 / (1 - p); dx_io stays
+ * unmasked.  dy may be dx_io (f32, add_resid = 0).  Every argument is checked before the first
+ * launch, so a rejected call changes nothing. */
 int vitk_layernorm_bwd(const void* dy, int dy_is_f32, const float* x, const float* mean,
                        const float* rstd, const float* gamma, float* dx_io, int add_resid,
                        void* dx_bf16, float* dgamma, float* dbeta, int rows, int D,
+                       float* dx_colsum, float dropout_p, unsigned int seed, int site, int layer,
                        vitk_stream_t stream);
+/* The classifier tail of vitk_classifier_loss_backward on its own: for each image b, with the
+ * CLS row x + b*row_stride (D floats), feat = LayerNorm(x_b; gamma, beta, eps), logits = feat
+ * head_w^T + head_b (head_w [n_classes, D]), loss_out += scale * CE(logits, labels[b]) and the
+ * backward of that loss: dlogits_ws [batch, n_classes] and feat_ws [batch, D] (both required),
+ * dx (required) and dx_bf16 (optional) at the CLS rows (same row_stride; nothing else is
+ * written), dgamma /
+ * dbeta (optional, together) and dhead_w / dhead_b (optional, together) accumulate.
+ * logits_out [batch, n_classes] and loss_out are optional; n_classes <= 1024. */
+int vitk_classifier_head_loss_backward(const float* x, long long row_stride, const float* gamma,
+                                       const float* beta, const float* head_w, const float* head_b,
+                                       const long long* labels, float scale, float eps, int batch,
+                                       int D, int n_classes, float* logits_out, float* loss_out,
+                                       float* feat_ws, float* dlogits_ws, float* dx,
+                                       void* dx_bf16, float* dgamma, float* dbeta, float* dhead_w,
+                                       float* dhead_b, vitk_stream_t stream);
 int vitk_attention_bwd(const void* qkv_bf16, const void* ctx_bf16, const void* dctx_bf16,
                        const float* lse, void* dqkv_bf16, int batch, int n_tokens, int num_heads,
                        int head_dim, vitk_stream_t stream);
@@ -485,6 +511,8 @@ int vitk_attention_src_bwd(const void* q, long long q_img, int ldq, const void* 
                            int lddq, void* dk, void* dv, long long dkv_img, int lddkv, int batch,
                            int n_q, int n_k, int num_heads, int head_dim, float dropout_p,
                            unsigned int seed, int site, int layer, vitk_stream_t stream);
+/* out[n] += sum_m y[m, n] over a bf16 [M, N] matrix of row pitch ld (N and ld multiples of 8, y
+ * 16-byte aligned). */
 int vitk_colsum_bf16(const void* y, long long ld, int M, int N, float* out, vitk_stream_t stream);
 
 /* ============ detection head (ObjectDetectionHead, evaluation.py:160-200 == train.py:691-731) ====

@@ -41,5 +41,5 @@ dxb = torch.empty(M, D, device="cuda", dtype=torch.bfloat16)
 st = torch.cuda.current_stream().cuda_stream
 ms = timeit(lambda: vitk._lib.check(vitk._lib.lib().vitk_layernorm_bwd(
     dy.data_ptr(), 0, x.data_ptr(), mean.data_ptr(), rstd.data_ptr(), g.data_ptr(), dx.data_ptr(), 1,
-    dxb.data_ptr(), dgam.data_ptr(), dbet.data_ptr(), M, D, st)))
+    dxb.data_ptr(), dgam.data_ptr(), dbet.data_ptr(), M, D, None, 0.0, 0, 0, 0, st)))
 print(f"layernorm bwd rows={M}: {ms*1e3:7.1f} us  {M*D*16/ms/1e6:7.0f} GB/s (algorithmic 16 B/elem)")

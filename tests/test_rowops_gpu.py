@@ -1,27 +1,11 @@
-"""LayerNorm / patchify / attention kernels through the C ABI vs fp32 PyTorch on the same inputs."""
+"""Patchify / attention kernels through the C ABI vs fp32 PyTorch on the same inputs (the LayerNorm
+forward is tested in test_train_rowops_gpu.py)."""
 import math
 
 import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.mark.parametrize("rows,D", [(1, 768), (197, 768), (6304, 768), (50, 1024), (33, 400), (7, 64)])
-@pytest.mark.parametrize("out_dtype", [torch.bfloat16, torch.float32])
-def test_layernorm(vitk, rows, D, out_dtype):
-    g = torch.Generator(device="cuda").manual_seed(0)
-    x = torch.randn(rows, D, generator=g, device="cuda") * 3 + 1.5
-    w = torch.randn(D, generator=g, device="cuda")
-    b = torch.randn(D, generator=g, device="cuda")
-    y, mean, rstd = vitk.ops.layernorm(x, w, b, 1e-5, out_dtype, return_stats=True)
-    ref = torch.nn.functional.layer_norm(x, (D,), w, b, 1e-5)
-    if out_dtype == torch.float32:
-        torch.testing.assert_close(y, ref, rtol=1e-5, atol=1e-5)
-    else:
-        torch.testing.assert_close(y.float(), ref.bfloat16().float(), rtol=1e-2, atol=1e-2)
-    torch.testing.assert_close(mean, x.mean(-1), rtol=1e-5, atol=1e-5)
-    torch.testing.assert_close(rstd, 1 / torch.sqrt(x.var(-1, unbiased=False) + 1e-5), rtol=1e-4, atol=1e-5)
 
 
 @pytest.mark.parametrize("B,C,S,p", [(2, 3, 224, 16), (3, 3, 32, 16), (1, 3, 384, 16), (2, 1, 64, 8)])
